@@ -3,7 +3,7 @@
 back-projection path (forward + backward) on B200, with the HBM roofline of the
 dominant kernel and the CPU baseline beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): one synthetic ScanNet-shaped scene per step
 -- V=20 views, 320x240 images -> 60x80 FPN features x 256 channels, D=12 depth
@@ -167,11 +167,11 @@ CPU_SAMPLE_VIEWS = 4          # reference views swept per CPU step: FIXED (round
                               # wall-clock budget, which moved the number by 1.9x between runs)
 
 
-def time_cpu_reference(cfg, steps: int, warmup: int, budget_s: float):
+def time_cpu_reference(cfg, steps: int, warmup: int, budget_s=None):
     """The oracle on the host cores: always ``CPU_SAMPLE_VIEWS`` of the scene's reference views per
     step (every stage of the path is linear in the number of reference views; the neighbours are
     still drawn from all V), ``warmup`` untimed + ``steps`` timed steps, MEDIAN step time, scaled to
-    a scene.  Only the number of timed steps is bounded by ``budget_s`` (never below 3)."""
+    a scene.  With ``budget_s`` the number of timed steps is bounded by it (never below 3)."""
     from mvsdet_b200.scene import make_scene
     threads = os.cpu_count() or 1
     torch.set_num_threads(threads)
@@ -183,7 +183,7 @@ def time_cpu_reference(cfg, steps: int, warmup: int, budget_s: float):
     t_first = time.perf_counter() - t0
     for _ in range(max(0, warmup - 1)):
         cpu_reference_step(scene, vs)
-    n_timed = max(3, min(max(1, steps), int(budget_s / max(t_first, 1e-3))))
+    n_timed = steps if budget_s is None else max(3, min(max(1, steps), int(budget_s / max(t_first, 1e-3))))
     times = []
     for _ in range(n_timed):
         t0 = time.perf_counter()
@@ -202,7 +202,7 @@ def run_reference_arm(args, cfg, cfg_json):
     rank, local, world = _dist_env()
     if rank != 0:
         return
-    val, t_step, threads, sample, nsteps = time_cpu_reference(cfg, args.steps, args.warmup, 200.0)
+    val, t_step, threads, sample, nsteps = time_cpu_reference(cfg, args.steps, args.warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
         "steps": nsteps, "warmup": args.warmup, "ms_per_step": t_step * 1e3,
@@ -254,6 +254,52 @@ def _time_steps(step_fn, steps, warmup, barrier):
     e1.record()
     barrier()
     return e0.elapsed_time(e1), wall0, time.time()
+
+
+DUMP_BUDGET = 64 << 20       # bytes: all dumped files together
+
+
+def snapshot_outputs(pipe):
+    """What ``pipe``'s last step handed its caller, in the caller's logical layouts, as float32 host
+    arrays: the variance volume [V,C,D,Hf,Wf] (input of the cost-regularisation net), the top-k
+    products, volume_mean [C,nx,ny,nz], count [nx,ny,nz], g_feature [V,C,Hf,Wf] and g_cost_out.
+    Each output gets an equal share of DUMP_BUDGET; a larger one is reduced to the elements at
+    fixed, seeded positions of its logical (row-major) index, so two builds sample the same ones."""
+    import numpy as np
+    cfg = pipe.cfg
+    outs = {
+        "variance": pipe.variance.permute(0, 4, 1, 2, 3),
+        "prob_volume": pipe.prob_volume, "off_pred": pipe.off_pred,
+        "est_depth": pipe.est_depth, "est_densities": pipe.est_dens, "est_idx": pipe.est_idx,
+        "depth_coding": pipe.depth_coding,
+        "volume_mean": pipe.volume_mean.view(cfg.channels, *cfg.n_voxels),
+        "count": pipe.count.view(*cfg.n_voxels),
+        "g_feature": pipe.g_feature, "g_cost_out": pipe.g_cost_out,
+    }
+    cap = DUMP_BUDGET // (4 * len(outs))             # float32 elements per output
+    arrays, info = {}, {}
+    for seed, (name, t) in enumerate(outs.items()):
+        if t.numel() <= cap:
+            arrays[name] = t.float().cpu().numpy()
+            info[name] = {"shape": list(t.shape)}
+            continue
+        flat = np.sort(np.random.default_rng(seed).choice(t.numel(), cap, replace=False))
+        idx = torch.from_numpy(np.stack(np.unravel_index(flat, tuple(t.shape)))).to(t.device)
+        arrays[name] = t[tuple(idx)].float().cpu().numpy()
+        info[name] = {"shape": list(t.shape), "sampled": cap,
+                      "sample": f"np.sort(np.random.default_rng({seed}).choice({t.numel()}, {cap}, "
+                                "replace=False)) of the row-major index"}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_BUDGET}-byte budget")
+    return arrays, info
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def _kernel_table(pipes, ksteps):
@@ -605,7 +651,13 @@ def run_own_arm(args, cfg, cfg_json):
     ms_total = rank_max(ms_total)
     ms_per_step = ms_total / args.steps
     value = world * args.steps / (ms_total * 1e-3)
-    # the same measurement over a long run (sustained clocks / power), when the driver's K is short
+    # the outputs of the last timed step, before any later leg reuses the buffers
+    dump = None
+    if args.dump_outputs and rank == 0:
+        arrays, dump = snapshot_outputs(pipes[(args.steps - 1) % NBUF])
+        write_outputs(args.dump_outputs, arrays)
+        del arrays
+    # the same measurement over a long run (sustained clocks / power), on request
     sustained = None
     if args.steps < args.sustained_steps:
         ms_s, ws0, ws1 = _time_steps(one_step, args.sustained_steps, 3, barrier)
@@ -862,6 +914,9 @@ def run_own_arm(args, cfg, cfg_json):
         }
         if sustained is not None:
             line["sustained"] = sustained
+        if dump is not None:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "dtype": "float32", "step": args.steps - 1,
+                                      "outputs": dump}
         if module_api is not None:
             line["module_api"] = module_api
         if f32_line is not None:
@@ -909,8 +964,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=30)
-    ap.add_argument("--sustained-steps", type=int, default=600,
-                    help="a second timed run of this many steps when --steps is shorter (sustained clocks)")
+    ap.add_argument("--sustained-steps", type=int, default=0,
+                    help="a second timed run of this many steps when --steps is shorter (sustained clocks); "
+                         "reported apart from the headline, off by default")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, 64 MB in all; "
+                         "a large output as a fixed, seeded sample), for comparing two builds")
     ap.add_argument("--no-extras", action="store_true", help="skip the fp32-feature and eager-GPU legs")
     ap.add_argument("--no-sharded", action="store_true", help="N > 1: skip the view-sharded V=80 leg")
     ap.add_argument("--sharded-views", type=int, default=80)
@@ -918,6 +977,10 @@ def main():
                     help="BASELINE.json configs[4] instead of the step benchmark: depth-plane / view-count / "
                          "resolution sweep of the plane-sweep kernels (tools/sweep_chart.py), one JSON line")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs needs --impl own")
     if args.sweep:
         run_sweep(args)
         return

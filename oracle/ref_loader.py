@@ -1,15 +1,16 @@
 """Loader for the UNMODIFIED reference functions of the MVSDet hot path.
 
 TEST INFRASTRUCTURE ONLY.  This module executes the reference's own Python
-source from ``/root/reference`` (read-only mount; it exists only in the build
-container, never on the GPU box).  Nothing is copied into this repository: the
-functions are sliced out of the reference files with ``ast`` at call time and
-``exec``-ed in a scratch namespace, exactly as SURVEY.md section 8(c) describes.
+source from a checkout of the original MVSDet project named by the environment
+variable ``MVSDET_REFERENCE_ROOT``; the repository does not contain one.  Nothing
+is copied into this repository: the functions are sliced out of the reference
+files with ``ast`` at call time and ``exec``-ed in a scratch namespace, exactly
+as SURVEY.md section 8(c) describes.
 
 It is used for two things only:
   * ``tests/golden/make_golden.py`` -- generate the committed golden vectors;
   * ``tests/test_oracle_vs_reference.py`` -- pin ``oracle/mvsdet_oracle.py``
-    against the live reference when the mount is present (skipped otherwise).
+    against the live reference when the checkout is given (skipped otherwise).
 
 Reference entry points loaded (all under projects/NeRF-Det/nerfdet/):
   mvs_models/module.py:105-146   homo_warping
@@ -25,7 +26,7 @@ Reference entry points loaded (all under projects/NeRF-Det/nerfdet/):
   mvsdet.py:1272-1313            get_camera_params, lift
   mvsdet.py:319-333              MVSDet.process_rgb_raw
 The last two groups call ``.cuda()`` on freshly created tensors (mvsdet.py:1283, :1302, :1313);
-``cpu_cuda_shim()`` makes ``Tensor.cuda`` the identity while they run in this GPU-less container
+``cpu_cuda_shim()`` makes ``Tensor.cuda`` the identity so they run on the CPU
 -- the executed source is still the reference's, unmodified.
 """
 from __future__ import annotations
@@ -37,7 +38,7 @@ import os
 import types
 import warnings
 
-REFERENCE_ROOT = os.environ.get("MVSDET_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("MVSDET_REFERENCE_ROOT", "")
 _NERFDET = os.path.join(REFERENCE_ROOT, "projects", "NeRF-Det", "nerfdet")
 
 _FREE_FUNCS = ("knn", "get_nearest_pose_ids", "get_points", "backproject_Weigh",
@@ -48,7 +49,7 @@ _METHODS = ("collect_proj", "sample_depth_prob", "compute_avg_depth",
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(_NERFDET, "mvsdet.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(_NERFDET, "mvsdet.py"))
 
 
 def _load_module_py():
@@ -63,8 +64,8 @@ def load() -> types.SimpleNamespace:
     """Return a namespace holding the reference callables (see module doc)."""
     if not available():
         raise FileNotFoundError(
-            f"reference tree not mounted at {REFERENCE_ROOT}; the reference "
-            "loader only works in the build container")
+            f"no MVSDet checkout at MVSDET_REFERENCE_ROOT={REFERENCE_ROOT!r}; set it to the "
+            "root of the original project")
     import numpy as np
     import torch
     import torch.nn.functional as F
@@ -97,7 +98,7 @@ def load() -> types.SimpleNamespace:
 
 
 class cpu_cuda_shim:
-    """Context manager: ``Tensor.cuda()`` returns the tensor itself (build container has no GPU)."""
+    """Context manager: ``Tensor.cuda()`` returns the tensor itself (the reference code runs on the CPU)."""
 
     def __enter__(self):
         import torch

@@ -1,13 +1,13 @@
 #!/usr/bin/env python
 """Generate the golden vectors under tests/golden/ by EXECUTING THE REFERENCE.
 
-Run in the build container only (needs the read-only mount /root/reference):
+Needs a checkout of the original MVSDet project:
 
-    python tests/golden/make_golden.py
+    MVSDET_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 
 For every case below it builds a seeded synthetic scene
 (mvsdet_b200.scene.make_scene), runs the reference's own functions -- sliced
-verbatim out of /root/reference by oracle/ref_loader.py -- through the glue
+verbatim out of that checkout by oracle/ref_loader.py -- through the glue
 of MVSDet.extract_feat (projects/NeRF-Det/nerfdet/mvsdet.py:404-515, :681-682,
 followed statement by statement, out-of-place training branch :458-459), and
 stores inputs, every intermediate the parity tests compare, and the autograd

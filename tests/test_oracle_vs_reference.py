@@ -1,10 +1,12 @@
-"""Pin the oracle against the LIVE reference (build container only).
+"""Pin the oracle and the product's geometry against the reference.
 
-``oracle/ref_loader.py`` slices the reference's own functions out of
-/root/reference and executes them verbatim; here fresh seeded scenes -- not the
-ones frozen in tests/golden -- go through both the reference chain
-(tests/golden/make_golden.py: mvsdet.py:404-515 followed statement by statement)
-and ``oracle.hot_path``.  Skipped where the mount does not exist (the GPU box).
+``oracle/ref_loader.py`` slices the reference's own functions out of a checkout
+of the original MVSDet project (``MVSDET_REFERENCE_ROOT``) and executes them
+verbatim; with it, fresh seeded scenes -- not the ones frozen in tests/golden --
+go through both the reference chain (tests/golden/make_golden.py: mvsdet.py:404-515
+followed statement by statement) and ``oracle.hot_path``.  The repository does
+not contain that checkout, so the tests that need it skip without it; the
+geometry comparison falls back to the reference outputs stored in tests/golden.
 """
 import importlib.util
 import os
@@ -13,12 +15,13 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import assert_close, oracle_chain
+from helpers import GOLDEN_CASES, assert_close, load_golden, oracle_chain
 from mvsdet_b200.scene import make_scene, tiny_config
 from oracle import ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(),
-                                reason="/root/reference is not mounted on this machine")
+needs_reference = pytest.mark.skipif(
+    not ref_loader.available(),
+    reason="needs a checkout of the original MVSDet project in MVSDET_REFERENCE_ROOT")
 
 CASES = [
     (tiny_config(n_views=6, channels=8, num_depth=8), 101),
@@ -41,6 +44,7 @@ def ref():
     return ref_loader.load()
 
 
+@needs_reference
 @pytest.mark.parametrize("cfg,seed", CASES)
 def test_oracle_equals_live_reference(ref, cfg, seed):
     mg = _make_golden_module()
@@ -55,11 +59,29 @@ def test_oracle_equals_live_reference(ref, cfg, seed):
         assert_close(got[key], want[key], rtol=1e-6, atol=1e-6, what=key)
 
 
-def test_geometry_mirrors_equal_live_reference(ref):
+def test_geometry_mirrors_equal_live_reference():
     """The product's host-side geometry (mvsdet_b200/geometry.py) against the
     reference's knn / get_nearest_pose_ids / collect_proj / get_points /
-    _compute_projection on the same camera set."""
+    _compute_projection: bit for bit against their outputs stored in tests/golden
+    for the golden scenes and, with the reference checkout, live on one more camera set."""
     from mvsdet_b200 import geometry as G
+    for case in GOLDEN_CASES:
+        scene, gold = load_golden(case)
+        cfg, meta = scene["cfg"], scene["img_meta"]
+        w2c = torch.tensor(np.array(meta["lidar2img"]["extrinsic"]))
+        c2w = w2c.inverse()
+        nbr = G.get_nearest_pose_ids(c2w, c2w, min(2, cfg.n_views - 1), maskself=True)   # mvsdet.py:432-434
+        assert np.array_equal(nbr.numpy(), gold["neighbor_ids"]), case
+        kf = G.feature_intrinsics(torch.tensor(np.array(meta["lidar2img"]["intrinsic"])), cfg.ratio)
+        ref_proj, nei_projs = G.collect_proj(w2c, kf, nbr)
+        assert np.array_equal(ref_proj.numpy(), gold["ref_proj"]), case
+        assert np.array_equal(torch.stack(nei_projs).numpy(), gold["nei_projs"]), case
+        assert np.array_equal(G.compute_projection(meta, cfg.stride).numpy(), gold["projection"]), case
+        points = G.get_points(cfg.n_voxels, cfg.voxel_size, meta["lidar2img"]["origin"])
+        assert np.array_equal(points.numpy(), gold["points"]), case
+    if not ref_loader.available():
+        return
+    ref = ref_loader.load()
     cfg = tiny_config(n_views=9, channels=4)
     scene = make_scene(cfg, 7)
     meta = scene["img_meta"]
@@ -81,6 +103,7 @@ def test_geometry_mirrors_equal_live_reference(ref):
     assert torch.equal(pts, G.get_points(cfg.n_voxels, cfg.voxel_size, meta["lidar2img"]["origin"]))
 
 
+@needs_reference
 def test_costreg_restatement_equals_reference_class():
     """oracle/costreg_oracle.CostRegNet3DGS (what the GPU tests attach to the drop-in) against the
     reference's CostRegNet_3DGS (mvs_models/mvsnet.py:73-113), loaded under a synthetic package
@@ -113,6 +136,7 @@ def test_costreg_restatement_equals_reference_class():
         assert torch.equal(theirs(x.clone()), mine(x.clone()))
 
 
+@needs_reference
 def test_group_correlation_equals_reference_statements(ref):
     """SURVEY 8f rank 4: the oracle's group-wise correlation against the reference's own statements
     (mvs_models/lss_fpn.py:496-503, sliced and executed verbatim) fed with the reference's own
