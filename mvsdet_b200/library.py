@@ -9,10 +9,11 @@ calls it"): dispatcher-visible ops ``torch.ops.mvsdet_b200.*`` with
 * autograd through ``register_autograd`` whose backward formulas call the ``*_bwd`` ops,
   themselves registered, so double tracing (AOT autograd) sees only these ops.
 
-The ``torch.autograd.Function`` layer in ``ops.py`` is the same arithmetic (both call the
-``_*_raw`` launchers there); it additionally offers caller-owned output buffers for the
-peer-memory multi-GPU combine, which a functional dispatcher op cannot (no aliasing of
-inputs).  ``MVSDetHotPath(dispatcher_ops=True)`` routes the drop-in through this module.
+The ``torch.autograd.Function`` layer in ``ops.py`` is the same arithmetic (both allocate
+through the ``_*_raw`` helpers there, check arguments with the same functions and launch
+through ``_lib``); it additionally offers caller-owned output buffers for the peer-memory
+multi-GPU combine, which a functional dispatcher op cannot (no aliasing of inputs).
+``MVSDetHotPath(dispatcher_ops=True)`` routes the drop-in through this module.
 
 Operators (reference lines as in ``ops.py``):
 
@@ -44,32 +45,13 @@ __all__ = ["plane_sweep_variance", "plane_sweep_group_correlation", "depth_topk"
 _NS = "mvsdet_b200"
 
 
-def _check(cond: bool, msg: str) -> None:
-    if not cond:
-        raise ValueError(msg)
-
-
-def _ndhwc_like(v, c, d, h, w, dtype, device) -> Tensor:
-    return torch.empty((v, d, h, w, c), dtype=dtype, device=device).permute(0, 4, 1, 2, 3)
-
-
-def _nhwc_like(v, c, h, w, dtype, device) -> Tensor:
-    return torch.empty((v, h, w, c), dtype=dtype, device=device).permute(0, 3, 1, 2)
-
-
 # --------------------------------------------------------------------------
 # plane sweep
 # --------------------------------------------------------------------------
 @torch.library.custom_op(f"{_NS}::plane_sweep_variance", mutates_args=(), device_types="cuda")
 def plane_sweep_variance(feat: Tensor, nbr_ids: Tensor, hom: Tensor, depth_values: Tensor,
                          out_bf16: bool = False, ref_begin: int = 0) -> Tensor:
-    _check(_ops._is_nhwc(feat), "feat must be channels_last; use ops.pack_features")
-    _check(nbr_ids.dtype == torch.int32 and nbr_ids.is_contiguous(), "nbr_ids must be contiguous int32 [V,k]")
-    v, k = nbr_ids.shape
-    _check(tuple(hom.shape) == (v, k, 12) and depth_values.shape[0] == v,
-           "nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
-    _check(0 <= ref_begin and ref_begin + v <= feat.shape[0], "reference views [ref_begin, ref_begin+V) exceed feat")
-    _check(hom.dtype == torch.float32 and depth_values.dtype == torch.float32, "hom and depth_values must be float32")
+    _ops._check_sweep(feat, nbr_ids, hom, depth_values, ref_begin)
     return _ops._sweep_fwd_raw(feat, nbr_ids, hom.contiguous(), depth_values.contiguous(),
                                torch.bfloat16 if out_bf16 else torch.float32, int(ref_begin))
 
@@ -77,8 +59,8 @@ def plane_sweep_variance(feat: Tensor, nbr_ids: Tensor, hom: Tensor, depth_value
 @plane_sweep_variance.register_fake
 def _(feat, nbr_ids, hom, depth_values, out_bf16=False, ref_begin=0):
     _, c, h, w = feat.shape
-    return _ndhwc_like(nbr_ids.shape[0], c, depth_values.shape[1], h, w,
-                       torch.bfloat16 if out_bf16 else torch.float32, feat.device)
+    return _ops._empty_ndhwc(nbr_ids.shape[0], c, depth_values.shape[1], h, w,
+                             torch.bfloat16 if out_bf16 else torch.float32, feat.device)
 
 
 @torch.library.custom_op(f"{_NS}::plane_sweep_variance_bwd", mutates_args=(), device_types="cuda")
@@ -90,7 +72,7 @@ def plane_sweep_variance_bwd(g: Tensor, feat: Tensor, nbr_ids: Tensor, hom: Tens
 @plane_sweep_variance_bwd.register_fake
 def _(g, feat, nbr_ids, hom, depth_values, ref_begin):
     v, c, h, w = feat.shape
-    return _nhwc_like(v, c, h, w, feat.dtype, feat.device)
+    return _ops._empty_nhwc(v, c, h, w, feat.dtype, feat.device)
 
 
 def _sweep_setup(ctx, inputs, output):
@@ -115,15 +97,7 @@ plane_sweep_variance.register_autograd(_sweep_backward, setup_context=_sweep_set
 @torch.library.custom_op(f"{_NS}::plane_sweep_group_correlation", mutates_args=(), device_types="cuda")
 def plane_sweep_group_correlation(feat: Tensor, nbr_ids: Tensor, hom: Tensor, depth_values: Tensor,
                                   num_groups: int = 8, ref_begin: int = 0) -> Tensor:
-    _check(_ops._is_nhwc(feat), "feat must be channels_last; use ops.pack_features")
-    _check(nbr_ids.dtype == torch.int32 and nbr_ids.is_contiguous(), "nbr_ids must be contiguous int32 [V,k]")
-    v, k = nbr_ids.shape
-    _check(k >= 1, "group correlation needs at least one neighbour")
-    _check(tuple(hom.shape) == (v, k, 12) and depth_values.dim() == 2 and depth_values.shape[0] == v,
-           "nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
-    _check(0 <= ref_begin and ref_begin + v <= feat.shape[0], "reference views [ref_begin, ref_begin+V) exceed feat")
-    _check(hom.dtype == torch.float32 and depth_values.dtype == torch.float32, "hom and depth_values must be float32")
-    _check(num_groups >= 1 and feat.shape[1] % num_groups == 0, "the channel count must be divisible by num_groups")
+    _ops._check_corr(feat, nbr_ids, hom, depth_values, num_groups, ref_begin)
     return _ops._corr_fwd_raw(feat, nbr_ids, hom.contiguous(), depth_values.contiguous(), int(num_groups),
                               int(ref_begin))
 
@@ -139,13 +113,13 @@ def _(feat, nbr_ids, hom, depth_values, num_groups=8, ref_begin=0):
 @torch.library.custom_op(f"{_NS}::plane_sweep_group_correlation_bwd", mutates_args=(), device_types="cuda")
 def plane_sweep_group_correlation_bwd(g: Tensor, feat: Tensor, nbr_ids: Tensor, hom: Tensor,
                                       depth_values: Tensor, num_groups: int, ref_begin: int) -> Tensor:
-    return _ops._corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, int(num_groups), int(ref_begin))
+    return _ops._corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, int(ref_begin))
 
 
 @plane_sweep_group_correlation_bwd.register_fake
 def _(g, feat, nbr_ids, hom, depth_values, num_groups, ref_begin):
     v, c, h, w = feat.shape
-    return _nhwc_like(v, c, h, w, feat.dtype, feat.device)
+    return _ops._empty_nhwc(v, c, h, w, feat.dtype, feat.device)
 
 
 def _corr_setup(ctx, inputs, output):
@@ -171,7 +145,7 @@ plane_sweep_group_correlation.register_autograd(_corr_backward, setup_context=_c
 @torch.library.custom_op(f"{_NS}::depth_topk", mutates_args=(), device_types="cuda")
 def depth_topk(cost_out: Tensor, near: float, interval: float, topk: int,
                raw: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
-    _check(cost_out.dim() == 5 and cost_out.shape[1] == 2, "cost_out must be [V,2,D,H,W]")
+    _ops._check_cost("cost_out", cost_out)
     _, outs = _ops._topk_fwd_raw(cost_out, near, interval, int(topk), int(raw))
     return outs
 
@@ -191,7 +165,7 @@ def depth_topk_bwd(cost_out: Tensor, est_idx: Tensor, g_prob: Optional[Tensor], 
                    g_depth: Optional[Tensor], g_dens: Optional[Tensor], g_coding: Optional[Tensor],
                    near: float, interval: float, topk: int, raw: bool) -> Tensor:
     return _ops._topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding,
-                              near, interval, int(topk), int(raw))
+                              near, interval, int(raw))
 
 
 @depth_topk_bwd.register_fake
@@ -222,22 +196,11 @@ depth_topk.register_autograd(_topk_backward, setup_context=_topk_setup)
 # --------------------------------------------------------------------------
 # back-projection + aggregation
 # --------------------------------------------------------------------------
-def _check_bp(feat, points, projection, est_depth, est_dens, height, width):
-    _check(_ops._is_nhwc(feat), "feat must be channels_last; use ops.pack_features")
-    v, _, fh, fw = feat.shape
-    for name, t in (("est_depth", est_depth), ("est_dens", est_dens)):
-        _check(t.dim() == 4 and t.shape[0] == v and t.shape[2] == fh and t.shape[3] == fw,
-               f"{name} must be [V,T,{fh},{fw}] (the full, un-cropped map)")
-        _check(t.dtype == torch.float32, f"{name} must be float32")
-    _check(tuple(projection.shape) == (v, 3, 4), "projection must be [V,3,4]")
-    _check(height <= fh and width <= fw, "crop exceeds the feature map")
-
-
 @torch.library.custom_op(f"{_NS}::backproject_aggregate", mutates_args=(), device_types="cuda")
 def backproject_aggregate(feat: Tensor, points: Tensor, projection: Tensor, est_depth: Tensor,
                           est_dens: Tensor, vs_z: float, height: int, width: int,
                           sum_only: bool = False, channels_first: bool = True) -> Tuple[Tensor, Tensor]:
-    _check_bp(feat, points, projection, est_depth, est_dens, height, width)
+    _ops._check_bp(feat, points, projection, est_depth, est_dens, height, width)
     if est_depth.stride() != est_dens.stride():
         est_depth, est_dens = est_depth.contiguous(), est_dens.contiguous()
     return _ops._bp_fwd_raw(feat, points.contiguous().float(), projection.contiguous().float(),
@@ -272,7 +235,7 @@ def _(g_out, feat, points, projection, est_depth, est_dens, count, vs_z, height,
     v, c, fh, fw = feat.shape
     if est_depth.stride() != est_dens.stride():
         est_dens = est_dens.contiguous()
-    return (_nhwc_like(v, c, fh, fw, feat.dtype, feat.device),
+    return (_ops._empty_nhwc(v, c, fh, fw, feat.dtype, feat.device),
             torch.empty_strided(est_dens.size(), est_dens.stride(), dtype=est_dens.dtype,
                                 device=est_dens.device))
 

@@ -19,7 +19,7 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib
-from ._lib import (BF16, BP_MEAN, BP_PER_VIEW, BP_SUM, CHANNELS_FIRST, CHANNELS_LAST, F32)
+from ._lib import BP_MEAN, BP_PER_VIEW, BP_SUM
 
 __all__ = ["pack_features", "plane_sweep_variance", "homo_warp", "depth_topk", "depth_topk_nvs",
            "topk_hypotheses", "ray_depth_scale", "rgb_downsample4", "backproject_aggregate",
@@ -29,30 +29,6 @@ __all__ = ["pack_features", "plane_sweep_variance", "homo_warp", "depth_topk", "
 # --------------------------------------------------------------------------
 # helpers
 # --------------------------------------------------------------------------
-_raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)
-
-
-def _stream() -> int:
-    """cudaStream_t of torch's current stream on the current device.  torch.cuda.current_stream()
-    builds a Stream object through three layers of device-index helpers (16 us per call, ten calls
-    per scene: 15 % of the drop-in's host time); the raw getter inductor uses is one C call."""
-    if _raw_stream is not None:
-        return _raw_stream(torch._C._cuda_getDevice())
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _ptr(t: Optional[torch.Tensor]):
-    return None if t is None else t.data_ptr()
-
-
-def _code(dtype: torch.dtype) -> int:
-    if dtype == torch.float32:
-        return F32
-    if dtype == torch.bfloat16:
-        return BF16
-    raise ValueError(f"mvsdet_b200 kernels take float32 or bfloat16, got {dtype}")
-
-
 def _need_cuda(name: str, t: torch.Tensor) -> None:
     if not isinstance(t, torch.Tensor):
         raise ValueError(f"{name} must be a tensor")
@@ -145,17 +121,26 @@ def fixed_to_float(q: torch.Tensor) -> torch.Tensor:
         raise ValueError("fixed_to_float takes an int64 accumulator")
     out = torch.empty_like(q, dtype=torch.float32)
     if q.numel():
-        _lib.call("mvsd_fixed_to_float", q.data_ptr(), out.data_ptr(), q.numel(), _stream())
+        _lib.fixed_to_float(q, out)
+    return out
+
+
+def _pack(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
+    out = _empty_nhwc(*x.shape, dtype, x.device)
+    _lib.pack(x, out)
+    return out
+
+
+def _unpack(acc: torch.Tensor) -> torch.Tensor:
+    out = torch.empty(acc.shape, dtype=torch.float32, device=acc.device)
+    _lib.unpack(acc, out)
     return out
 
 
 class _PackFeaturesSink(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x: torch.Tensor, dtype: torch.dtype, sink: FeatureGradSink):
-        v, c, h, w = x.shape
-        out = _empty_nhwc(v, c, h, w, dtype, x.device)
-        _lib.call("mvsd_pack_nchw_to_nhwc", x.data_ptr(), out.data_ptr(), _code(dtype),
-                  v, c, h, w, _stream())
+        out = _pack(x, dtype)
         ctx.sink = sink
         ctx.set_materialize_grads(False)
         return out
@@ -168,31 +153,21 @@ class _PackFeaturesSink(torch.autograd.Function):
             acc = g if acc is None else acc.add_(g)
         if acc is None:
             return None, None, None
-        v, c, h, w = acc.shape
         if not _is_nhwc(acc):
             acc = acc.contiguous(memory_format=torch.channels_last)
-        out = torch.empty((v, c, h, w), dtype=torch.float32, device=acc.device)
-        _lib.call("mvsd_unpack_nhwc_to_nchw", acc.data_ptr(), out.data_ptr(), 0, v, c, h, w, _stream())
-        return out, None, None
+        return _unpack(acc), None, None
 
 
 class _PackFeatures(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x: torch.Tensor, dtype: torch.dtype):
-        v, c, h, w = x.shape
-        out = _empty_nhwc(v, c, h, w, dtype, x.device)
-        _lib.call("mvsd_pack_nchw_to_nhwc", x.data_ptr(), out.data_ptr(), _code(dtype),
-                  v, c, h, w, _stream())
-        return out
+        return _pack(x, dtype)
 
     @staticmethod
     def backward(ctx, g: torch.Tensor):
-        v, c, h, w = g.shape
         if g.dtype != torch.float32 or not _is_nhwc(g):
             g = g.float().contiguous(memory_format=torch.channels_last)
-        out = torch.empty((v, c, h, w), dtype=torch.float32, device=g.device)
-        _lib.call("mvsd_unpack_nhwc_to_nchw", g.data_ptr(), out.data_ptr(), 0, v, c, h, w, _stream())
-        return out, None
+        return _unpack(g), None
 
 
 def pack_features(x: torch.Tensor, dtype: torch.dtype = torch.float32, sink: bool = False,
@@ -227,17 +202,13 @@ class _VolumeToNCDHW(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, vol):
-        v, c, d, h, w = vol.shape
-        out = torch.empty((v, c, d, h, w), dtype=torch.float32, device=vol.device)
-        _lib.call("mvsd_unpack_nhwc_to_nchw", vol.data_ptr(), out.data_ptr(), 0, v, c, d * h, w, _stream())
-        return out
+        return _unpack(vol)
 
     @staticmethod
     def backward(ctx, g):
-        v, c, d, h, w = g.shape
         g = g.float().contiguous()
-        out = _empty_ndhwc(v, c, d, h, w, torch.float32, g.device)
-        _lib.call("mvsd_pack_nchw_to_nhwc", g.data_ptr(), out.data_ptr(), F32, v, c, d * h, w, _stream())
+        out = _empty_ndhwc(*g.shape, torch.float32, g.device)
+        _lib.pack(g, out)
         return out
 
 
@@ -260,40 +231,24 @@ def volume_to_ncdhw(vol: torch.Tensor) -> torch.Tensor:
 # plane sweep
 # --------------------------------------------------------------------------
 def _sweep_fwd_raw(feat, nbr_ids, hom, depth_values, out_dtype, ref_begin):
-    """enqueue mvsd_plane_sweep_fwd; -> variance, logical [V,C,D,H,W] in channels_last_3d"""
+    """-> variance, logical [V,C,D,H,W] in channels_last_3d"""
     _, c, h, w = feat.shape
-    v = nbr_ids.shape[0]
-    d = depth_values.shape[1]
-    k = nbr_ids.shape[1]
-    out = _empty_ndhwc(v, c, d, h, w, out_dtype, feat.device)
-    _lib.call("mvsd_plane_sweep_fwd", feat.data_ptr(), _code(feat.dtype), _ptr(nbr_ids),
-              _ptr(hom), depth_values.data_ptr(), out.data_ptr(), _code(out_dtype),
-              CHANNELS_LAST, v, c, d, h, w, k, ref_begin, feat.shape[0], _stream())
+    out = _empty_ndhwc(nbr_ids.shape[0], c, depth_values.shape[1], h, w, out_dtype, feat.device)
+    _lib.plane_sweep_fwd(feat, nbr_ids, hom, depth_values, out, ref_begin=ref_begin)
     return out
 
 
 def _sweep_bwd_raw(g, feat, nbr_ids, hom, depth_values, ref_begin, acc=None):
-    """enqueue mvsd_plane_sweep_bwd; -> dL/dfeat in feat's dtype, channels_last.  ``acc``: an
-    fp32 channels-last accumulator to RED into instead (FeatureGradSink); returns None then."""
-    vf, c, h, w = feat.shape
-    v = nbr_ids.shape[0]
-    d = depth_values.shape[1]
-    k = nbr_ids.shape[1]
+    """-> dL/dfeat in feat's dtype, channels_last.  ``acc``: an fp32 channels-last accumulator to
+    RED into instead (FeatureGradSink); returns None then."""
     gdt = torch.bfloat16 if (g.dtype == torch.bfloat16 and feat.dtype == torch.bfloat16) else torch.float32
     g = _as_ndhwc(g, gdt)
     if acc is not None and acc.dtype == torch.int64:        # deterministic sink: fixed-point integer REDs
-        _lib.call("mvsd_plane_sweep_bwd_det", g.data_ptr(), _code(g.dtype), CHANNELS_LAST,
-                  feat.data_ptr(), _code(feat.dtype), _ptr(nbr_ids), _ptr(hom),
-                  depth_values.data_ptr(), acc.data_ptr(), v, c, d, h, w, k, ref_begin, vf, _stream())
+        _lib.plane_sweep_bwd_det(g, feat, nbr_ids, hom, depth_values, acc, ref_begin=ref_begin)
         return None
-    g_feat = acc if acc is not None else _zeros_nhwc(vf, c, h, w, torch.float32, feat.device)
-    _lib.call("mvsd_plane_sweep_bwd", g.data_ptr(), _code(g.dtype), CHANNELS_LAST,
-              feat.data_ptr(), _code(feat.dtype), _ptr(nbr_ids), _ptr(hom),
-              depth_values.data_ptr(), g_feat.data_ptr(), v, c, d, h, w, k, ref_begin, vf,
-              _stream())
-    if acc is not None:
-        return None
-    return g_feat.to(feat.dtype) if feat.dtype != torch.float32 else g_feat
+    g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
+    _lib.plane_sweep_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin=ref_begin)
+    return None if acc is not None else g_feat.to(feat.dtype)
 
 
 class _PlaneSweepVariance(torch.autograd.Function):
@@ -313,15 +268,9 @@ class _PlaneSweepVariance(torch.autograd.Function):
         return g_feat, None, None, None, None, None, None
 
 
-def plane_sweep_variance(feat: torch.Tensor, nbr_ids: torch.Tensor, hom: torch.Tensor,
-                         depth_values: torch.Tensor,
-                         out_dtype: torch.dtype = torch.float32,
-                         ref_begin: int = 0, grad_sink: Optional[FeatureGradSink] = None) -> torch.Tensor:
-    """Fused mvsdet.py:439-467: channels-last features [Vf,C,H,W] (fp32/bf16),
-    neighbour ids [V,k] int32 (indices into feat), homographies [V,k,12], depth
-    planes [V,D] -> variance volume, logical [V,C,D,H,W] in channels_last_3d.
-    Reference view v is feat[ref_begin + v]; V < Vf sweeps a slice of the views
-    (view-sharded multi-GPU)."""
+# The argument checks of an operator (_check_*) are shared by its function here and its
+# dispatcher op in library.py.
+def _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink=None) -> None:
     for n, t in (("feat", feat), ("nbr_ids", nbr_ids), ("hom", hom), ("depth_values", depth_values)):
         _need_cuda(n, t)
     if not _is_nhwc(feat):
@@ -337,38 +286,42 @@ def plane_sweep_variance(feat: torch.Tensor, nbr_ids: torch.Tensor, hom: torch.T
         raise ValueError("hom and depth_values must be float32")
     if grad_sink is not None and grad_sink.shape != tuple(feat.shape):
         raise ValueError("grad_sink belongs to a different feature tensor")
+
+
+def plane_sweep_variance(feat: torch.Tensor, nbr_ids: torch.Tensor, hom: torch.Tensor,
+                         depth_values: torch.Tensor,
+                         out_dtype: torch.dtype = torch.float32,
+                         ref_begin: int = 0, grad_sink: Optional[FeatureGradSink] = None) -> torch.Tensor:
+    """Fused mvsdet.py:439-467: channels-last features [Vf,C,H,W] (fp32/bf16),
+    neighbour ids [V,k] int32 (indices into feat), homographies [V,k,12], depth
+    planes [V,D] -> variance volume, logical [V,C,D,H,W] in channels_last_3d.
+    Reference view v is feat[ref_begin + v]; V < Vf sweeps a slice of the views
+    (view-sharded multi-GPU)."""
+    _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink)
     return _PlaneSweepVariance.apply(feat, nbr_ids, hom.contiguous(), depth_values.contiguous(),
                                      out_dtype, int(ref_begin), grad_sink)
 
 
 def _corr_fwd_raw(feat, nbr_ids, hom, depth_values, num_groups, ref_begin):
-    """enqueue mvsd_plane_sweep_groupcorr_fwd; -> logical [V,k,G,D,H,W] fp32, groups innermost in memory"""
-    vf, c, h, w = feat.shape
+    """-> logical [V,k,G,D,H,W] fp32, groups innermost in memory"""
+    _, _, h, w = feat.shape
     v, k = nbr_ids.shape
-    d = depth_values.shape[1]
-    out = torch.empty((v, k, d, h, w, num_groups), dtype=torch.float32, device=feat.device)
-    _lib.call("mvsd_plane_sweep_groupcorr_fwd", feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
-              hom.data_ptr(), depth_values.data_ptr(), out.data_ptr(), v, c, d, h, w, k, num_groups,
-              ref_begin, vf, _stream())
-    return out.permute(0, 1, 5, 2, 3, 4)
+    out = torch.empty((v, k, depth_values.shape[1], h, w, num_groups), dtype=torch.float32,
+                      device=feat.device).permute(0, 1, 5, 2, 3, 4)
+    _lib.plane_sweep_groupcorr_fwd(feat, nbr_ids, hom, depth_values, out, ref_begin=ref_begin)
+    return out
 
 
-def _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, num_groups, ref_begin, acc=None):
-    """enqueue mvsd_plane_sweep_groupcorr_bwd; -> dL/dfeat in feat's dtype (channels_last), or None
-    when it was accumulated into the fp32 accumulator ``acc`` (FeatureGradSink)"""
-    vf, c, h, w = feat.shape
-    v, k = nbr_ids.shape
-    d = depth_values.shape[1]
-    g = g.float().permute(0, 1, 3, 4, 5, 2).contiguous()          # no copy when it arrives in out's layout
+def _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, ref_begin, acc=None):
+    """-> dL/dfeat in feat's dtype (channels_last), or None when it was accumulated into the fp32
+    accumulator ``acc`` (FeatureGradSink)"""
+    # no copy when it arrives in the forward's layout
+    g = g.float().permute(0, 1, 3, 4, 5, 2).contiguous().permute(0, 1, 5, 2, 3, 4)
     if acc is not None and acc.dtype != torch.float32:
         raise ValueError("the group-correlation backward has no deterministic form")
-    g_feat = acc if acc is not None else _zeros_nhwc(vf, c, h, w, torch.float32, feat.device)
-    _lib.call("mvsd_plane_sweep_groupcorr_bwd", g.data_ptr(), feat.data_ptr(), _code(feat.dtype),
-              nbr_ids.data_ptr(), hom.data_ptr(), depth_values.data_ptr(), g_feat.data_ptr(),
-              v, c, d, h, w, k, num_groups, ref_begin, vf, _stream())
-    if acc is not None:
-        return None
-    return g_feat if feat.dtype == torch.float32 else g_feat.to(feat.dtype)
+    g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
+    _lib.plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin=ref_begin)
+    return None if acc is not None else g_feat.to(feat.dtype)
 
 
 class _GroupCorrelation(torch.autograd.Function):
@@ -376,17 +329,26 @@ class _GroupCorrelation(torch.autograd.Function):
     def forward(ctx, feat, nbr_ids, hom, depth_values, num_groups, ref_begin, sink=None):
         out = _corr_fwd_raw(feat, nbr_ids, hom, depth_values, num_groups, ref_begin)
         ctx.save_for_backward(feat, nbr_ids, hom, depth_values)
-        ctx.meta = (num_groups, ref_begin)
+        ctx.ref_begin = ref_begin
         ctx.sink = sink
         return out
 
     @staticmethod
     def backward(ctx, g):
         feat, nbr_ids, hom, depth_values = ctx.saved_tensors
-        num_groups, ref_begin = ctx.meta
         acc = ctx.sink.get() if ctx.sink is not None else None
-        g_feat = _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, num_groups, ref_begin, acc)
+        g_feat = _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, ctx.ref_begin, acc)
         return g_feat, None, None, None, None, None, None
+
+
+def _check_corr(feat, nbr_ids, hom, depth_values, num_groups, ref_begin, grad_sink=None) -> None:
+    _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink)
+    if nbr_ids.shape[1] < 1:
+        raise ValueError("group correlation needs at least one neighbour")
+    if depth_values.dim() != 2:
+        raise ValueError("nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
+    if num_groups < 1 or feat.shape[1] % num_groups != 0:
+        raise ValueError("the channel count must be divisible by num_groups")
 
 
 def plane_sweep_group_correlation(feat: torch.Tensor, nbr_ids: torch.Tensor, hom: torch.Tensor,
@@ -397,25 +359,7 @@ def plane_sweep_group_correlation(feat: torch.Tensor, nbr_ids: torch.Tensor, hom
     as ``plane_sweep_variance``; -> logical [V,k,num_groups,D,H,W] fp32, one volume per neighbour,
     ``mean over the group's channels of ref * warped_j``.  C / num_groups must be 4 ... 128 and divide
     128.  The memory order is [V,k,D,H,W,num_groups]."""
-    for n, t in (("feat", feat), ("nbr_ids", nbr_ids), ("hom", hom), ("depth_values", depth_values)):
-        _need_cuda(n, t)
-    if not _is_nhwc(feat):
-        raise ValueError("feat must be channels_last; use ops.pack_features")
-    if nbr_ids.dtype != torch.int32 or not nbr_ids.is_contiguous():
-        raise ValueError("nbr_ids must be contiguous int32 [V,k]")
-    v, k = nbr_ids.shape
-    if k < 1:
-        raise ValueError("group correlation needs at least one neighbour")
-    if tuple(hom.shape) != (v, k, 12) or depth_values.shape[0] != v or depth_values.dim() != 2:
-        raise ValueError("nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
-    if ref_begin < 0 or ref_begin + v > feat.shape[0]:
-        raise ValueError("reference views [ref_begin, ref_begin+V) exceed feat")
-    if hom.dtype != torch.float32 or depth_values.dtype != torch.float32:
-        raise ValueError("hom and depth_values must be float32")
-    if num_groups < 1 or feat.shape[1] % num_groups != 0:
-        raise ValueError("the channel count must be divisible by num_groups")
-    if grad_sink is not None and grad_sink.shape != tuple(feat.shape):
-        raise ValueError("grad_sink belongs to a different feature tensor")
+    _check_corr(feat, nbr_ids, hom, depth_values, num_groups, ref_begin, grad_sink)
     return _GroupCorrelation.apply(feat, nbr_ids, hom.contiguous(), depth_values.contiguous(),
                                    int(num_groups), int(ref_begin), grad_sink)
 
@@ -424,11 +368,8 @@ class _HomoWarp(torch.autograd.Function):
     @staticmethod
     def forward(ctx, src, hom, depth_values, out_dtype):
         b, c, h, w = src.shape
-        d = depth_values.shape[1]
-        out = _empty_ndhwc(b, c, d, h, w, out_dtype, src.device)
-        _lib.call("mvsd_homo_warp_fwd", src.data_ptr(), _code(src.dtype), hom.data_ptr(),
-                  depth_values.data_ptr(), out.data_ptr(), _code(out_dtype), CHANNELS_LAST,
-                  b, c, d, h, w, int(depth_values.dim() == 4), _stream())
+        out = _empty_ndhwc(b, c, depth_values.shape[1], h, w, out_dtype, src.device)
+        _lib.homo_warp_fwd(src, hom, depth_values, out)
         ctx.save_for_backward(hom, depth_values)
         ctx.src_meta = (src.shape, src.dtype)
         return out
@@ -436,14 +377,11 @@ class _HomoWarp(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         hom, depth_values = ctx.saved_tensors
-        (b, c, h, w), sdtype = ctx.src_meta
-        d = depth_values.shape[1]
+        shape, sdtype = ctx.src_meta
         g = _as_ndhwc(g, torch.float32 if g.dtype != torch.bfloat16 else torch.bfloat16)
-        g_src = _zeros_nhwc(b, c, h, w, torch.float32, g.device)
-        _lib.call("mvsd_homo_warp_bwd", g.data_ptr(), _code(g.dtype), CHANNELS_LAST, hom.data_ptr(),
-                  depth_values.data_ptr(), g_src.data_ptr(), b, c, d, h, w,
-                  int(depth_values.dim() == 4), _stream())
-        return (g_src if sdtype == torch.float32 else g_src.to(sdtype)), None, None, None
+        g_src = _zeros_nhwc(*shape, torch.float32, g.device)
+        _lib.homo_warp_bwd(g, hom, depth_values, g_src)
+        return g_src.to(sdtype), None, None, None
 
 
 def homo_warp(src: torch.Tensor, hom: torch.Tensor, depth_values: torch.Tensor,
@@ -464,35 +402,31 @@ def homo_warp(src: torch.Tensor, hom: torch.Tensor, depth_values: torch.Tensor,
 # --------------------------------------------------------------------------
 # softmax / sigmoid / top-k / expectation
 # --------------------------------------------------------------------------
-def _cost_strides(cost_out: torch.Tensor):
-    """(tensor, s_v, s_c, s_d, s_p) for NCDHW-contiguous or channels_last_3d."""
-    v, two, d, h, w = cost_out.shape
+def _as_cost(cost_out: torch.Tensor) -> torch.Tensor:
+    """fp32, NCDHW-contiguous or channels_last_3d (any strides with s_h = W * s_w)"""
     if cost_out.dtype != torch.float32:
         cost_out = cost_out.float()
     sv, sc, sd, sh, sw = cost_out.stride()
-    if sh != w * sw or (cost_out.numel() and min(sv, sc, sd, sw) < 1):
+    if sh != cost_out.shape[4] * sw or (cost_out.numel() and min(sv, sc, sd, sw) < 1):
         cost_out = cost_out.contiguous()
-        sv, sc, sd, sh, sw = cost_out.stride()
-    return cost_out, sv, sc, sd, sw
+    return cost_out
 
 
 def _ray_intr(ray_intr, v):
-    """[4,4] or [V,4,4] fp32 feature-level intrinsics -> (tensor, per_view flag)"""
+    """[4,4] or [V,4,4] fp32 feature-level intrinsics"""
     if ray_intr is None:
-        return None, 0
+        return None
     _need_cuda("ray_intrinsics", ray_intr)
     k = ray_intr.float().contiguous()
-    if tuple(k.shape) == (4, 4):
-        return k, 0
-    if tuple(k.shape) == (v, 4, 4):
-        return k, 1
+    if tuple(k.shape) in ((4, 4), (v, 4, 4)):
+        return k
     raise ValueError(f"ray intrinsics must be [4,4] or [{v},4,4], got {tuple(ray_intr.shape)}")
 
 
 def _topk_fwd_raw(cost_out, near, interval, topk, raw, ray_intr=None):
-    """enqueue mvsd_depth_topk_fwd; -> (cost_out as the kernel read it, the six outputs, and with
-    ``ray_intr`` the four NVS outputs opacity, depth_scale, est_ray_depth, ray_depth_coding)"""
-    cost_out, sv, sc, sd, sp = _cost_strides(cost_out)
+    """-> (cost_out as the kernel read it, the six outputs, and with ``ray_intr`` the four NVS
+    outputs opacity, depth_scale, est_ray_depth, ray_depth_coding)"""
+    cost_out = _as_cost(cost_out)
     v, _, d, h, w = cost_out.shape
     dev = cost_out.device
     f32 = dict(dtype=torch.float32, device=dev)
@@ -502,35 +436,37 @@ def _topk_fwd_raw(cost_out, near, interval, topk, raw, ray_intr=None):
     est_dens = torch.empty((v, topk, h, w), **f32)
     est_idx = torch.empty((v, topk, h, w), dtype=torch.int64, device=dev)
     coding = torch.empty((v, h, w), **f32)
-    kmat, per_view = _ray_intr(ray_intr, v)
+    kmat = _ray_intr(ray_intr, v)
     nvs = ()
     if kmat is not None:
         nvs = (torch.empty((v, h, w), **f32), torch.empty((v, h, w), **f32),
                torch.empty((v, topk, h, w), **f32), torch.empty((v, h, w), **f32))
-    _lib.call("mvsd_depth_topk_fwd", cost_out.data_ptr(), sv, sc, sd, sp, prob.data_ptr(),
-              off.data_ptr(), est_depth.data_ptr(), est_dens.data_ptr(), est_idx.data_ptr(),
-              coding.data_ptr(), _ptr(kmat), per_view, *(_ptr(t) for t in (nvs or (None,) * 4)),
-              float(near), float(interval), int(raw), v, d, h, w, topk, _stream())
+    _lib.depth_topk_fwd(cost_out, prob, off, est_depth, est_dens, est_idx, coding, near=near,
+                        interval=interval, raw=raw, ray_intr=kmat, nvs=nvs or (None,) * 4)
     return cost_out, (prob, off, est_depth, est_dens, est_idx, coding) + nvs
 
 
 def _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, near, interval,
-                  topk, raw, ray_intr=None, g_ray_depth=None, g_ray_coding=None):
-    """enqueue mvsd_depth_topk_bwd (any of the upstream gradients may be None)"""
-    cost_out, sv, sc, sd, sp = _cost_strides(cost_out)
-    v, _, d, h, w = cost_out.shape
+                  raw, ray_intr=None, g_ray_depth=None, g_ray_coding=None):
+    """-> dL/dcost_out (any of the upstream gradients may be None)"""
+    cost_out = _as_cost(cost_out)
 
     def prep(g):
         return None if g is None else g.contiguous().float()
     g_prob, g_off, g_depth, g_dens, g_coding, g_ray_depth, g_ray_coding = map(
         prep, (g_prob, g_off, g_depth, g_dens, g_coding, g_ray_depth, g_ray_coding))
-    kmat, per_view = _ray_intr(ray_intr, v)
-    g_cost = torch.empty((v, 2, d, h, w), dtype=torch.float32, device=cost_out.device)
-    _lib.call("mvsd_depth_topk_bwd", cost_out.data_ptr(), sv, sc, sd, sp, est_idx.data_ptr(),
-              _ptr(g_prob), _ptr(g_off), _ptr(g_depth), _ptr(g_dens), _ptr(g_coding),
-              _ptr(kmat), per_view, _ptr(g_ray_depth), _ptr(g_ray_coding),
-              g_cost.data_ptr(), float(near), float(interval), int(raw), v, d, h, w, topk, _stream())
+    kmat = _ray_intr(ray_intr, cost_out.shape[0])
+    g_cost = torch.empty(cost_out.shape, dtype=torch.float32, device=cost_out.device)
+    _lib.depth_topk_bwd(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, g_cost, near=near,
+                        interval=interval, raw=raw, ray_intr=kmat, g_ray_depth=g_ray_depth,
+                        g_ray_coding=g_ray_coding)
     return g_cost
+
+
+def _check_cost(name, cost_out) -> None:
+    _need_cuda(name, cost_out)
+    if cost_out.dim() != 5 or cost_out.shape[1] != 2:
+        raise ValueError(f"{name} must be [V,2,D,H,W]")
 
 
 class _DepthTopk(torch.autograd.Function):
@@ -538,16 +474,16 @@ class _DepthTopk(torch.autograd.Function):
     def forward(ctx, cost_out, near, interval, topk, raw):
         cost_out, outs = _topk_fwd_raw(cost_out, near, interval, topk, raw)
         ctx.save_for_backward(cost_out, outs[4])
-        ctx.consts = (float(near), float(interval), topk, int(raw))
+        ctx.consts = (float(near), float(interval), int(raw))
         ctx.mark_non_differentiable(outs[4])
         return outs
 
     @staticmethod
     def backward(ctx, g_prob, g_off, g_depth, g_dens, _g_idx, g_coding):
         cost_out, est_idx = ctx.saved_tensors
-        near, interval, topk, raw = ctx.consts
+        near, interval, raw = ctx.consts
         g_cost = _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding,
-                               near, interval, topk, raw)
+                               near, interval, raw)
         return g_cost, None, None, None, None
 
 
@@ -559,7 +495,7 @@ class _DepthTopkNVS(torch.autograd.Function):
     def forward(ctx, cost_out, near, interval, topk, ray_intr):
         cost_out, outs = _topk_fwd_raw(cost_out, near, interval, topk, 0, ray_intr)
         ctx.save_for_backward(cost_out, outs[4], ray_intr)
-        ctx.consts = (float(near), float(interval), topk)
+        ctx.consts = (float(near), float(interval))
         ctx.mark_non_differentiable(outs[4], outs[7])
         return outs
 
@@ -567,12 +503,12 @@ class _DepthTopkNVS(torch.autograd.Function):
     def backward(ctx, g_prob, g_off, g_depth, g_dens, _g_idx, g_coding, g_opacity, _g_scale,
                  g_ray_depth, g_ray_coding):
         cost_out, est_idx, ray_intr = ctx.saved_tensors
-        near, interval, topk = ctx.consts
+        near, interval = ctx.consts
         if g_opacity is not None:                      # opacity == est_dens[:, 0]
             g_dens = torch.zeros_like(est_idx, dtype=torch.float32) if g_dens is None else g_dens.clone()
             g_dens[:, 0] += g_opacity
         g_cost = _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding,
-                               near, interval, topk, 0, ray_intr, g_ray_depth, g_ray_coding)
+                               near, interval, 0, ray_intr, g_ray_depth, g_ray_coding)
         return g_cost, None, None, None, None
 
 
@@ -581,9 +517,7 @@ def depth_topk(cost_out: torch.Tensor, near: float, interval: float, topk: int):
     (:298-317).  cost_out [V,2,D,H,W] -> (prob_volume [V,D,H,W], off_pred
     [V,D,H,W], est_depth [V,T,H,W], est_densities [V,T,H,W], est_idx int64
     [V,T,H,W], depth_coding [V,H,W])."""
-    _need_cuda("cost_out", cost_out)
-    if cost_out.dim() != 5 or cost_out.shape[1] != 2:
-        raise ValueError("cost_out must be [V,2,D,H,W]")
+    _check_cost("cost_out", cost_out)
     return _DepthTopk.apply(cost_out, near, interval, int(topk), 0)
 
 
@@ -597,20 +531,17 @@ def depth_topk_nvs(cost_out: torch.Tensor, near: float, interval: float, topk: i
       est_ray_depth [V,T,H,W]   est_depth / (depth_scale + 1e-8)           mvsdet.py:494
       ray_depth_coding [V,H,W]  depth_coding / (depth_scale + 1e-8)        mvsdet.py:583
     (full, un-cropped maps; the caller crops / reshapes as it does est_depth)."""
-    _need_cuda("cost_out", cost_out)
-    if cost_out.dim() != 5 or cost_out.shape[1] != 2:
-        raise ValueError("cost_out must be [V,2,D,H,W]")
-    kmat, _ = _ray_intr(k_feat, cost_out.shape[0])
+    _check_cost("cost_out", cost_out)
+    kmat = _ray_intr(k_feat, cost_out.shape[0])
     return _DepthTopkNVS.apply(cost_out, near, interval, int(topk), kmat)
 
 
 def ray_depth_scale(k_feat: torch.Tensor, n_views: int, height: int, width: int) -> torch.Tensor:
     """compute_depth_scale / compute_depth_scale_MultiIntrin (mvsdet.py:1158-1218) alone:
     [4,4] or [V,4,4] feature-level intrinsics -> depth_scale [V,height,width]."""
-    kmat, per_view = _ray_intr(k_feat, n_views)
+    kmat = _ray_intr(k_feat, n_views)
     out = torch.empty((n_views, height, width), dtype=torch.float32, device=kmat.device)
-    _lib.call("mvsd_ray_depth_scale", kmat.data_ptr(), per_view, out.data_ptr(), n_views, height,
-              width, _stream())
+    _lib.ray_depth_scale(kmat, out)
     return out
 
 
@@ -620,7 +551,7 @@ def rgb_downsample4(rgb: torch.Tensor, src_ids, height: int, width: int) -> torc
     if rgb.dim() != 4 or rgb.shape[1] != 3:
         raise ValueError("rgb must be [V,3,H,W]")
     rgb = rgb.float().contiguous()
-    v, _, hh, ww = rgb.shape
+    v = rgb.shape[0]
     ids = None
     n = v
     if src_ids is not None:
@@ -630,8 +561,7 @@ def rgb_downsample4(rgb: torch.Tensor, src_ids, height: int, width: int) -> torc
         ids = ids.to(rgb.device)
         n = ids.numel()
     out = torch.empty((1, n, height * width, 3), dtype=torch.float32, device=rgb.device)
-    _lib.call("mvsd_rgb_downsample4", rgb.data_ptr(), _ptr(ids), n, out.data_ptr(), v, hh, ww,
-              int(height), int(width), _stream())
+    _lib.rgb_downsample4(rgb, ids, out, height=int(height), width=int(width))
     return out
 
 
@@ -639,9 +569,7 @@ def topk_hypotheses(prob_off: torch.Tensor, near: float, interval: float, topk: 
     """Stand-alone form of ``depth_topk`` for inputs that are already
     probabilities / offsets: prob_off [V,2,D,H,W] = stack(prob_volume, off_pred).
     Same six outputs (the first two are pass-through copies)."""
-    _need_cuda("prob_off", prob_off)
-    if prob_off.dim() != 5 or prob_off.shape[1] != 2:
-        raise ValueError("prob_off must be [V,2,D,H,W]")
+    _check_cost("prob_off", prob_off)
     return _DepthTopk.apply(prob_off, near, interval, int(topk), 1)
 
 
@@ -656,12 +584,10 @@ def _zeros_strided_like(t: torch.Tensor) -> torch.Tensor:
 
 def _bp_fwd_raw(feat, points, projection, est_depth, est_dens, vs_z, h, w, mode, channels_first,
                 out=None, count=None):
-    """enqueue mvsd_backproject_fwd (aggregating modes); -> (volume logical [C,N], count)"""
-    v, c, fh, fw = feat.shape
-    t = est_depth.shape[1]
+    """aggregating modes; -> (volume logical [C,N], count)"""
+    c = feat.shape[1]
     n = points.numel() // 3
     dev = feat.device
-    sv, st, sy, sx = est_depth.stride()
     shape = (c, n) if channels_first else (n, c)
     if out is None:
         out = torch.empty(shape, dtype=torch.float32, device=dev)
@@ -671,62 +597,37 @@ def _bp_fwd_raw(feat, points, projection, est_depth, est_dens, vs_z, h, w, mode,
         count = torch.empty((n,), dtype=torch.int32, device=dev)
     elif count.numel() != n or count.dtype != torch.int32 or not count.is_contiguous():
         raise ValueError("count must be a contiguous int32 [N] tensor")
-    _lib.call("mvsd_backproject_fwd", feat.data_ptr(), _code(feat.dtype), fh, fw,
-              points.data_ptr(), projection.data_ptr(), est_depth.data_ptr(),
-              est_dens.data_ptr(), sv, sy, sx, st, float(vs_z), mode, out.data_ptr(),
-              CHANNELS_FIRST if channels_first else CHANNELS_LAST, count.data_ptr(), None,
-              None, v, c, h, w, t, n, _stream())
-    return (out if channels_first else out.t()), count
+    vol = out if channels_first else out.t()
+    _lib.backproject_fwd(feat, points, projection, est_depth, est_dens, vol, vs_z=vs_z, mode=mode, height=h,
+                         width=w, channels_first=channels_first, count=count)
+    return vol, count
 
 
 def _bp_bwd_raw(g_out, feat, points, projection, est_depth, est_dens, count, vs_z, h, w, mode,
                 channels_first, acc=None):
-    """enqueue mvsd_backproject_bwd + mvsd_prob_norm_bwd; -> (dL/dfeat, dL/dest_dens); with ``acc``
+    """back-projection + prob-norm backward; -> (dL/dfeat, dL/dest_dens); with ``acc``
     (FeatureGradSink accumulator) the feature gradient is RED-added there and None is returned"""
-    v, c, fh, fw = feat.shape
-    t = est_depth.shape[1]
-    n = points.numel() // 3
-    sv, st, sy, sx = est_depth.stride()
     g_out = g_out.float()
-    g_mem = g_out.contiguous() if channels_first else g_out.t().contiguous()
+    g_mem = g_out.contiguous() if channels_first else g_out.t().contiguous().t()
     if acc is not None and acc.dtype == torch.int64:        # deterministic sink (MEAN mode only)
         if mode != BP_MEAN:
             raise ValueError("the deterministic backward is built for the mean aggregation only")
         g_pn_q = torch.zeros(est_dens.shape, dtype=torch.int64, device=feat.device)
         g_prob = _zeros_strided_like(est_dens)
-        qs = g_pn_q.stride()                                 # contiguous [V,T,fh,fw]
-        if (qs[0], qs[2], qs[3], qs[1]) != (sv, sy, sx, st):
+        if g_pn_q.stride() != est_depth.stride():           # g_pn_q: contiguous [V,T,fh,fw]
             raise ValueError("the deterministic backward needs contiguous [V,T,H,W] hypotheses")
-        _lib.call("mvsd_backproject_bwd_det", g_mem.data_ptr(),
-                  CHANNELS_FIRST if channels_first else CHANNELS_LAST, count.data_ptr(),
-                  feat.data_ptr(), _code(feat.dtype), fh, fw, points.data_ptr(), projection.data_ptr(),
-                  est_depth.data_ptr(), est_dens.data_ptr(), sv, sy, sx, st, float(vs_z),
-                  acc.data_ptr(), g_pn_q.data_ptr(), v, c, h, w, t, n, _stream())
-        g_pn = fixed_to_float(g_pn_q)
-        _lib.call("mvsd_prob_norm_bwd", est_dens.data_ptr(), g_pn.data_ptr(), g_prob.data_ptr(),
-                  sv, sy, sx, st, v, h, w, t, _stream())
+        _lib.backproject_bwd_det(g_mem, count, feat, points, projection, est_depth, est_dens, acc, g_pn_q,
+                                 vs_z=vs_z, height=h, width=w, channels_first=channels_first)
+        _lib.prob_norm_bwd(est_dens, fixed_to_float(g_pn_q), g_prob, height=h, width=w)
         return None, g_prob
-    g_feat = acc if acc is not None else _zeros_nhwc(v, c, fh, fw, torch.float32, feat.device)
+    g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
     g_pn = _zeros_strided_like(est_dens)
     g_prob = _zeros_strided_like(est_dens)
-    _lib.call("mvsd_backproject_bwd", g_mem.data_ptr(),
-              CHANNELS_FIRST if channels_first else CHANNELS_LAST, mode,
-              count.data_ptr() if mode == BP_MEAN else None,
-              feat.data_ptr(), _code(feat.dtype), fh, fw, points.data_ptr(),
-              projection.data_ptr(), est_depth.data_ptr(), est_dens.data_ptr(),
-              sv, sy, sx, st, float(vs_z), g_feat.data_ptr(), g_pn.data_ptr(),
-              v, c, h, w, t, n, _stream())
-    _lib.call("mvsd_prob_norm_bwd", est_dens.data_ptr(), g_pn.data_ptr(), g_prob.data_ptr(),
-              sv, sy, sx, st, v, h, w, t, _stream())
-    if acc is not None:
-        return None, g_prob
-    g_feat = g_feat if feat.dtype == torch.float32 else g_feat.to(feat.dtype)
-    return g_feat, g_prob
-
-
-def ctx_count_is_external(count, out) -> bool:
-    """True when the back-projection wrote into caller-owned buffers (``out=`` / ``count_out=``)."""
-    return out is not None
+    _lib.backproject_bwd(g_mem, feat, points, projection, est_depth, est_dens, g_feat, g_pn, vs_z=vs_z,
+                         mode=mode, height=h, width=w, channels_first=channels_first,
+                         count=count if mode == BP_MEAN else None)
+    _lib.prob_norm_bwd(est_dens, g_pn, g_prob, height=h, width=w)
+    return (None if acc is not None else g_feat.to(feat.dtype)), g_prob
 
 
 class _BackprojectAggregate(torch.autograd.Function):
@@ -736,7 +637,6 @@ class _BackprojectAggregate(torch.autograd.Function):
         external = out is not None or count is not None
         res, count = _bp_fwd_raw(feat, points, projection, est_depth, est_dens, vs_z, h, w, mode,
                                  channels_first, out, count)
-        out = res if external else None
         # Only MEAN mode needs the count in its backward (s_u = 1/(count+1e-8)); SUM mode saves
         # nothing that aliases caller-owned (reused, peer-mapped) buffers, so a later call that
         # overwrites them cannot corrupt this graph.
@@ -744,7 +644,7 @@ class _BackprojectAggregate(torch.autograd.Function):
         # backward keeps its own copy (N int32 = 100 KB): a later writer cannot change s_u.
         keep = None
         if mode == BP_MEAN:
-            keep = count.clone() if ctx_count_is_external(count, out) else count
+            keep = count.clone() if external else count
         ctx.save_for_backward(feat, points, projection, est_depth, est_dens, keep)
         ctx.consts = (float(vs_z), h, w, mode, channels_first)
         ctx.sink = sink
@@ -769,6 +669,23 @@ def _check_hyp(name, t, v, fh, fw):
         raise ValueError(f"{name} must be float32")
 
 
+def _check_bp(feat, points, projection, est_depth, est_dens, height, width, grad_sink=None) -> None:
+    _need_cuda("feat", feat)
+    if not _is_nhwc(feat):
+        raise ValueError("feat must be channels_last; use ops.pack_features")
+    v, _, fh, fw = feat.shape
+    _check_hyp("est_depth", est_depth, v, fh, fw)
+    _check_hyp("est_dens", est_dens, v, fh, fw)
+    _need_cuda("points", points)
+    _need_cuda("projection", projection)
+    if tuple(projection.shape) != (v, 3, 4):
+        raise ValueError("projection must be [V,3,4]")
+    if height > fh or width > fw:
+        raise ValueError("crop exceeds the feature map")
+    if grad_sink is not None and grad_sink.shape != tuple(feat.shape):
+        raise ValueError("grad_sink belongs to a different feature tensor")
+
+
 def backproject_aggregate(feat, points, projection, est_depth, est_dens, vs_z: float,
                           height: int, width: int, *, mode: str = "mean",
                           channels_first: bool = True, out: Optional[torch.Tensor] = None,
@@ -790,45 +707,33 @@ def backproject_aggregate(feat, points, projection, est_depth, est_dens, vs_z: f
     (mvsdet.py:695).  The buffers are overwritten in place without bumping autograd's version
     counters; the backward keeps a private copy of the count, so reusing the buffers later cannot
     corrupt this graph -- but the VALUES handed back are the buffers themselves."""
-    _need_cuda("feat", feat)
-    if not _is_nhwc(feat):
-        raise ValueError("feat must be channels_last; use ops.pack_features")
-    v, c, fh, fw = feat.shape
-    _check_hyp("est_depth", est_depth, v, fh, fw)
-    _check_hyp("est_dens", est_dens, v, fh, fw)
+    _check_bp(feat, points, projection, est_depth, est_dens, height, width, grad_sink)
     if est_depth.stride() != est_dens.stride():
         est_depth, est_dens = est_depth.contiguous(), est_dens.contiguous()
-    _need_cuda("points", points)
-    _need_cuda("projection", projection)
-    if tuple(projection.shape) != (v, 3, 4):
-        raise ValueError("projection must be [V,3,4]")
-    if height > fh or width > fw:
-        raise ValueError("crop exceeds the feature map")
     m = {"mean": BP_MEAN, "sum": BP_SUM}[mode]
-    if grad_sink is not None and grad_sink.shape != tuple(feat.shape):
-        raise ValueError("grad_sink belongs to a different feature tensor")
     return _BackprojectAggregate.apply(feat, points.contiguous().float(),
                                        projection.contiguous().float(), est_depth, est_dens,
                                        float(vs_z), int(height), int(width), m, bool(channels_first),
                                        out, count_out, grad_sink)
 
 
+def _per_view_hyp(t, h, w):
+    """[V, h*w, 1, T] -> the [V,T,h,w] view the kernels take"""
+    return t.view(t.shape[0], h, w, t.shape[3]).permute(0, 3, 1, 2)
+
+
 class _BackprojectPerView(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, feat, points, projection, depth, prob, vs_z, h, w, strides):
-        v, c, fh, fw = feat.shape
+    def forward(ctx, feat, points, projection, depth, prob, vs_z, h, w):
+        v, c = feat.shape[:2]
         n = points.numel() // 3
-        t = strides[4]
         dev = feat.device
         out = torch.zeros((v, n, c), dtype=torch.float32, device=dev)
         valid = torch.empty((v, n), dtype=torch.uint8, device=dev)
-        _lib.call("mvsd_backproject_fwd", feat.data_ptr(), _code(feat.dtype), fh, fw,
-                  points.data_ptr(), projection.data_ptr(), depth.data_ptr(), prob.data_ptr(),
-                  strides[0], strides[1], strides[2], strides[3], float(vs_z), BP_PER_VIEW,
-                  out.data_ptr(), CHANNELS_LAST, None, valid.data_ptr(), None,
-                  v, c, h, w, t, n, _stream())
+        _lib.backproject_fwd(feat, points, projection, _per_view_hyp(depth, h, w), _per_view_hyp(prob, h, w),
+                             out.permute(0, 2, 1), vs_z=vs_z, mode=BP_PER_VIEW, height=h, width=w, valid=valid)
         ctx.save_for_backward(feat, points, projection, depth, prob)
-        ctx.consts = (float(vs_z), h, w, strides)
+        ctx.consts = (float(vs_z), h, w)
         valid = valid.bool()
         ctx.mark_non_differentiable(valid)
         return out.permute(0, 2, 1), valid
@@ -836,23 +741,16 @@ class _BackprojectPerView(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_out, _g_valid):
         feat, points, projection, depth, prob = ctx.saved_tensors
-        vs_z, h, w, strides = ctx.consts
-        v, c, fh, fw = feat.shape
-        n = points.numel() // 3
-        t = strides[4]
-        g_mem = g_out.float().permute(0, 2, 1).contiguous()
-        g_feat = _zeros_nhwc(v, c, fh, fw, torch.float32, feat.device)
+        vs_z, h, w = ctx.consts
+        g_mem = g_out.float().permute(0, 2, 1).contiguous().permute(0, 2, 1)
+        g_feat = _zeros_nhwc(*feat.shape, torch.float32, feat.device)
         g_pn = _zeros_strided_like(prob)
         g_prob = _zeros_strided_like(prob)
-        _lib.call("mvsd_backproject_bwd", g_mem.data_ptr(), CHANNELS_LAST, BP_PER_VIEW, None,
-                  feat.data_ptr(), _code(feat.dtype), fh, fw, points.data_ptr(),
-                  projection.data_ptr(), depth.data_ptr(), prob.data_ptr(),
-                  strides[0], strides[1], strides[2], strides[3], vs_z, g_feat.data_ptr(),
-                  g_pn.data_ptr(), v, c, h, w, t, n, _stream())
-        _lib.call("mvsd_prob_norm_bwd", prob.data_ptr(), g_pn.data_ptr(), g_prob.data_ptr(),
-                  strides[0], strides[1], strides[2], strides[3], v, h, w, t, _stream())
-        g_feat = g_feat if feat.dtype == torch.float32 else g_feat.to(feat.dtype)
-        return g_feat, None, None, None, g_prob, None, None, None, None
+        prob_t = _per_view_hyp(prob, h, w)
+        _lib.backproject_bwd(g_mem, feat, points, projection, _per_view_hyp(depth, h, w), prob_t, g_feat, g_pn,
+                             vs_z=vs_z, mode=BP_PER_VIEW, height=h, width=w)
+        _lib.prob_norm_bwd(prob_t, g_pn, g_prob, height=h, width=w)
+        return g_feat.to(feat.dtype), None, None, None, g_prob, None, None, None
 
 
 def backproject_per_view(feat, points, projection, depth, prob, vs_z: float, height: int,
@@ -874,30 +772,21 @@ def backproject_per_view(feat, points, projection, depth, prob, vs_z: float, hei
     if depth.shape[2] != 1 or depth.stride() != prob.stride():
         depth = depth.reshape(v, height * width, 1, t).contiguous()
         prob = prob.reshape(v, height * width, 1, t).contiguous()
-    sv, sp, _, st = depth.stride()
-    strides = (sv, sp * width, sp, st, t)
     return _BackprojectPerView.apply(feat, points.contiguous().float(),
                                      projection.contiguous().float(), depth, prob, float(vs_z),
-                                     int(height), int(width), strides)
+                                     int(height), int(width))
 
 
 def voxel_normalize(volume_sum: torch.Tensor, count: torch.Tensor) -> torch.Tensor:
     """sum / (count + 1e-8), zero where count == 0 (mvsdet.py:514-515) for a
     [C,N] (either memory order) partial sum after the multi-GPU all-reduce."""
     _need_cuda("volume_sum", volume_sum)
-    c, n = volume_sum.shape
-    if volume_sum.is_contiguous():
-        out = torch.empty_like(volume_sum)
-        _lib.call("mvsd_voxel_normalize", volume_sum.data_ptr(), count.data_ptr(), out.data_ptr(),
-                  CHANNELS_FIRST, c, n, _stream())
-        return out
-    mem = volume_sum.t()
-    if not mem.is_contiguous():
+    channels_first = volume_sum.is_contiguous()
+    if not channels_first and not volume_sum.t().is_contiguous():
         raise ValueError("volume_sum must be [C,N] contiguous or the transpose of [N,C]")
-    out = torch.empty_like(mem)
-    _lib.call("mvsd_voxel_normalize", mem.data_ptr(), count.data_ptr(), out.data_ptr(),
-              CHANNELS_LAST, c, n, _stream())
-    return out.t()
+    out = torch.empty_like(volume_sum)          # same memory order
+    _lib.voxel_normalize(volume_sum, count, out, channels_first=channels_first)
+    return out
 
 
 # --------------------------------------------------------------------------
@@ -916,13 +805,10 @@ def scene_setup(w2c: torch.Tensor, k_feat: torch.Tensor, ref_proj: torch.Tensor,
             raise ValueError(f"{n} must be contiguous float32")
     v = w2c.shape[0]
     n_ref = v - ref_begin if n_ref is None else int(n_ref)
-    per_view = int(k_feat.dim() == 3)
     dev = w2c.device
     out = torch.empty(n_ref * k * 13 + n_ref * 12, dtype=torch.float32, device=dev)
     nbr = out[:n_ref * k].view(torch.int32).view(n_ref, k)
     hom = out[n_ref * k:n_ref * k * 13].view(n_ref, k, 12)
     proj = out[n_ref * k * 13:].view(n_ref, 3, 4)
-    _lib.call("mvsd_scene_setup", w2c.data_ptr(), k_feat.data_ptr(), per_view, ref_proj.data_ptr(),
-              inv_ref.data_ptr(), _ptr(nbr) if k else None, _ptr(hom) if k else None, proj.data_ptr(),
-              v, int(k), int(ref_begin), n_ref, _stream())
+    _lib.scene_setup(w2c, k_feat, ref_proj, inv_ref, nbr, hom, proj, ref_begin=int(ref_begin))
     return nbr, hom, proj

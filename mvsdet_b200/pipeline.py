@@ -29,15 +29,11 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib
-from ._lib import BF16, BP_MEAN, CHANNELS_FIRST, CHANNELS_LAST, F32
+from ._lib import BP_MEAN
 from .geometry import SceneGeometry
 from .scene import SceneConfig
 
 __all__ = ["ScenePipeline"]
-
-
-def _code(dtype):
-    return BF16 if dtype == torch.bfloat16 else F32
 
 
 class ScenePipeline:
@@ -79,6 +75,11 @@ class ScenePipeline:
         self.count = torch.empty((n,), dtype=torch.int32, device=dev)
         self.g_feature = torch.empty((v, c, hf, wf), **f32)
         self.g_cost_out = torch.empty((v, 2, d, hf, wf), **f32)
+        # the logical [V,C,H,W] / [V,C,D,H,W] views of the channels-last buffers the kernels take
+        self._feat = self.feat_cl.permute(0, 3, 1, 2)
+        self._g_feat = self.g_feat_cl.permute(0, 3, 1, 2)
+        self._variance = self.variance.permute(0, 4, 1, 2, 3)
+        self._g_variance = self.g_variance.permute(0, 4, 1, 2, 3)
         self.geo: Optional[SceneGeometry] = None
         self._host = None
         self._side = torch.cuda.Stream(device=dev)     # zero-fills of the gradient accumulators
@@ -132,23 +133,34 @@ class ScenePipeline:
         if geo is None:
             raise RuntimeError("set_geometry() first")
         cfg = self.cfg
-        v, c, d, t, k = cfg.n_views, cfg.channels, cfg.num_depth, cfg.topk, geo.k
-        hf, wf = cfg.feat_hw
         h, w = geo.height, geo.width
-        n = self.count.numel()
-        st = torch.cuda.current_stream().cuda_stream
-        fdt, vdt = _code(self.feature_dtype), _code(self.variance_dtype)
-        sv, s_t, sy, sx = self.est_depth.stride()
+        near, interval = cfg.near_far_range[0], cfg.depth_interval
+        sweep = (self._feat, geo.neighbor_ids, geo.hom, geo.depth_values)
+        hyp = (self._feat, geo.points, geo.projection, self.est_depth, self.est_dens)
+        bp = dict(vs_z=cfg.voxel_size[2], mode=BP_MEAN, height=h, width=w, channels_first=True, count=self.count)
 
-        def run(name, *args):
+        def run(name, launch, *args, **kwargs):
             if timers is None:
-                _lib.call(*args)
+                launch(*args, **kwargs)
                 return
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            _lib.call(*args)
+            launch(*args, **kwargs)
             e1.record()
             timers.setdefault(name, []).append((e0, e1))
+
+        def small_kernels():
+            with torch.cuda.stream(aux):
+                run("depth_topk_fwd", _lib.depth_topk_fwd, self.cost_out, self.prob_volume, self.off_pred,
+                    self.est_depth, self.est_dens, self.est_idx, self.depth_coding, near=near, interval=interval)
+                run("backproject_fwd", _lib.backproject_fwd, *hyp, self.volume_mean, **bp)
+                # ---- backward
+                aux.wait_stream(self._side)
+                run("backproject_bwd", _lib.backproject_bwd, self.g_volume_mean, *hyp, self._g_feat, self.g_pn, **bp)
+                run("prob_norm_bwd", _lib.prob_norm_bwd, self.est_dens, self.g_pn, self.g_est_dens, height=h,
+                    width=w)
+                run("depth_topk_bwd", _lib.depth_topk_bwd, self.cost_out, self.est_idx, None, None, None,
+                    self.g_est_dens, None, self.g_cost_out, near=near, interval=interval)
 
         # Three streams (fork/join edges once the step is captured into a graph):
         #   cur    pack -> sweep fwd -> sweep bwd -> unpack      (the two 1.2 GB streaming kernels)
@@ -162,8 +174,7 @@ class ScenePipeline:
         overlap = timers is None and self.overlap_small
         aux = self._aux if overlap else cur
         if self.pack_input:
-            run("pack", "mvsd_pack_nchw_to_nhwc", self.feature.data_ptr(), self.feat_cl.data_ptr(),
-                fdt, v, c, hf, wf, st)
+            run("pack", _lib.pack, self.feature, self._feat)
         # the fills start after the pack (which is HBM-bound on its own: 0.029 ms alone, 0.045 ms
         # next to a 98 MB memset) and run under the forward sweep instead
         self._side.wait_stream(cur)
@@ -172,49 +183,16 @@ class ScenePipeline:
             self.g_pn.zero_()
         if overlap:
             aux.wait_stream(cur)
-        else:
-            run("plane_sweep_fwd", "mvsd_plane_sweep_fwd", self.feat_cl.data_ptr(), fdt,
-                geo.neighbor_ids.data_ptr(), geo.hom.data_ptr(), geo.depth_values.data_ptr(),
-                self.variance.data_ptr(), vdt, CHANNELS_LAST, v, c, d, hf, wf, k, 0, v, st)
-        sc = self.cost_out.stride()
-        with torch.cuda.stream(aux):
-            sa = aux.cuda_stream
-            run("depth_topk_fwd", "mvsd_depth_topk_fwd", self.cost_out.data_ptr(), sc[0], sc[1], sc[2],
-                sc[4], self.prob_volume.data_ptr(), self.off_pred.data_ptr(), self.est_depth.data_ptr(),
-                self.est_dens.data_ptr(), self.est_idx.data_ptr(), self.depth_coding.data_ptr(),
-                None, 0, None, None, None, None,
-                float(cfg.near_far_range[0]), float(cfg.depth_interval), 0, v, d, hf, wf, t, sa)
-            run("backproject_fwd", "mvsd_backproject_fwd", self.feat_cl.data_ptr(), fdt, hf, wf,
-                geo.points.data_ptr(), geo.projection.data_ptr(), self.est_depth.data_ptr(),
-                self.est_dens.data_ptr(), sv, sy, sx, s_t, float(cfg.voxel_size[2]), BP_MEAN,
-                self.volume_mean.data_ptr(), CHANNELS_FIRST, self.count.data_ptr(), None, None,
-                v, c, h, w, t, n, sa)
-            # ---- backward
-            aux.wait_stream(self._side)
-            run("backproject_bwd", "mvsd_backproject_bwd", self.g_volume_mean.data_ptr(), CHANNELS_FIRST,
-                BP_MEAN, self.count.data_ptr(), self.feat_cl.data_ptr(), fdt, hf, wf,
-                geo.points.data_ptr(), geo.projection.data_ptr(), self.est_depth.data_ptr(),
-                self.est_dens.data_ptr(), sv, sy, sx, s_t, float(cfg.voxel_size[2]),
-                self.g_feat_cl.data_ptr(), self.g_pn.data_ptr(), v, c, h, w, t, n, sa)
-            run("prob_norm_bwd", "mvsd_prob_norm_bwd", self.est_dens.data_ptr(), self.g_pn.data_ptr(),
-                self.g_est_dens.data_ptr(), sv, sy, sx, s_t, v, h, w, t, sa)
-            run("depth_topk_bwd", "mvsd_depth_topk_bwd", self.cost_out.data_ptr(), sc[0], sc[1], sc[2],
-                sc[4], self.est_idx.data_ptr(), None, None, None, self.g_est_dens.data_ptr(), None,
-                None, 0, None, None,
-                self.g_cost_out.data_ptr(), float(cfg.near_far_range[0]), float(cfg.depth_interval), 0,
-                v, d, hf, wf, t, sa)
+            small_kernels()
+        run("plane_sweep_fwd", _lib.plane_sweep_fwd, *sweep, self._variance)
         if overlap:
-            run("plane_sweep_fwd", "mvsd_plane_sweep_fwd", self.feat_cl.data_ptr(), fdt,
-                geo.neighbor_ids.data_ptr(), geo.hom.data_ptr(), geo.depth_values.data_ptr(),
-                self.variance.data_ptr(), vdt, CHANNELS_LAST, v, c, d, hf, wf, k, 0, v, st)
             cur.wait_stream(self._side)
-        run("plane_sweep_bwd", "mvsd_plane_sweep_bwd", self.g_variance.data_ptr(), vdt, CHANNELS_LAST,
-            self.feat_cl.data_ptr(), fdt, geo.neighbor_ids.data_ptr(), geo.hom.data_ptr(),
-            geo.depth_values.data_ptr(), self.g_feat_cl.data_ptr(), v, c, d, hf, wf, k, 0, v, st)
+        else:
+            small_kernels()
+        run("plane_sweep_bwd", _lib.plane_sweep_bwd, self._g_variance, *sweep, self._g_feat)
         if overlap:
             cur.wait_stream(aux)
-        run("unpack", "mvsd_unpack_nhwc_to_nchw", self.g_feat_cl.data_ptr(), self.g_feature.data_ptr(),
-            0, v, c, hf, wf, st)
+        run("unpack", _lib.unpack, self._g_feat, self.g_feature)
 
     # ------------------------------------------------------------------
     def capture(self) -> "torch.cuda.CUDAGraph":

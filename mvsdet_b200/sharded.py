@@ -35,7 +35,8 @@ from typing import Callable, Dict, List, Optional, Tuple
 import torch
 import torch.distributed as dist
 
-from ._lib import CHANNELS_FIRST, CHANNELS_LAST
+from . import _lib, ops
+from ._lib import BP_MEAN, BP_SUM
 
 __all__ = ["partition_views", "halo_views", "halo_pull_table", "halo_counts", "pose_order", "permute_img_meta",
            "pack_partials", "unpack_partials", "allreduce_partials", "LocalGeometry", "ShardedSceneForward",
@@ -234,7 +235,6 @@ class P2PVoxelReducer:
         return self.part[:self.total].view(shape), self.part[self.total:].view(torch.int32)
 
     def __call__(self, volume_sum: torch.Tensor, count: torch.Tensor):
-        from . import _lib
         mem = volume_sum if volume_sum.is_contiguous() else volume_sum.t()
         if not mem.is_contiguous() or mem.numel() != self.total:
             raise ValueError("volume_sum must be [C,N] contiguous or the transpose of a contiguous [N,C]")
@@ -242,10 +242,8 @@ class P2PVoxelReducer:
             self.part[:self.total].copy_(mem.reshape(-1))
             self.part[self.total:].view(torch.int32).copy_(count.reshape(-1))
         self.h_part.barrier(channel=0)          # every rank's partials are complete and visible
-        _lib.call("mvsd_voxel_reduce_p2p", self.h_part.buffer_ptrs_dev, self.h_out.buffer_ptrs_dev,
-                  self.count_local.data_ptr(), self.world, self.rank,
-                  CHANNELS_FIRST if self.cfirst else CHANNELS_LAST, self.c, self.n,
-                  torch.cuda.current_stream().cuda_stream)
+        _lib.voxel_reduce_p2p(self.h_part.buffer_ptrs_dev, self.h_out.buffer_ptrs_dev, self.count_local,
+                              world=self.world, rank=self.rank, channels=self.c, channels_first=self.cfirst)
         self.h_out.barrier(channel=0)           # every rank's slice has landed in every out buffer
         vol = self.out[:self.total]
         vol = vol.view(self.c, self.n) if self.cfirst else vol.view(self.n, self.c).t()
@@ -291,23 +289,19 @@ class ShardedSceneForward:
     def _pack_local(self, feature: torch.Tensor, lg: LocalGeometry) -> torch.Tensor:
         """fp32 NCHW [V,C,H,W] -> channels-last buffer of the views in ``lg.views``
         (contiguous runs of views go through one transpose launch each)."""
-        from . import _lib, ops
         v, c, h, w = feature.shape
         dt = self.hot.feature_dtype
         if feature.dtype != torch.float32 or not feature.is_contiguous():
             return ops.pack_features(feature[lg.views], dt)       # already channels-last / bf16 inputs
-        out = torch.empty((len(lg.views), h, w, c), dtype=dt, device=feature.device)
-        code = _lib.BF16 if dt == torch.bfloat16 else _lib.F32
-        st = torch.cuda.current_stream().cuda_stream
+        out = ops._empty_nhwc(len(lg.views), c, h, w, dt, feature.device)
         i = 0
         while i < len(lg.views):
             j = i
             while j + 1 < len(lg.views) and lg.views[j + 1] == lg.views[j] + 1:
                 j += 1
-            _lib.call("mvsd_pack_nchw_to_nhwc", feature[lg.views[i]].data_ptr(), out[i].data_ptr(), code,
-                      j - i + 1, c, h, w, st)
+            _lib.pack(feature[lg.views[i]:lg.views[j] + 1], out[i:j + 1])
             i = j + 1
-        return out.permute(0, 3, 1, 2)
+        return out
 
     def local_partials(self, feature: torch.Tensor, img_meta: dict, cost_net: Callable,
                        geometry: Optional[LocalGeometry] = None, rank_world: Optional[Tuple[int, int]] = None,
@@ -315,7 +309,6 @@ class ShardedSceneForward:
         """This rank's contribution before the collective: (volume_sum logical
         [C,N], count int32 [N], (begin, end)).  ``rank_world`` overrides the
         process group (used by the single-GPU tests to play every rank)."""
-        from . import ops
         hot = self.hot
         rank, world = rank_world or self._world()
         v_all = feature.shape[0]
@@ -352,7 +345,6 @@ class ShardedSceneForward:
 
     def __call__(self, feature: torch.Tensor, img_meta: dict,
                  cost_regularization: Optional[Callable] = None, geometry=None) -> Dict[str, torch.Tensor]:
-        from . import ops
         hot = self.hot
         cost_net = cost_regularization or hot.cost_regularization
         if cost_net is None:
@@ -406,24 +398,18 @@ class ShardedScenePipeline:
 
     def __init__(self, hot_path, cfg, device, group=None):
         import torch.distributed._symmetric_memory as symm
-        from . import _lib
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("ShardedScenePipeline needs an initialised process group")
         self.hot, self.cfg, self.device = hot_path, cfg, torch.device(device)
         self.group = group if group is not None else dist.group.WORLD
         self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
-        self._lib = _lib
         self._symm = symm
         self.c = cfg.channels
         self.n = cfg.n_voxels[0] * cfg.n_voxels[1] * cfg.n_voxels[2]
-        self.total = self.c * self.n
         dev = self.device
-        self.part = [symm.empty(self.total + self.n, dtype=torch.float32, device=dev) for _ in range(2)]
-        self.out = [symm.empty(self.total + self.n, dtype=torch.float32, device=dev) for _ in range(2)]
-        self.h_part = [symm.rendezvous(t, self.group) for t in self.part]
-        self.h_out = [symm.rendezvous(t, self.group) for t in self.out]
-        self.count_local = [torch.empty(self.n, dtype=torch.int32, device=dev) for _ in range(2)]
-        self.nccl_out = [torch.empty(self.total, dtype=torch.float32, device=dev) for _ in range(2)]
+        # per slot: the peer-mapped partial and result buffers and the p2p combine over them
+        self._red = [P2PVoxelReducer(self.c, self.n, True, dev, self.group) for _ in range(2)]
+        self.nccl_out = [torch.empty(self.c * self.n, dtype=torch.float32, device=dev) for _ in range(2)]
         # higher priority: the combine's barrier / reduce CTAs are dispatched as soon as SM slots free up,
         # ahead of the next scene's queued sweep CTAs (at equal priority they wait for the sweep's last wave)
         self.s_comm = torch.cuda.Stream(device=dev, priority=-1)
@@ -469,8 +455,8 @@ class ShardedScenePipeline:
         f32 = dict(dtype=torch.float32, device=dev)
         self.feature = feature[[order[i] for i in views]].to(dev, dtype=torch.float32).contiguous()
         self.cost_out = cost_out[order[begin:end]].to(dev, dtype=torch.float32).contiguous()
-        self.feat_cl = torch.empty((vl, hf, wf, self.c), dtype=hot.feature_dtype, device=dev)
-        self.variance = torch.empty((vb, d, hf, wf, self.c), dtype=hot.variance_dtype, device=dev)
+        self.feat_cl = ops._empty_nhwc(vl, self.c, hf, wf, hot.feature_dtype, dev)
+        self.variance = ops._empty_ndhwc(vb, self.c, d, hf, wf, hot.variance_dtype, dev)
         self.est_depth = torch.empty((vb, t, hf, wf), **f32)
         self.est_dens = torch.empty((vb, t, hf, wf), **f32)
         self.est_idx = torch.empty((vb, t, hf, wf), dtype=torch.int64, device=dev)
@@ -480,32 +466,17 @@ class ShardedScenePipeline:
         self._bwd_graphs = {}
         torch.cuda.synchronize(dev)
 
-    def _code(self, dtype):
-        return self._lib.BF16 if dtype == torch.bfloat16 else self._lib.F32
-
     def _enqueue_compute(self, slot: int) -> None:
-        """pack -> sweep -> top-k -> back-projection(SUM) into part[slot]; current stream; capturable."""
-        lib, cfg, lg, geo = self._lib, self.cfg, self.lg, self.lg.geo
-        st = torch.cuda.current_stream().cuda_stream
-        vl, vb, c = self.vl, self.vb, self.c
-        d, t, k = cfg.num_depth, cfg.topk, geo.k
-        hf, wf = cfg.feat_hw
-        fdt, vdt = self._code(self.hot.feature_dtype), self._code(self.hot.variance_dtype)
-        lib.call("mvsd_pack_nchw_to_nhwc", self.feature.data_ptr(), self.feat_cl.data_ptr(), fdt, vl, c, hf, wf, st)
-        lib.call("mvsd_plane_sweep_fwd", self.feat_cl.data_ptr(), fdt, lg.neighbor_ids_local.data_ptr(),
-                 geo.hom.data_ptr(), geo.depth_values.data_ptr(), self.variance.data_ptr(), vdt,
-                 CHANNELS_LAST, vb, c, d, hf, wf, k, 0, vl, st)
-        sc = self.cost_out.stride()
-        lib.call("mvsd_depth_topk_fwd", self.cost_out.data_ptr(), sc[0], sc[1], sc[2], sc[4], None, None,
-                 self.est_depth.data_ptr(), self.est_dens.data_ptr(), self.est_idx.data_ptr(), None,
-                 None, 0, None, None, None, None, float(cfg.near_far_range[0]), float(cfg.depth_interval), 0,
-                 vb, d, hf, wf, t, st)
-        sv, s_t, sy, sx = self.est_depth.stride()
-        part = self.part[slot]
-        lib.call("mvsd_backproject_fwd", self.feat_cl.data_ptr(), fdt, hf, wf, geo.points.data_ptr(),
-                 geo.projection.data_ptr(), self.est_depth.data_ptr(), self.est_dens.data_ptr(), sv, sy, sx, s_t,
-                 float(cfg.voxel_size[2]), self._lib.BP_SUM, part.data_ptr(), CHANNELS_FIRST,
-                 part[self.total:].data_ptr(), None, None, vb, c, geo.height, geo.width, t, self.n, st)
+        """pack -> sweep -> top-k -> back-projection(SUM) into the slot's partials; current stream; capturable."""
+        cfg, lg, geo = self.cfg, self.lg, self.lg.geo
+        _lib.pack(self.feature, self.feat_cl)
+        _lib.plane_sweep_fwd(self.feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self.variance)
+        _lib.depth_topk_fwd(self.cost_out, None, None, self.est_depth, self.est_dens, self.est_idx, None,
+                            near=cfg.near_far_range[0], interval=cfg.depth_interval)
+        vol_sum, count = self._red[slot].partial_buffers()
+        _lib.backproject_fwd(self.feat_cl, geo.points, geo.projection, self.est_depth, self.est_dens, vol_sum,
+                             vs_z=cfg.voxel_size[2], mode=BP_SUM, height=geo.height, width=geo.width,
+                             channels_first=True, count=count)
 
     def _compute(self, slot: int, use_graph: bool = True) -> None:
         if not use_graph:
@@ -526,27 +497,20 @@ class ShardedScenePipeline:
 
     def _combine(self, slot: int, mode: str) -> Dict[str, torch.Tensor]:
         """sum over ranks + normalise, on the current stream -> views of this slot's result buffers"""
-        c, n, total = self.c, self.n, self.total
+        c, n = self.c, self.n
         nx, ny, nz = self.cfg.n_voxels
-        st = torch.cuda.current_stream().cuda_stream
+        red = self._red[slot]
         if mode == "p2p":
-            self.h_part[slot].barrier(channel=0)
-            self._lib.call("mvsd_voxel_reduce_p2p", self.h_part[slot].buffer_ptrs_dev,
-                           self.h_out[slot].buffer_ptrs_dev, self.count_local[slot].data_ptr(), self.world,
-                           self.rank, CHANNELS_FIRST, c, n, st)
-            self.h_out[slot].barrier(channel=0)
-            vol = self.out[slot][:total].view(c, nx, ny, nz)
-            count = self.out[slot][total:].view(torch.int32)
+            vol, count = red(*red.partial_buffers())
+            vol = vol.view(c, nx, ny, nz)
         elif mode == "nccl":
-            part = self.part[slot]
-            dist.all_reduce(part[:total], op=dist.ReduceOp.SUM, group=self.group)
-            cnt = part[total:].view(torch.int32)
+            vol_sum, cnt = red.partial_buffers()
+            dist.all_reduce(vol_sum, op=dist.ReduceOp.SUM, group=self.group)
             dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=self.group)
-            self.count_local[slot].copy_(cnt)
-            self._lib.call("mvsd_voxel_normalize", part.data_ptr(), cnt.data_ptr(),
-                           self.nccl_out[slot].data_ptr(), CHANNELS_FIRST, c, n, st)
+            red.count_local.copy_(cnt)
+            _lib.voxel_normalize(vol_sum, cnt, self.nccl_out[slot].view(c, n), channels_first=True)
             vol = self.nccl_out[slot].view(c, nx, ny, nz)
-            count = self.count_local[slot]
+            count = red.count_local
         else:
             raise ValueError("mode must be 'p2p' or 'nccl'")
         return dict(volume_mean=vol, count=count, valid=count.view(1, nx, ny, nz),
@@ -592,13 +556,11 @@ class ShardedScenePipeline:
         ``g_variance`` logical [Vb,C,D,Hf,Wf] in channels_last_3d for this rank's reference views (rows in
         the order of ``self.view_ids``).
         -> (g_feature [Vb,C,Hf,Wf] fp32 for the rank's own views ``self.view_ids``, g_cost_out [Vb,2,D,Hf,Wf])."""
-        lib, cfg, lg, geo = self._lib, self.cfg, self.lg, self.lg.geo
+        cfg, lg, geo = self.cfg, self.lg, self.lg.geo
         dev = self.device
-        st = torch.cuda.current_stream().cuda_stream
         vl, vb, c, n = self.vl, self.vb, self.c, self.n
-        d, t, k = cfg.num_depth, cfg.topk, geo.k
+        d, t = cfg.num_depth, cfg.topk
         hf, wf = cfg.feat_hw
-        fdt = self._code(self.hot.feature_dtype)
         if self._g_feat is None:
             view_elems = hf * wf * c
             # every rank allocates for the same (maximum) number of local views: symmetric allocation
@@ -622,31 +584,20 @@ class ShardedScenePipeline:
             """zero-fills + back-projection / prob-norm / top-k / sweep backward into the accumulator;
             current stream; capturable (no allocation, no host sync)"""
             cur = torch.cuda.current_stream()
-            count = self.count_local[slot]
-            vdt = self._code(gv.dtype)
+            hyp = (self.feat_cl, geo.points, geo.projection, self.est_depth, self.est_dens)
             self._g_feat.zero_()
             self.g_pn.zero_()
             # the three small kernels run on a higher-priority side stream under the sweep backward
             # (all of them RED into the same accumulator: the order does not matter)
             self.s_aux.wait_stream(cur)
             with torch.cuda.stream(self.s_aux):
-                sa_ = self.s_aux.cuda_stream
-                sv, s_t, sy, sx = self.est_depth.stride()
-                lib.call("mvsd_backproject_bwd", g_vol.data_ptr(), CHANNELS_FIRST, self._lib.BP_MEAN, count.data_ptr(),
-                         self.feat_cl.data_ptr(), fdt, hf, wf, geo.points.data_ptr(), geo.projection.data_ptr(),
-                         self.est_depth.data_ptr(), self.est_dens.data_ptr(), sv, sy, sx, s_t,
-                         float(cfg.voxel_size[2]), self._g_feat.data_ptr(), self.g_pn.data_ptr(), vb, c,
-                         geo.height, geo.width, t, n, sa_)
-                lib.call("mvsd_prob_norm_bwd", self.est_dens.data_ptr(), self.g_pn.data_ptr(),
-                         self.g_est_dens.data_ptr(), sv, sy, sx, s_t, vb, geo.height, geo.width, t, sa_)
-                sc = self.cost_out.stride()
-                lib.call("mvsd_depth_topk_bwd", self.cost_out.data_ptr(), sc[0], sc[1], sc[2], sc[4],
-                         self.est_idx.data_ptr(), None, None, None, self.g_est_dens.data_ptr(), None, None, 0, None,
-                         None, self.g_cost_out.data_ptr(), float(cfg.near_far_range[0]), float(cfg.depth_interval),
-                         0, vb, d, hf, wf, t, sa_)
-            lib.call("mvsd_plane_sweep_bwd", gv.data_ptr(), vdt, CHANNELS_LAST, self.feat_cl.data_ptr(), fdt,
-                     lg.neighbor_ids_local.data_ptr(), geo.hom.data_ptr(), geo.depth_values.data_ptr(),
-                     self._g_feat.data_ptr(), vb, c, d, hf, wf, k, 0, vl, cur.cuda_stream)
+                _lib.backproject_bwd(g_vol, *hyp, self._g_feat, self.g_pn, vs_z=cfg.voxel_size[2], mode=BP_MEAN,
+                                     height=geo.height, width=geo.width, channels_first=True,
+                                     count=self._red[slot].count_local)
+                _lib.prob_norm_bwd(self.est_dens, self.g_pn, self.g_est_dens, height=geo.height, width=geo.width)
+                _lib.depth_topk_bwd(self.cost_out, self.est_idx, None, None, None, self.g_est_dens, None,
+                                    self.g_cost_out, near=cfg.near_far_range[0], interval=cfg.depth_interval)
+            _lib.plane_sweep_bwd(gv, self.feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self._g_feat)
             cur.wait_stream(self.s_aux)
 
         # the local chain is replayed as one CUDA graph while the caller keeps handing in the same
@@ -673,10 +624,10 @@ class ShardedScenePipeline:
         # owners pull the halo contributions of their peers
         self._h_g.barrier(channel=0)
         if self._n_pull:
-            lib.call("mvsd_halo_reduce_p2p", self._h_g.buffer_ptrs_dev, self._pull_offs.data_ptr(),
-                     self._pull_src.data_ptr(), self.world, self.rank, vb, hf * wf * c, st)
+            _lib.halo_reduce_p2p(self._h_g.buffer_ptrs_dev, self._pull_offs, self._pull_src, world=self.world,
+                                 rank=self.rank, view_elems=hf * wf * c)
         self._h_g.barrier(channel=0)
-        lib.call("mvsd_unpack_nhwc_to_nchw", self._g_feat.data_ptr(), self.g_feature.data_ptr(), 0, vb, c, hf, wf, st)
+        _lib.unpack(self._g_feat, self.g_feature)
         return self.g_feature, self.g_cost_out
 
     def close(self) -> None:

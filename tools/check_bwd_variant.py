@@ -36,7 +36,7 @@ def run(variant, feat, geo, g):
     old = _lib.set_tuning(5, variant)
     try:
         acc = torch.zeros(feat.shape, dtype=torch.float32, device=feat.device).contiguous(memory_format=torch.channels_last)
-        ops._sweep_bwd_raw(g, feat, geo.neighbor_ids, geo.hom, geo.depth_values, 0, acc)
+        _lib.plane_sweep_bwd(g, feat, geo.neighbor_ids, geo.hom, geo.depth_values, acc)
         torch.cuda.synchronize()
     finally:
         _lib.set_tuning(5, old)
@@ -54,7 +54,7 @@ def timed(variant, feat, geo, g, reps=12):
             acc.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            ops._sweep_bwd_raw(g, feat, geo.neighbor_ids, geo.hom, geo.depth_values, 0, acc)
+            _lib.plane_sweep_bwd(g, feat, geo.neighbor_ids, geo.hom, geo.depth_values, acc)
             e1.record()
             torch.cuda.synchronize()
             ms.append(e0.elapsed_time(e1))
