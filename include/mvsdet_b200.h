@@ -26,6 +26,11 @@
  * (torch.channels_last_3d of logical [V,C,D,H,W]).  C must be a multiple of 4
  * and at most 512.  Accumulation is always fp32 (64-bit fixed point in the
  * bit-reproducible *_det forms of the two scatter backwards).
+ *
+ * Additive symbols (no ABI version change; every earlier signature is unchanged):
+ *   mvsd_plane_sweep_fwd_px, mvsd_plane_sweep_bwd_px, mvsd_plane_sweep_bwd_det_px,
+ *   mvsd_plane_sweep_groupcorr_fwd_px, mvsd_plane_sweep_groupcorr_bwd_px --
+ *   the fused sweeps with per-pixel depth hypotheses.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -153,6 +158,33 @@ int mvsd_plane_sweep_bwd_det(const void* g_out, int g_dtype, int g_layout,
                              int n_feat_views, void* stream);
 int mvsd_fixed_to_float(const int64_t* src, float* dst, int64_t n, void* stream);
 
+/* Per-pixel depth hypotheses: homo_warping's [B,D,H,W] depth_values branch
+ * (mvs_models/module.py:130-133) in the fused sweep, e.g. a narrow second sweep
+ * around the hypotheses of mvsd_depth_topk_fwd.  Same arguments and semantics as
+ * mvsd_plane_sweep_fwd / _bwd / _bwd_det, except that depth_values is
+ * [V,D,H,W] fp32 contiguous: plane d of pixel (x, y) of reference view v lies at
+ * depth_values[((v*D + d)*H + y)*W + x].  A NaN depth gives no sample.  A map
+ * that is constant per (v, d) gives the bits of the per-view call (forward and
+ * deterministic backward; the fp32-RED backward to summation order). */
+int mvsd_plane_sweep_fwd_px(const void* feat, int feat_dtype,
+                            const int32_t* nbr_ids, const float* hom,
+                            const float* depth_values,
+                            void* out, int out_dtype, int out_layout,
+                            int V, int C, int D, int H, int W, int k, int ref_begin,
+                            int n_feat_views, void* stream);
+int mvsd_plane_sweep_bwd_px(const void* g_out, int g_dtype, int g_layout,
+                            const void* feat, int feat_dtype,
+                            const int32_t* nbr_ids, const float* hom,
+                            const float* depth_values, float* g_feat,
+                            int V, int C, int D, int H, int W, int k, int ref_begin,
+                            int n_feat_views, void* stream);
+int mvsd_plane_sweep_bwd_det_px(const void* g_out, int g_dtype, int g_layout,
+                                const void* feat, int feat_dtype,
+                                const int32_t* nbr_ids, const float* hom,
+                                const float* depth_values, int64_t* g_feat_q,
+                                int V, int C, int D, int H, int W, int k, int ref_begin,
+                                int n_feat_views, void* stream);
+
 /* ---- f4: group-wise correlation cost volume over the same sweep ----------- *
  * The optional cost volume of SURVEY.md 8(f) rank 4; in the reference it is the
  * inline arithmetic of mvs_models/lss_fpn.py:485-506 (a branch no shipped config
@@ -174,6 +206,18 @@ int mvsd_plane_sweep_groupcorr_bwd(const float* g_out, const void* feat, int fea
                                    const float* depth_values, float* g_feat,
                                    int V, int C, int D, int H, int W, int k, int num_groups,
                                    int ref_begin, int n_feat_views, void* stream);
+/* The same with per-pixel depth hypotheses [V,D,H,W] fp32 contiguous
+ * (mvs_models/module.py:130-133; layout as for mvsd_plane_sweep_fwd_px). */
+int mvsd_plane_sweep_groupcorr_fwd_px(const void* feat, int feat_dtype,
+                                      const int32_t* nbr_ids, const float* hom,
+                                      const float* depth_values, float* out,
+                                      int V, int C, int D, int H, int W, int k, int num_groups,
+                                      int ref_begin, int n_feat_views, void* stream);
+int mvsd_plane_sweep_groupcorr_bwd_px(const float* g_out, const void* feat, int feat_dtype,
+                                      const int32_t* nbr_ids, const float* hom,
+                                      const float* depth_values, float* g_feat,
+                                      int V, int C, int D, int H, int W, int k, int num_groups,
+                                      int ref_begin, int n_feat_views, void* stream);
 
 /* ---- a3 alone: homo_warping (mvs_models/module.py:105-146) --------------- *
  *   src  nhwc [B,H,W,C]; hom [B,12]; out [B,D,H,W,C];

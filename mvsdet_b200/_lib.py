@@ -35,11 +35,16 @@ SIGNATURES = {
     "mvsd_plane_sweep_fwd": ([_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_bwd": ([_p, _i, _i, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_bwd_det": ([_p, _i, _i, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_fwd_px": ([_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_bwd_px": ([_p, _i, _i, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_bwd_det_px": ([_p, _i, _i, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_fixed_to_float": ([_p, _p, _l, _p], _i),
     "mvsd_backproject_bwd_det": ([_p, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _l, _l, _l, _l,
                                   _f, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_groupcorr_fwd": ([_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_groupcorr_bwd": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_groupcorr_fwd_px": ([_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_groupcorr_bwd_px": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_homo_warp_fwd": ([_p, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_homo_warp_bwd": ([_p, _i, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_depth_topk_fwd": ([_p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p,
@@ -119,11 +124,16 @@ def scene_setup(w2c, k_feat, ref_proj, inv_ref, nbr_ids, hom, projection, *, ref
          w2c.shape[0], k, ref_begin, projection.shape[0], _stream())
 
 
+def _sweep_entry(name, depth_values) -> str:
+    """the entry point for depth_values [V,D] (per-view planes) or [V,D,H,W] (per-pixel hypotheses)"""
+    return name + "_px" if depth_values.dim() == 4 else name
+
+
 def plane_sweep_fwd(feat, nbr_ids, hom, depth_values, out, *, ref_begin=0):
-    """feat [Vf,C,H,W], nbr_ids [V,k], depth_values [V,D] -> out [V,C,D,H,W]"""
+    """feat [Vf,C,H,W], nbr_ids [V,k], depth_values [V,D] or [V,D,H,W] -> out [V,C,D,H,W]"""
     vf, c, h, w = feat.shape
     v, k = nbr_ids.shape
-    call("mvsd_plane_sweep_fwd", feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(), hom.data_ptr(),
+    call(_sweep_entry("mvsd_plane_sweep_fwd", depth_values), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(), hom.data_ptr(),
          depth_values.data_ptr(), out.data_ptr(), _code(out.dtype), CHANNELS_LAST, v, c, depth_values.shape[1],
          h, w, k, ref_begin, vf, _stream())
 
@@ -131,7 +141,7 @@ def plane_sweep_fwd(feat, nbr_ids, hom, depth_values, out, *, ref_begin=0):
 def _sweep_bwd(name, g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin):
     vf, c, h, w = feat.shape
     v, k = nbr_ids.shape
-    call(name, g.data_ptr(), _code(g.dtype), CHANNELS_LAST, feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
+    call(_sweep_entry(name, depth_values), g.data_ptr(), _code(g.dtype), CHANNELS_LAST, feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
          hom.data_ptr(), depth_values.data_ptr(), g_feat.data_ptr(), v, c, depth_values.shape[1], h, w, k,
          ref_begin, vf, _stream())
 
@@ -150,7 +160,7 @@ def plane_sweep_groupcorr_fwd(feat, nbr_ids, hom, depth_values, out, *, ref_begi
     """-> fp32 out [V,k,G,D,H,W], groups innermost in memory"""
     vf, c, h, w = feat.shape
     v, k = nbr_ids.shape
-    call("mvsd_plane_sweep_groupcorr_fwd", feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(), hom.data_ptr(),
+    call(_sweep_entry("mvsd_plane_sweep_groupcorr_fwd", depth_values), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(), hom.data_ptr(),
          depth_values.data_ptr(), out.data_ptr(), v, c, depth_values.shape[1], h, w, k, out.shape[2], ref_begin,
          vf, _stream())
 
@@ -159,7 +169,7 @@ def plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, *, re
     """fp32 g laid out as the forward's out -> RED into the fp32 g_feat"""
     vf, c, h, w = feat.shape
     v, k = nbr_ids.shape
-    call("mvsd_plane_sweep_groupcorr_bwd", g.data_ptr(), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
+    call(_sweep_entry("mvsd_plane_sweep_groupcorr_bwd", depth_values), g.data_ptr(), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
          hom.data_ptr(), depth_values.data_ptr(), g_feat.data_ptr(), v, c, depth_values.shape[1], h, w, k,
          g.shape[2], ref_begin, vf, _stream())
 

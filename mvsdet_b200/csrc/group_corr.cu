@@ -44,7 +44,8 @@ __device__ __forceinline__ float lane_sum4(P4 v) {
 constexpr int kCorrPatchW = 2, kCorrPatchH = 2;
 constexpr int kCorrWarps = kCorrPatchW * kCorrPatchH, kCorrThreads = kCorrWarps * 32;
 
-template <typename TIn, int KMAX, int G, bool FULL>
+// PX (both kernels): per-pixel depth hypotheses [V,D,H,W] (the *_px entry points)
+template <typename TIn, int KMAX, int G, bool FULL, bool PX = false>
 __global__ void __launch_bounds__(kCorrThreads, 8) corr_fwd_kernel(const CorrParams q) {
   const SweepParams& p = q.s;
   __shared__ WarpSample s_tab[kCorrWarps][kSlots];
@@ -89,7 +90,7 @@ __global__ void __launch_bounds__(kCorrThreads, 8) corr_fwd_kernel(const CorrPar
   const int dc = kSlots / k;
   for (int d0 = 0; d0 < p.D; d0 += dc) {
     __syncwarp();
-    fill_samples(s_tab[warp], p, c, d0, dc, lane);
+    fill_samples<PX ? kDepthPixels : kDepthPlanes>(s_tab[warp], p, c, d0, dc, lane);
     __syncwarp();
     const int dend = min(p.D, d0 + dc);
     for (int d = d0; d < dend; ++d) {
@@ -172,7 +173,7 @@ __device__ __forceinline__ void corr_red_tap(float* dst, unsigned off, const flo
     if (group_on<FULL>(c0, g, C)) red_add_f32x4(a + 128 * g, f4scale(gw[g], w));
 }
 
-template <typename TIn, int G, bool FULL>
+template <typename TIn, int G, bool FULL, bool PX = false>
 __global__ void __launch_bounds__(kSweepThreads) corr_bwd_kernel(const CorrParams q) {
   const SweepParams& p = q.s;
   __shared__ WarpSample s_tab[kSweepWarps][kSlots];
@@ -193,7 +194,7 @@ __global__ void __launch_bounds__(kSweepThreads) corr_bwd_kernel(const CorrParam
   const int dc = kSlots / k;
   for (int d0 = 0; d0 < p.D; d0 += dc) {
     __syncwarp();
-    fill_samples(s_tab[warp], p, c, d0, dc, lane);
+    fill_samples<PX ? kDepthPixels : kDepthPlanes>(s_tab[warp], p, c, d0, dc, lane);
     __syncwarp();
     const int dend = min(p.D, d0 + dc);
     for (int d = d0; d < dend; ++d) {
@@ -244,7 +245,7 @@ static int corr_setup(const char* who, CorrParams& q, int num_groups) {
   return MVSD_OK;
 }
 
-template <bool BWD, typename TIn>
+template <bool BWD, typename TIn, bool PX>
 static int corr_launch(CorrParams& q, cudaStream_t st) {
   dim3 grid;
   const int G = sweep_groups(q.s.C);
@@ -259,9 +260,9 @@ static int corr_launch(CorrParams& q, cudaStream_t st) {
   const bool full = q.s.C % (128 * G) == 0;
 #define MVSD_CORR(GG, FU)                                                        \
   do {                                                                           \
-    if constexpr (BWD) corr_bwd_kernel<TIn, GG, FU><<<grid, kSweepThreads, 0, st>>>(q); \
-    else if (q.s.k == 2) corr_fwd_kernel<TIn, 2, GG, FU><<<grid, kCorrThreads, 0, st>>>(q); \
-    else corr_fwd_kernel<TIn, 4, GG, FU><<<grid, kCorrThreads, 0, st>>>(q);      \
+    if constexpr (BWD) corr_bwd_kernel<TIn, GG, FU, PX><<<grid, kSweepThreads, 0, st>>>(q); \
+    else if (q.s.k == 2) corr_fwd_kernel<TIn, 2, GG, FU, PX><<<grid, kCorrThreads, 0, st>>>(q); \
+    else corr_fwd_kernel<TIn, 4, GG, FU, PX><<<grid, kCorrThreads, 0, st>>>(q);  \
   } while (0)
   if (G == 2) { if (full) MVSD_CORR(2, true); else MVSD_CORR(2, false); }
   else { if (full) MVSD_CORR(1, true); else MVSD_CORR(1, false); }
@@ -272,47 +273,50 @@ static int corr_launch(CorrParams& q, cudaStream_t st) {
 
 int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st);     // plane_sweep_bwd_run.cu
 
-}  // namespace mvsd
+template <bool BWD, typename TIn>
+static int corr_launch_px(CorrParams& q, cudaStream_t st) {
+  return q.s.depth_per_pixel ? corr_launch<BWD, TIn, true>(q, st) : corr_launch<BWD, TIn, false>(q, st);
+}
 
-using namespace mvsd;
-
-extern "C" int mvsd_plane_sweep_groupcorr_fwd(const void* feat, int feat_dtype, const int32_t* nbr_ids,
-                                              const float* hom, const float* depth_values, float* out,
-                                              int V, int C, int D, int H, int W, int k, int num_groups,
-                                              int ref_begin, int n_feat_views, void* stream) {
-  if (int e = sweep_check("plane_sweep_groupcorr_fwd", V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
+// per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133)
+static int groupcorr_fwd(const char* who, const void* feat, int feat_dtype, const int32_t* nbr_ids,
+                         const float* hom, const float* depth_values, float* out, int V, int C, int D, int H,
+                         int W, int k, int num_groups, int ref_begin, int n_feat_views, bool per_pixel,
+                         void* stream) {
+  if (int e = sweep_check(who, V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
   if (!feat || !out || !depth_values || !nbr_ids || !hom)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_fwd: null pointer");
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
   if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_fwd: reference views [%d, %d) exceed the %d feature views",
-                ref_begin, ref_begin + V, n_feat_views);
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat_views);
   CorrParams q{};
   SweepParams& p = q.s;
   p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.out = out;
   p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  if (int e = corr_setup("plane_sweep_groupcorr_fwd", q, num_groups)) return e;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
+  if (int e = corr_setup(who, q, num_groups)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (feat_dtype == MVSD_F32) return corr_launch<false, float>(q, st);
-  if (feat_dtype == MVSD_BF16) return corr_launch<false, __nv_bfloat16>(q, st);
-  return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_fwd: bad dtype");
+  if (feat_dtype == MVSD_F32) return corr_launch_px<false, float>(q, st);
+  if (feat_dtype == MVSD_BF16) return corr_launch_px<false, __nv_bfloat16>(q, st);
+  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
 }
 
-extern "C" int mvsd_plane_sweep_groupcorr_bwd(const float* g_out, const void* feat, int feat_dtype,
-                                              const int32_t* nbr_ids, const float* hom,
-                                              const float* depth_values, float* g_feat, int V, int C,
-                                              int D, int H, int W, int k, int num_groups, int ref_begin,
-                                              int n_feat_views, void* stream) {
-  if (int e = sweep_check("plane_sweep_groupcorr_bwd", V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
+static int groupcorr_bwd(const char* who, const float* g_out, const void* feat, int feat_dtype,
+                         const int32_t* nbr_ids, const float* hom, const float* depth_values, float* g_feat,
+                         int V, int C, int D, int H, int W, int k, int num_groups, int ref_begin,
+                         int n_feat_views, bool per_pixel, void* stream) {
+  if (int e = sweep_check(who, V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
   if (!g_out || !feat || !g_feat || !depth_values || !nbr_ids || !hom)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_bwd: null pointer");
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
   if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_bwd: reference views [%d, %d) exceed the %d feature views",
-                ref_begin, ref_begin + V, n_feat_views);
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat_views);
   CorrParams q{};
   SweepParams& p = q.s;
   p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out; p.g_feat = g_feat;
   p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  if (int e = corr_setup("plane_sweep_groupcorr_bwd", q, num_groups)) return e;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
+  if (int e = corr_setup(who, q, num_groups)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // bf16 features, k = 2: the run-merging hand-off kernel of the variance backward with the correlation
   // algebra in its pixel body (same gather, same merged scatter); anything else (and the test hook
@@ -321,7 +325,45 @@ extern "C" int mvsd_plane_sweep_groupcorr_bwd(const float* g_out, const void* fe
     const int rc = launch_bwd_run_corr(p, feat_dtype, st);
     if (rc >= 0) return rc;
   }
-  if (feat_dtype == MVSD_F32) return corr_launch<true, float>(q, st);
-  if (feat_dtype == MVSD_BF16) return corr_launch<true, __nv_bfloat16>(q, st);
-  return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_groupcorr_bwd: bad dtype");
+  if (feat_dtype == MVSD_F32) return corr_launch_px<true, float>(q, st);
+  if (feat_dtype == MVSD_BF16) return corr_launch_px<true, __nv_bfloat16>(q, st);
+  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
+}
+
+}  // namespace mvsd
+
+using namespace mvsd;
+
+extern "C" int mvsd_plane_sweep_groupcorr_fwd(const void* feat, int feat_dtype, const int32_t* nbr_ids,
+                                              const float* hom, const float* depth_values, float* out,
+                                              int V, int C, int D, int H, int W, int k, int num_groups,
+                                              int ref_begin, int n_feat_views, void* stream) {
+  return groupcorr_fwd("plane_sweep_groupcorr_fwd", feat, feat_dtype, nbr_ids, hom, depth_values, out, V, C, D, H,
+                       W, k, num_groups, ref_begin, n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_groupcorr_fwd_px(const void* feat, int feat_dtype, const int32_t* nbr_ids,
+                                                 const float* hom, const float* depth_values, float* out,
+                                                 int V, int C, int D, int H, int W, int k, int num_groups,
+                                                 int ref_begin, int n_feat_views, void* stream) {
+  return groupcorr_fwd("plane_sweep_groupcorr_fwd_px", feat, feat_dtype, nbr_ids, hom, depth_values, out, V, C, D,
+                       H, W, k, num_groups, ref_begin, n_feat_views, true, stream);
+}
+
+extern "C" int mvsd_plane_sweep_groupcorr_bwd(const float* g_out, const void* feat, int feat_dtype,
+                                              const int32_t* nbr_ids, const float* hom,
+                                              const float* depth_values, float* g_feat, int V, int C,
+                                              int D, int H, int W, int k, int num_groups, int ref_begin,
+                                              int n_feat_views, void* stream) {
+  return groupcorr_bwd("plane_sweep_groupcorr_bwd", g_out, feat, feat_dtype, nbr_ids, hom, depth_values, g_feat, V,
+                       C, D, H, W, k, num_groups, ref_begin, n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_groupcorr_bwd_px(const float* g_out, const void* feat, int feat_dtype,
+                                                 const int32_t* nbr_ids, const float* hom,
+                                                 const float* depth_values, float* g_feat, int V, int C,
+                                                 int D, int H, int W, int k, int num_groups, int ref_begin,
+                                                 int n_feat_views, void* stream) {
+  return groupcorr_bwd("plane_sweep_groupcorr_bwd_px", g_out, feat, feat_dtype, nbr_ids, hom, depth_values,
+                       g_feat, V, C, D, H, W, k, num_groups, ref_begin, n_feat_views, true, stream);
 }

@@ -41,7 +41,7 @@ struct SweepParams {
   const void* feat;        // nhwc features
   const int32_t* nbr;      // [V,k] or nullptr (warp-only: source = same index)
   const float* hom;        // [V,k,12]
-  const float* depth;      // [V,D], or [V,D,H,W] when depth_per_pixel (stand-alone warp only)
+  const float* depth;      // [V,D], or [V,D,H,W] when depth_per_pixel
   void* out;               // fwd output [V,D,H,W,C]
   const void* g_out;       // bwd upstream gradient, same layout
   float* g_feat;           // bwd: nhwc fp32, accumulated with RED
@@ -92,12 +92,23 @@ __device__ __forceinline__ float depth_or_nan(float depth, int n, int n_feat) {
   return (unsigned)n < (unsigned)n_feat ? depth : __int_as_float(0x7fc00000);
 }
 
+// Depth of plane d at pixel (x, y) of reference view v: the per-view planes [V,D], or with
+// PER_PIXEL_DEPTH homo_warping's per-pixel hypotheses [V,D,H,W] (module.py:130-133).
+template <bool PER_PIXEL_DEPTH>
+__device__ __forceinline__ float plane_depth(const SweepParams& p, int v, int d, int x, int y) {
+  const size_t di = (size_t)v * p.D + d;
+  return PER_PIXEL_DEPTH ? __ldg(p.depth + (di * p.H + y) * p.W + x) : __ldg(p.depth + di);
+}
+
+// Which depth_values form a kernel's fill reads.  The fused kernels are compiled per form (the
+// per-pixel ones serve the *_px entry points): as a run-time select inside the per-view kernels'
+// fill it cost the forward sweep 6 % (measured: 0.291 vs 0.273 ms).  Only the stand-alone warp
+// selects at run time, from p.depth_per_pixel.
+enum DepthForm { kDepthPlanes, kDepthPixels, kDepthEither };
+
 // One pass of sample geometry for this warp's pixel: lane s computes the sample
 // of (plane d0 + s / k, neighbour s % k).
-// PER_PIXEL_DEPTH: homo_warping's [B,D,H,W] depth_values branch (module.py:130-133), compiled into
-// the stand-alone warp only -- as a run-time select inside the fused kernels' fill it cost the
-// forward sweep 6 % (measured: 0.291 vs 0.273 ms).
-template <bool PER_PIXEL_DEPTH = false>
+template <int DEPTH = kDepthPlanes>
 __device__ __forceinline__ void fill_samples(WarpSample* tab, const SweepParams& p,
                                              const SweepCoord& c, int d0, int dc, int lane) {
   const int k = p.k;
@@ -114,8 +125,8 @@ __device__ __forceinline__ void fill_samples(WarpSample* tab, const SweepParams&
 #pragma unroll
       for (int t = 0; t < 12; ++t) mm[t] = __ldg(m + t);
       const size_t di = (size_t)c.v * p.D + d;
-      const float depth = (PER_PIXEL_DEPTH && p.depth_per_pixel) ? __ldg(p.depth + (di * p.H + c.y) * p.W + c.x)
-                                                                 : __ldg(p.depth + di);
+      const bool per_pixel = DEPTH == kDepthPixels || (DEPTH == kDepthEither && p.depth_per_pixel);
+      const float depth = per_pixel ? __ldg(p.depth + (di * p.H + c.y) * p.W + c.x) : __ldg(p.depth + di);
       s = make_warp_sample(mm, (float)c.x, (float)c.y, depth_or_nan(depth, n, p.n_feat), p.H, p.W, p.C);
     }
     tab[lane] = s;

@@ -23,7 +23,9 @@ __device__ __forceinline__ void red_tap(TAcc* dst, unsigned off, const float4 (&
     if (group_on<FULL>(c0, g, C)) red_vec(a + 128 * g, f4scale(gw[g], w));
 }
 
-template <typename TIn, typename TG, int KMAX, int G, bool FULL, bool WARP_ONLY, typename TAcc = float>
+// PX: per-pixel depth hypotheses [V,D,H,W] (the *_px entry points)
+template <typename TIn, typename TG, int KMAX, int G, bool FULL, bool WARP_ONLY, typename TAcc = float,
+          bool PX = false>
 __global__ void __launch_bounds__(kSweepThreads) sweep_bwd_kernel(const SweepParams p) {
   TAcc* const g_acc = sizeof(TAcc) == 8 ? reinterpret_cast<TAcc*>(p.g_feat_q) : reinterpret_cast<TAcc*>(p.g_feat);
   __shared__ WarpSample s_tab[kSweepWarps][kSlots];
@@ -60,7 +62,7 @@ __global__ void __launch_bounds__(kSweepThreads) sweep_bwd_kernel(const SweepPar
   for (int d0 = 0; d0 < p.D; d0 += dc) {
     if (k > 0) {
       __syncwarp();
-      fill_samples<WARP_ONLY>(s_tab[warp], p, c, d0, dc, lane);
+      fill_samples<WARP_ONLY ? kDepthEither : (PX ? kDepthPixels : kDepthPlanes)>(s_tab[warp], p, c, d0, dc, lane);
       __syncwarp();
     }
     const int dend = min(p.D, d0 + dc);
@@ -124,11 +126,13 @@ static int launch_bwd_k(SweepParams& p, cudaStream_t st) {
   if (!sweep_grid(p, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: grid too large");
   // generic fallback (k = 3, 4, the stand-alone warp, and the test hook): one instantiation per
   // dtype and channel-group count, every k <= 4 and ragged C handled by predication
-#define MVSD_BWD(KM, GG) sweep_bwd_kernel<TIn, TG, KM, GG, false, WARP_ONLY><<<grid, kSweepThreads, 0, st>>>(p)
+#define MVSD_BWD(KM, GG, PX) sweep_bwd_kernel<TIn, TG, KM, GG, false, WARP_ONLY, float, PX><<<grid, kSweepThreads, 0, st>>>(p)
   if constexpr (WARP_ONLY) {
-    if (G == 2) MVSD_BWD(1, 2); else MVSD_BWD(1, 1);
+    if (G == 2) MVSD_BWD(1, 2, false); else MVSD_BWD(1, 1, false);
+  } else if (p.depth_per_pixel) {
+    if (G == 2) MVSD_BWD(4, 2, true); else MVSD_BWD(4, 1, true);
   } else {
-    if (G == 2) MVSD_BWD(4, 2); else MVSD_BWD(4, 1);
+    if (G == 2) MVSD_BWD(4, 2, false); else MVSD_BWD(4, 1, false);
   }
 #undef MVSD_BWD
   count_launch();
@@ -141,8 +145,13 @@ static int launch_bwd_det(SweepParams& p, cudaStream_t st) {
   dim3 grid;
   const int G = sweep_groups(p.C);
   if (!sweep_grid(p, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd_det: grid too large");
-  if (G == 2) sweep_bwd_kernel<TIn, TG, 4, 2, false, false, long long><<<grid, kSweepThreads, 0, st>>>(p);
-  else sweep_bwd_kernel<TIn, TG, 4, 1, false, false, long long><<<grid, kSweepThreads, 0, st>>>(p);
+#define MVSD_BWD_DET(GG, PX) sweep_bwd_kernel<TIn, TG, 4, GG, false, false, long long, PX><<<grid, kSweepThreads, 0, st>>>(p)
+  if (p.depth_per_pixel) {
+    if (G == 2) MVSD_BWD_DET(2, true); else MVSD_BWD_DET(1, true);
+  } else {
+    if (G == 2) MVSD_BWD_DET(2, false); else MVSD_BWD_DET(1, false);
+  }
+#undef MVSD_BWD_DET
   count_launch();
   return check_launch("plane_sweep_bwd_det");
 }
@@ -158,21 +167,22 @@ __global__ void fixed_to_float_kernel(const long long* __restrict__ src, float* 
 
 using namespace mvsd;
 
-extern "C" int mvsd_plane_sweep_bwd(const void* g_out, int g_dtype, int g_layout, const void* feat,
-                                    int feat_dtype, const int32_t* nbr_ids, const float* hom,
-                                    const float* depth_values, float* g_feat, int V, int C, int D,
-                                    int H, int W, int k, int ref_begin, int n_feat_views,
-                                    void* stream) {
-  if (int e = sweep_check("plane_sweep_bwd", V, C, D, H, W, k, g_layout)) return e;
+// per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133)
+static int plane_sweep_bwd(const char* who, const void* g_out, int g_dtype, int g_layout, const void* feat,
+                           int feat_dtype, const int32_t* nbr_ids, const float* hom,
+                           const float* depth_values, float* g_feat, int V, int C, int D, int H, int W,
+                           int k, int ref_begin, int n_feat_views, bool per_pixel, void* stream) {
+  if (int e = sweep_check(who, V, C, D, H, W, k, g_layout)) return e;
   if (!g_out || !feat || !g_feat || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_bwd: null pointer");
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
   if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_bwd: reference views [%d, %d) exceed the %d feature views",
-                ref_begin, ref_begin + V, n_feat_views);
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat_views);
   SweepParams p{};
   p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
   p.g_feat = g_feat;
   p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // Kernel selection.  k in {1, 2} (the reference uses k = min(2, V-1), mvsdet.py:432): the
   // run-merging kernels of plane_sweep_bwd_run.cu -- row hand-off + pipelined loads for bf16
@@ -185,7 +195,47 @@ extern "C" int mvsd_plane_sweep_bwd(const void* g_out, int g_dtype, int g_layout
     return launch_bwd_k<__nv_bfloat16, float, false>(p, st);
   if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16)
     return launch_bwd_k<__nv_bfloat16, __nv_bfloat16, false>(p, st);
-  return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: dtype combination not built");
+  return fail(MVSD_ERR_UNSUPPORTED, "%s: dtype combination not built", who);
+}
+
+static int plane_sweep_bwd_det(const char* who, const void* g_out, int g_dtype, int g_layout, const void* feat,
+                               int feat_dtype, const int32_t* nbr_ids, const float* hom,
+                               const float* depth_values, int64_t* g_feat_q, int V, int C, int D, int H,
+                               int W, int k, int ref_begin, int n_feat_views, bool per_pixel, void* stream) {
+  if (int e = sweep_check(who, V, C, D, H, W, k, g_layout)) return e;
+  if (!g_out || !feat || !g_feat_q || !depth_values || (k > 0 && (!nbr_ids || !hom)))
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat_views);
+  SweepParams p{};
+  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
+  p.g_feat_q = reinterpret_cast<long long*>(g_feat_q);
+  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_det<float, float>(p, st);
+  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32) return launch_bwd_det<__nv_bfloat16, float>(p, st);
+  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16) return launch_bwd_det<__nv_bfloat16, __nv_bfloat16>(p, st);
+  return fail(MVSD_ERR_UNSUPPORTED, "%s: dtype combination not built", who);
+}
+
+extern "C" int mvsd_plane_sweep_bwd(const void* g_out, int g_dtype, int g_layout, const void* feat,
+                                    int feat_dtype, const int32_t* nbr_ids, const float* hom,
+                                    const float* depth_values, float* g_feat, int V, int C, int D,
+                                    int H, int W, int k, int ref_begin, int n_feat_views,
+                                    void* stream) {
+  return plane_sweep_bwd("plane_sweep_bwd", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom, depth_values,
+                         g_feat, V, C, D, H, W, k, ref_begin, n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_bwd_px(const void* g_out, int g_dtype, int g_layout, const void* feat,
+                                       int feat_dtype, const int32_t* nbr_ids, const float* hom,
+                                       const float* depth_values, float* g_feat, int V, int C, int D,
+                                       int H, int W, int k, int ref_begin, int n_feat_views,
+                                       void* stream) {
+  return plane_sweep_bwd("plane_sweep_bwd_px", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
+                         depth_values, g_feat, V, C, D, H, W, k, ref_begin, n_feat_views, true, stream);
 }
 
 extern "C" int mvsd_plane_sweep_bwd_det(const void* g_out, int g_dtype, int g_layout, const void* feat,
@@ -193,21 +243,17 @@ extern "C" int mvsd_plane_sweep_bwd_det(const void* g_out, int g_dtype, int g_la
                                         const float* depth_values, int64_t* g_feat_q, int V, int C, int D,
                                         int H, int W, int k, int ref_begin, int n_feat_views,
                                         void* stream) {
-  if (int e = sweep_check("plane_sweep_bwd_det", V, C, D, H, W, k, g_layout)) return e;
-  if (!g_out || !feat || !g_feat_q || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_bwd_det: null pointer");
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_bwd_det: reference views [%d, %d) exceed the %d feature views",
-                ref_begin, ref_begin + V, n_feat_views);
-  SweepParams p{};
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
-  p.g_feat_q = reinterpret_cast<long long*>(g_feat_q);
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_det<float, float>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32) return launch_bwd_det<__nv_bfloat16, float>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16) return launch_bwd_det<__nv_bfloat16, __nv_bfloat16>(p, st);
-  return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd_det: dtype combination not built");
+  return plane_sweep_bwd_det("plane_sweep_bwd_det", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
+                             depth_values, g_feat_q, V, C, D, H, W, k, ref_begin, n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_bwd_det_px(const void* g_out, int g_dtype, int g_layout, const void* feat,
+                                           int feat_dtype, const int32_t* nbr_ids, const float* hom,
+                                           const float* depth_values, int64_t* g_feat_q, int V, int C, int D,
+                                           int H, int W, int k, int ref_begin, int n_feat_views,
+                                           void* stream) {
+  return plane_sweep_bwd_det("plane_sweep_bwd_det_px", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
+                             depth_values, g_feat_q, V, C, D, H, W, k, ref_begin, n_feat_views, true, stream);
 }
 
 extern "C" int mvsd_fixed_to_float(const int64_t* src, float* dst, int64_t n, void* stream) {

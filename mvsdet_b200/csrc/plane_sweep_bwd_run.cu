@@ -50,6 +50,8 @@ __device__ __forceinline__ RunCoord run_coord(const SweepParams& p, int warp, in
 }
 
 // lane s -> sample (plane d0 + s / (kRun*k), pixel x0 + (s % (kRun*k)) / k, neighbour s % k)
+// PX: per-pixel depth hypotheses [V,D,H,W] (the *_px entry points), in every run kernel below
+template <bool PX>
 __device__ __forceinline__ void fill_run_samples(WarpSample* tab, const SweepParams& p,
                                                  const RunCoord& c, int d0, int ppf, int lane) {
   const int k = p.k, spp = kRun * k;
@@ -67,7 +69,7 @@ __device__ __forceinline__ void fill_run_samples(WarpSample* tab, const SweepPar
 #pragma unroll
       for (int t = 0; t < 12; ++t) mm[t] = __ldg(m + t);
       s = make_warp_sample(mm, (float)(c.x0 + i), (float)c.y,
-                           depth_or_nan(__ldg(p.depth + (size_t)c.v * p.D + d), n, p.n_feat), p.H, p.W, p.C);
+                           depth_or_nan(plane_depth<PX>(p, c.v, d, c.x0 + i, c.y), n, p.n_feat), p.H, p.W, p.C);
     }
     tab[lane] = s;
   }
@@ -235,7 +237,7 @@ __device__ __forceinline__ void pixel_q(RunPending<KMAX, G>& pend, const WarpSam
 }
 
 // requires p.k == KMAX (the launcher instantiates KMAX = k for k in {1, 2})
-template <typename TIn, typename TG, int KMAX, int G, bool FULL, int MINB>
+template <typename TIn, typename TG, int KMAX, int G, bool FULL, int MINB, bool PX = false>
 __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runq_kernel(const SweepParams p) {
   constexpr int kCols = kRun * G * 4;
   __shared__ WarpSample s_tab[kRunRows][32];
@@ -289,7 +291,7 @@ __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runq_kernel(const
 
     for (int d0 = 0; d0 < p.D; d0 += ppf) {
       __syncwarp();
-      fill_run_samples(s_tab[warp], p, c, d0, ppf, lane);
+      fill_run_samples<PX>(s_tab[warp], p, c, d0, ppf, lane);
       __syncwarp();
       const int dend = min(p.D, d0 + ppf);
       for (int d = d0; d < dend; ++d) {
@@ -411,9 +413,14 @@ __device__ __forceinline__ void issue_pixel_loads(PixelRaw<TIn, TG, G>& raw, con
 // the other warp gets) and stores the outcome as four flag bits next to the sample; a warp
 // then reads only its own table, the per-pixel decision is a byte load, and the only
 // coupling left between the warps of a CTA is the hand-off queue itself.
+// With per-pixel depth (PX) the adjacent rows' samples are computed with THEIR pixels' depths,
+// (x, y+1) and (x, y-1): exactly the bits the other warp computes for its own row.  The depth of
+// this row would hand a weighted vector to a row that does not have that tap wherever the depth
+// changes between rows.
 // ---------------------------------------------------------------------------
 constexpr unsigned kHoSend = 1u, kHoRecv = 2u, kHoNzLeft = 4u, kHoNzRight = 8u;
 
+template <bool PX>
 __device__ __forceinline__ void fill_run_samples_ho(WarpSample* tab, unsigned char* flg,
                                                     const SweepParams& p, const RunCoord& c, int d0,
                                                     int ppf, int lane, bool has_up, bool has_dn) {
@@ -432,16 +439,18 @@ __device__ __forceinline__ void fill_run_samples_ho(WarpSample* tab, unsigned ch
       float mm[12];
 #pragma unroll
       for (int t = 0; t < 12; ++t) mm[t] = __ldg(m + t);
-      const float depth = depth_or_nan(__ldg(p.depth + (size_t)c.v * p.D + d), n, p.n_feat);
+      const float depth = depth_or_nan(plane_depth<PX>(p, c.v, d, c.x0 + i, c.y), n, p.n_feat);
       const float x = (float)(c.x0 + i);
       s = make_warp_sample(mm, x, (float)c.y, depth, p.H, p.W, p.C);
       if (s.p00 != kNoSample) {
         if (has_dn) {
-          const WarpSample dn = make_warp_sample(mm, x, (float)(c.y + 1), depth, p.H, p.W, p.C);
+          const float depth_dn = PX ? depth_or_nan(plane_depth<PX>(p, c.v, d, c.x0 + i, c.y + 1), n, p.n_feat) : depth;
+          const WarpSample dn = make_warp_sample(mm, x, (float)(c.y + 1), depth_dn, p.H, p.W, p.C);
           if (dn.p00 != kNoSample && dn.p00 == s.p10 && dn.p01 == s.p11) f |= kHoSend;
         }
         if (has_up) {
-          const WarpSample up = make_warp_sample(mm, x, (float)(c.y - 1), depth, p.H, p.W, p.C);
+          const float depth_up = PX ? depth_or_nan(plane_depth<PX>(p, c.v, d, c.x0 + i, c.y - 1), n, p.n_feat) : depth;
+          const WarpSample up = make_warp_sample(mm, x, (float)(c.y - 1), depth_up, p.H, p.W, p.C);
           if (up.p00 != kNoSample && up.p10 == s.p00 && up.p11 == s.p01) {
             f |= kHoRecv;
             if (s.w00 != 0.f || up.w10 != 0.f) f |= kHoNzLeft;
@@ -645,7 +654,7 @@ __device__ __forceinline__ void pixel_q3(RunPending<KMAX, G>& pend, PixelRaw<TIn
 }
 
 // requires p.k == KMAX
-template <typename TIn, typename TG, int KMAX, int G, bool FULL, int MINB, int NSTG, int MODE = 0>
+template <typename TIn, typename TG, int KMAX, int G, bool FULL, int MINB, int NSTG, int MODE = 0, bool PX = false>
 __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runs_kernel(const SweepParams p) {
   static_assert(MODE == 0 || (KMAX == 2 && sizeof(TG) == 4), "correlation mode: two neighbours, fp32 gradients");
   constexpr int kCols = kRun * G * 4;
@@ -725,8 +734,8 @@ __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runs_kernel(const
     tmem_wait_st();
 
     PixelRaw<TIn, TG, G> raw;
-    fill_run_samples_ho(s_tab[warp][0], s_flg[warp][0], p, c, 0, ppf, lane, has_up, has_dn);
-    if (ppf < p.D) fill_run_samples_ho(s_tab[warp][1], s_flg[warp][1], p, c, ppf, ppf, lane, has_up, has_dn);
+    fill_run_samples_ho<PX>(s_tab[warp][0], s_flg[warp][0], p, c, 0, ppf, lane, has_up, has_dn);
+    if (ppf < p.D) fill_run_samples_ho<PX>(s_tab[warp][1], s_flg[warp][1], p, c, ppf, ppf, lane, has_up, has_dn);
     __syncwarp();
     // pipeline prologue: first pixel of the first plane
     issue_pixel_loads<TIn, TG, KMAX, G, FULL, MODE>(raw, s_tab[warp][0], g_d, ref_row, nsrc, c.c0, C, p);
@@ -783,7 +792,7 @@ __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runs_kernel(const
       // this buffer's planes are done (the loads already in flight read the other buffer): refill it
       __syncwarp();
       if (d0 + 2 * ppf < p.D)
-        fill_run_samples_ho(s_tab[warp][buf], s_flg[warp][buf], p, c, d0 + 2 * ppf, ppf, lane, has_up, has_dn);
+        fill_run_samples_ho<PX>(s_tab[warp][buf], s_flg[warp][buf], p, c, d0 + 2 * ppf, ppf, lane, has_up, has_dn);
       __syncwarp();
     }
     tmem_wait_st();
@@ -803,7 +812,7 @@ __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runs_kernel(const
 // One run kernel is built per feature dtype: the hand-off kernel for bf16 features, the lean
 // kernel for fp32 features -- with fp32 features the raw loads of a pixel are 80 registers
 // instead of 44 and the pipelined kernel spills (ptxas: 160 B of stack).
-template <typename TIn, typename TG>
+template <typename TIn, typename TG, bool PX>
 static int launch_bwd_run_t(SweepParams& p, cudaStream_t st) {
   const int G = sweep_groups(p.C);
   p.tiles_x = (p.W + kRun - 1) / kRun;
@@ -816,7 +825,7 @@ static int launch_bwd_run_t(SweepParams& p, cudaStream_t st) {
 #define MVSD_RUN(KM, GG, FU)                                                                \
   do {                                                                                      \
     if constexpr (sizeof(TIn) == 2) {                                                       \
-      auto kern = sweep_bwd_runs_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks, 2>;            \
+      auto kern = sweep_bwd_runs_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks, 2, 0, PX>;     \
       constexpr size_t dyn = run_slot_bytes<KM, GG, 2>();                                   \
       static bool attr_set = false;                                                         \
       if (!attr_set) {                                                                      \
@@ -825,7 +834,7 @@ static int launch_bwd_run_t(SweepParams& p, cudaStream_t st) {
       }                                                                                     \
       kern<<<grid, kRunThreads, dyn, st>>>(p);                                              \
     } else {                                                                                \
-      sweep_bwd_runq_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks><<<grid, kRunThreads, 0, st>>>(p); \
+      sweep_bwd_runq_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks, PX><<<grid, kRunThreads, 0, st>>>(p); \
     }                                                                                       \
   } while (0)
   if (p.k == 1) {
@@ -842,8 +851,8 @@ static int launch_bwd_run_t(SweepParams& p, cudaStream_t st) {
 
 // Group-wise correlation backward (group_corr.cu) through the hand-off kernel: bf16 features, k = 2.
 // Returns -1 when this configuration is not built (the caller falls back to its pixel kernel).
-int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st) {
-  if (feat_dtype != MVSD_BF16 || p.k != 2) return -1;
+template <bool PX>
+static int launch_bwd_run_corr_t(SweepParams& p, cudaStream_t st) {
   typedef __nv_bfloat16 TIn;
   const int G = sweep_groups(p.C);
   p.tiles_x = (p.W + kRun - 1) / kRun;
@@ -855,7 +864,7 @@ int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st) {
   const bool full = p.C % (128 * G) == 0;
 #define MVSD_RUNC(GG, FU)                                                                   \
   do {                                                                                      \
-    auto kern = sweep_bwd_runs_kernel<TIn, float, 2, GG, FU, kRunQMinBlocks, 2, 1>;         \
+    auto kern = sweep_bwd_runs_kernel<TIn, float, 2, GG, FU, kRunQMinBlocks, 2, 1, PX>;     \
     constexpr size_t dyn = run_slot_bytes<2, GG, 2>();                                      \
     static bool attr_set = false;                                                           \
     if (!attr_set) {                                                                        \
@@ -871,13 +880,24 @@ int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st) {
   return check_launch("plane_sweep_groupcorr_bwd(run)");
 }
 
-int launch_bwd_run(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st) {
-  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_run_t<float, float>(p, st);
+int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st) {
+  if (feat_dtype != MVSD_BF16 || p.k != 2) return -1;
+  return p.depth_per_pixel ? launch_bwd_run_corr_t<true>(p, st) : launch_bwd_run_corr_t<false>(p, st);
+}
+
+template <bool PX>
+static int launch_bwd_run_px(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st) {
+  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_run_t<float, float, PX>(p, st);
   if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16)
-    return launch_bwd_run_t<__nv_bfloat16, __nv_bfloat16>(p, st);
+    return launch_bwd_run_t<__nv_bfloat16, __nv_bfloat16, PX>(p, st);
   if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32)
-    return launch_bwd_run_t<__nv_bfloat16, float>(p, st);
+    return launch_bwd_run_t<__nv_bfloat16, float, PX>(p, st);
   return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: dtype combination not built");
+}
+
+int launch_bwd_run(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st) {
+  return p.depth_per_pixel ? launch_bwd_run_px<true>(p, feat_dtype, g_dtype, st)
+                           : launch_bwd_run_px<false>(p, feat_dtype, g_dtype, st);
 }
 
 }  // namespace mvsd

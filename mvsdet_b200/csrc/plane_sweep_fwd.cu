@@ -37,7 +37,7 @@ __global__ void __launch_bounds__(kSweepThreads) sweep_fwd_kernel(const SweepPar
   for (int d0 = 0; d0 < p.D; d0 += dc) {
     if (k > 0) {
       __syncwarp();
-      fill_samples<WARP_ONLY>(s_tab[warp], p, c, d0, dc, lane);
+      fill_samples<WARP_ONLY ? kDepthEither : kDepthPlanes>(s_tab[warp], p, c, d0, dc, lane);
       __syncwarp();
     }
     const int dend = min(p.D, d0 + dc);
@@ -97,7 +97,8 @@ __global__ void __launch_bounds__(kSweepThreads) sweep_fwd_kernel(const SweepPar
 constexpr int kFwdPatchW = 2, kFwdPatchH = 2;
 constexpr int kFwdWarps = kFwdPatchW * kFwdPatchH, kFwdThreads = kFwdWarps * 32;
 
-template <typename TIn, typename TOut, int KMAX, int G, bool FULL>
+// PX: per-pixel depth hypotheses [V,D,H,W] (mvsd_plane_sweep_fwd_px); PX = false is the per-view kernel.
+template <typename TIn, typename TOut, int KMAX, int G, bool FULL, bool PX>
 // 8 CTAs x 4 warps per SM = 64 registers (9 CTAs at 56 registers measured the same, 10 at 48 spill: 0.313 ms)
 __global__ void __launch_bounds__(kFwdThreads, 8) sweep_fwd_p_kernel(const SweepParams p) {
   __shared__ WarpSample s_tab[kFwdWarps][kSlots];
@@ -144,7 +145,7 @@ __global__ void __launch_bounds__(kFwdThreads, 8) sweep_fwd_p_kernel(const Sweep
   for (int d0 = 0; d0 < p.D; d0 += dc) {
     if (k > 0) {
       __syncwarp();
-      fill_samples(s_tab[warp], p, c, d0, dc, lane);
+      fill_samples<PX ? kDepthPixels : kDepthPlanes>(s_tab[warp], p, c, d0, dc, lane);
       __syncwarp();
     }
     const int dend = min(p.D, d0 + dc);
@@ -279,8 +280,10 @@ static int launch_fwd_k(SweepParams& p, cudaStream_t st) {
   do {                                                                                 \
     if constexpr (WARP_ONLY)                                                           \
       sweep_fwd_kernel<TIn, TOut, KM, GG, FU, true><<<grid, kSweepThreads, 0, st>>>(p); \
+    else if (p.depth_per_pixel)                                                        \
+      sweep_fwd_p_kernel<TIn, TOut, KM, GG, FU, true><<<grid, kFwdThreads, 0, st>>>(p); \
     else                                                                               \
-      sweep_fwd_p_kernel<TIn, TOut, KM, GG, FU><<<grid, kFwdThreads, 0, st>>>(p);      \
+      sweep_fwd_p_kernel<TIn, TOut, KM, GG, FU, false><<<grid, kFwdThreads, 0, st>>>(p); \
   } while (0)
 #define MVSD_FWD_G(KM)                                                            \
   do {                                                                            \
@@ -318,20 +321,38 @@ static int launch_fwd(SweepParams& p, int in_dtype, int out_dtype, cudaStream_t 
 
 using namespace mvsd;
 
+// per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133)
+static int plane_sweep_fwd(const char* who, const void* feat, int feat_dtype, const int32_t* nbr_ids,
+                           const float* hom, const float* depth_values, void* out, int out_dtype,
+                           int out_layout, int V, int C, int D, int H, int W, int k, int ref_begin,
+                           int n_feat_views, bool per_pixel, void* stream) {
+  if (int e = sweep_check(who, V, C, D, H, W, k, out_layout)) return e;
+  if (!feat || !out || !depth_values || (k > 0 && (!nbr_ids || !hom)))
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat_views);
+  SweepParams p{};
+  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.out = out;
+  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
+  return launch_fwd<false>(p, feat_dtype, out_dtype, static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int mvsd_plane_sweep_fwd(const void* feat, int feat_dtype, const int32_t* nbr_ids,
                                     const float* hom, const float* depth_values, void* out,
                                     int out_dtype, int out_layout, int V, int C, int D, int H,
                                     int W, int k, int ref_begin, int n_feat_views, void* stream) {
-  if (int e = sweep_check("plane_sweep_fwd", V, C, D, H, W, k, out_layout)) return e;
-  if (!feat || !out || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_fwd: null pointer");
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "plane_sweep_fwd: reference views [%d, %d) exceed the %d feature views",
-                ref_begin, ref_begin + V, n_feat_views);
-  SweepParams p{};
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.out = out;
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  return launch_fwd<false>(p, feat_dtype, out_dtype, static_cast<cudaStream_t>(stream));
+  return plane_sweep_fwd("plane_sweep_fwd", feat, feat_dtype, nbr_ids, hom, depth_values, out, out_dtype,
+                         out_layout, V, C, D, H, W, k, ref_begin, n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_fwd_px(const void* feat, int feat_dtype, const int32_t* nbr_ids,
+                                       const float* hom, const float* depth_values, void* out,
+                                       int out_dtype, int out_layout, int V, int C, int D, int H,
+                                       int W, int k, int ref_begin, int n_feat_views, void* stream) {
+  return plane_sweep_fwd("plane_sweep_fwd_px", feat, feat_dtype, nbr_ids, hom, depth_values, out, out_dtype,
+                         out_layout, V, C, D, H, W, k, ref_begin, n_feat_views, true, stream);
 }
 
 extern "C" int mvsd_homo_warp_fwd(const void* src, int src_dtype, const float* hom,

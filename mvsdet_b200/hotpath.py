@@ -87,13 +87,18 @@ class MVSDetHotPath(nn.Module):
 
     # -- stages ------------------------------------------------------------
     def variance(self, feat_cl: torch.Tensor, geo: SceneGeometry, ref_begin: int = 0,
-                 grad_sink=None) -> torch.Tensor:
+                 grad_sink=None, depth_values: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The variance volume over the scene's neighbour ids and homographies.  ``depth_values``
+        (default: the scene's planes ``geo.depth_values`` [V,D]) may be the caller's own planes, e.g.
+        per-pixel hypotheses [V,D,Hf,Wf] for a second, narrow sweep around ``est_depth``; with the
+        ``grad_sink`` of the first sweep both sweeps' feature gradients go to one accumulator."""
+        depth = geo.depth_values if depth_values is None else depth_values
         if self.dispatcher_ops:
             if self.variance_dtype not in (torch.float32, torch.bfloat16):
                 raise ValueError("variance_dtype must be float32 or bfloat16")
-            return library.plane_sweep_variance(feat_cl, geo.neighbor_ids, geo.hom, geo.depth_values,
+            return library.plane_sweep_variance(feat_cl, geo.neighbor_ids, geo.hom, depth,
                                                 self.variance_dtype == torch.bfloat16, ref_begin)
-        return ops.plane_sweep_variance(feat_cl, geo.neighbor_ids, geo.hom, geo.depth_values,
+        return ops.plane_sweep_variance(feat_cl, geo.neighbor_ids, geo.hom, depth,
                                         out_dtype=self.variance_dtype, ref_begin=ref_begin,
                                         grad_sink=grad_sink)
 

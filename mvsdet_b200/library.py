@@ -18,7 +18,8 @@ multi-GPU combine, which a functional dispatcher op cannot (no aliasing of input
 Operators (reference lines as in ``ops.py``):
 
   plane_sweep_variance(feat, nbr_ids, hom, depth_values, out_bf16=False, ref_begin=0) -> variance
-      mvsdet.py:439-467 + mvs_models/module.py:105-146
+      mvsdet.py:439-467 + mvs_models/module.py:105-146; depth_values [V,D] or per-pixel
+      [V,D,H,W] (module.py:130-133), in this op and in plane_sweep_group_correlation
   plane_sweep_group_correlation(feat, nbr_ids, hom, depth_values, num_groups=8, ref_begin=0) -> [V,k,G,D,H,W]
       mvs_models/lss_fpn.py:485-506 over mvs_models/module.py:105-146 (optional operator)
   depth_topk(cost_out, near, interval, topk, raw=False)

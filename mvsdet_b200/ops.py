@@ -278,6 +278,9 @@ def _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink=None) ->
     if nbr_ids.dtype != torch.int32 or not nbr_ids.is_contiguous():
         raise ValueError("nbr_ids must be contiguous int32 [V,k]")
     v, k = nbr_ids.shape
+    if depth_values.dim() not in (2, 4) or \
+            (depth_values.dim() == 4 and tuple(depth_values.shape[2:]) != tuple(feat.shape[2:])):
+        raise ValueError("depth_values must be [V,D] or [V,D,H,W] with feat's H,W")
     if tuple(hom.shape) != (v, k, 12) or depth_values.shape[0] != v:
         raise ValueError("nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
     if ref_begin < 0 or ref_begin + v > feat.shape[0]:
@@ -296,7 +299,12 @@ def plane_sweep_variance(feat: torch.Tensor, nbr_ids: torch.Tensor, hom: torch.T
     neighbour ids [V,k] int32 (indices into feat), homographies [V,k,12], depth
     planes [V,D] -> variance volume, logical [V,C,D,H,W] in channels_last_3d.
     Reference view v is feat[ref_begin + v]; V < Vf sweeps a slice of the views
-    (view-sharded multi-GPU)."""
+    (view-sharded multi-GPU).
+    ``depth_values`` may also be per-pixel hypotheses [V,D,H,W] with feat's H,W
+    (homo_warping's branch, mvs_models/module.py:130-133), e.g. a narrow second
+    sweep around ``depth_topk``'s ``est_depth``; plane d of pixel (x, y) then lies at
+    depth_values[v, d, y, x], and a NaN depth gives no sample.  Any other shape is a
+    ``ValueError``."""
     _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink)
     return _PlaneSweepVariance.apply(feat, nbr_ids, hom.contiguous(), depth_values.contiguous(),
                                      out_dtype, int(ref_begin), grad_sink)
@@ -345,8 +353,6 @@ def _check_corr(feat, nbr_ids, hom, depth_values, num_groups, ref_begin, grad_si
     _check_sweep(feat, nbr_ids, hom, depth_values, ref_begin, grad_sink)
     if nbr_ids.shape[1] < 1:
         raise ValueError("group correlation needs at least one neighbour")
-    if depth_values.dim() != 2:
-        raise ValueError("nbr_ids [V,k], hom [V,k,12] and depth_values [V,D] must agree")
     if num_groups < 1 or feat.shape[1] % num_groups != 0:
         raise ValueError("the channel count must be divisible by num_groups")
 
@@ -356,7 +362,8 @@ def plane_sweep_group_correlation(feat: torch.Tensor, nbr_ids: torch.Tensor, hom
                                   grad_sink: Optional[FeatureGradSink] = None) -> torch.Tensor:
     """Group-wise correlation cost volumes over the plane sweep (SURVEY.md 8f rank 4; the reference's
     arithmetic is mvs_models/lss_fpn.py:485-506, the warp mvs_models/module.py:105-146): same arguments
-    as ``plane_sweep_variance``; -> logical [V,k,num_groups,D,H,W] fp32, one volume per neighbour,
+    as ``plane_sweep_variance``, including per-pixel ``depth_values`` [V,D,H,W];
+    -> logical [V,k,num_groups,D,H,W] fp32, one volume per neighbour,
     ``mean over the group's channels of ref * warped_j``.  C / num_groups must be 4 ... 128 and divide
     128.  The memory order is [V,k,D,H,W,num_groups]."""
     _check_corr(feat, nbr_ids, hom, depth_values, num_groups, ref_begin, grad_sink)
