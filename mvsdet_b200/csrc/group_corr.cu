@@ -245,37 +245,24 @@ static int corr_setup(const char* who, CorrParams& q, int num_groups) {
   return MVSD_OK;
 }
 
-template <bool BWD, typename TIn, bool PX>
-static int corr_launch(CorrParams& q, cudaStream_t st) {
-  dim3 grid;
-  const int G = sweep_groups(q.s.C);
-  if (!sweep_grid(q.s, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_groupcorr: grid too large");
-  if constexpr (!BWD) {                          // the forward has its own CTA patch
-    q.s.tiles_x = (q.s.W + kCorrPatchW - 1) / kCorrPatchW;
-    q.s.tiles_y = (q.s.H + kCorrPatchH - 1) / kCorrPatchH;
-    const long long blocks = (long long)q.s.V * q.s.slices * q.s.tiles_y * q.s.tiles_x;
-    if (blocks > 2147483647LL) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_groupcorr: grid too large");
-    grid = dim3((unsigned)blocks);
-  }
-  const bool full = q.s.C % (128 * G) == 0;
-#define MVSD_CORR(GG, FU)                                                        \
-  do {                                                                           \
-    if constexpr (BWD) corr_bwd_kernel<TIn, GG, FU, PX><<<grid, kSweepThreads, 0, st>>>(q); \
-    else if (q.s.k == 2) corr_fwd_kernel<TIn, 2, GG, FU, PX><<<grid, kCorrThreads, 0, st>>>(q); \
-    else corr_fwd_kernel<TIn, 4, GG, FU, PX><<<grid, kCorrThreads, 0, st>>>(q);  \
-  } while (0)
-  if (G == 2) { if (full) MVSD_CORR(2, true); else MVSD_CORR(2, false); }
-  else { if (full) MVSD_CORR(1, true); else MVSD_CORR(1, false); }
-#undef MVSD_CORR
-  count_launch();
-  return check_launch(BWD ? "plane_sweep_groupcorr_bwd" : "plane_sweep_groupcorr_fwd");
+template <bool BWD, typename TIn>
+static int corr_launch_t(CorrParams& q, cudaStream_t st) {
+  // the forward has its own CTA patch
+  return sweep_launch(q.s, "plane_sweep_groupcorr", BWD ? kPatchW : kCorrPatchW, BWD ? kPatchH : kCorrPatchH,
+                      BWD ? "plane_sweep_groupcorr_bwd" : "plane_sweep_groupcorr_fwd",
+                      [&](dim3 grid, auto G2, auto FULL, auto PX) {
+    constexpr int GG = G2 ? 2 : 1;
+    if constexpr (BWD) corr_bwd_kernel<TIn, GG, FULL, PX><<<grid, kSweepThreads, 0, st>>>(q);
+    else if (q.s.k == 2) corr_fwd_kernel<TIn, 2, GG, FULL, PX><<<grid, kCorrThreads, 0, st>>>(q);
+    else corr_fwd_kernel<TIn, 4, GG, FULL, PX><<<grid, kCorrThreads, 0, st>>>(q);
+  });
 }
 
-int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st);     // plane_sweep_bwd_run.cu
-
-template <bool BWD, typename TIn>
-static int corr_launch_px(CorrParams& q, cudaStream_t st) {
-  return q.s.depth_per_pixel ? corr_launch<BWD, TIn, true>(q, st) : corr_launch<BWD, TIn, false>(q, st);
+template <bool BWD>
+static int corr_launch(CorrParams& q, const char* who, int feat_dtype, cudaStream_t st) {
+  if (feat_dtype == MVSD_F32) return corr_launch_t<BWD, float>(q, st);
+  if (feat_dtype == MVSD_BF16) return corr_launch_t<BWD, __nv_bfloat16>(q, st);
+  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
 }
 
 // per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133)
@@ -283,51 +270,32 @@ static int groupcorr_fwd(const char* who, const void* feat, int feat_dtype, cons
                          const float* hom, const float* depth_values, float* out, int V, int C, int D, int H,
                          int W, int k, int num_groups, int ref_begin, int n_feat_views, bool per_pixel,
                          void* stream) {
-  if (int e = sweep_check(who, V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
-  if (!feat || !out || !depth_values || !nbr_ids || !hom)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
-                who, ref_begin, ref_begin + V, n_feat_views);
   CorrParams q{};
-  SweepParams& p = q.s;
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.out = out;
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  p.depth_per_pixel = per_pixel ? 1 : 0;
+  if (int e = sweep_setup(q.s, who, {feat, out}, true, feat, nbr_ids, hom, depth_values, V, C, D, H, W, k,
+                          MVSD_CHANNELS_LAST, ref_begin, n_feat_views, per_pixel))
+    return e;
+  q.s.out = out;
   if (int e = corr_setup(who, q, num_groups)) return e;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (feat_dtype == MVSD_F32) return corr_launch_px<false, float>(q, st);
-  if (feat_dtype == MVSD_BF16) return corr_launch_px<false, __nv_bfloat16>(q, st);
-  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
+  return corr_launch<false>(q, who, feat_dtype, static_cast<cudaStream_t>(stream));
 }
 
 static int groupcorr_bwd(const char* who, const float* g_out, const void* feat, int feat_dtype,
                          const int32_t* nbr_ids, const float* hom, const float* depth_values, float* g_feat,
                          int V, int C, int D, int H, int W, int k, int num_groups, int ref_begin,
                          int n_feat_views, bool per_pixel, void* stream) {
-  if (int e = sweep_check(who, V, C, D, H, W, k, MVSD_CHANNELS_LAST)) return e;
-  if (!g_out || !feat || !g_feat || !depth_values || !nbr_ids || !hom)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
-                who, ref_begin, ref_begin + V, n_feat_views);
   CorrParams q{};
-  SweepParams& p = q.s;
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out; p.g_feat = g_feat;
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  p.depth_per_pixel = per_pixel ? 1 : 0;
+  if (int e = sweep_setup(q.s, who, {g_out, feat, g_feat}, true, feat, nbr_ids, hom, depth_values, V, C, D, H, W,
+                          k, MVSD_CHANNELS_LAST, ref_begin, n_feat_views, per_pixel))
+    return e;
+  q.s.g_out = g_out;
+  q.s.g_feat = g_feat;
   if (int e = corr_setup(who, q, num_groups)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // bf16 features, k = 2: the run-merging hand-off kernel of the variance backward with the correlation
   // algebra in its pixel body (same gather, same merged scatter); anything else (and the test hook
   // mvsd_set_tuning(5, 1)): the pixel-per-warp kernel above
-  if (tuning(5) != 1) {
-    const int rc = launch_bwd_run_corr(p, feat_dtype, st);
-    if (rc >= 0) return rc;
-  }
-  if (feat_dtype == MVSD_F32) return corr_launch_px<true, float>(q, st);
-  if (feat_dtype == MVSD_BF16) return corr_launch_px<true, __nv_bfloat16>(q, st);
-  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
+  if (feat_dtype == MVSD_BF16 && k == 2 && tuning(5) != 1) return launch_bwd_run_corr(q.s, st);
+  return corr_launch<true>(q, who, feat_dtype, st);
 }
 
 }  // namespace mvsd

@@ -28,6 +28,9 @@
 //
 // HBM-bound by design (SURVEY.md section 0): no contraction, no tensor cores.
 #pragma once
+#include <initializer_list>
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mvsd {
@@ -412,9 +415,48 @@ __device__ __forceinline__ void blend_taps(const RawTaps<TIn, G>& r, const WarpS
   }
 }
 
-// host-side helpers shared by the two translation units
-int sweep_check(const char* who, int V, int C, int D, int H, int W, int k, int layout);
-bool sweep_grid(SweepParams& p, int G, dim3& grid);
-int sweep_groups(int C);
+// ---- host side, shared by the sweep translation units ---------------------------------------------
+
+// Validates the arguments of a sweep entry point and fills p's inputs, sizes and depth form; the
+// caller sets the output fields.  Checks in this order: dimensions, C, k, map size and layout, then
+// null pointers, then the reference-view range.  `bufs` are the call's feature, output and gradient
+// buffers; the neighbour ids and homographies are required too when `need_nbr`.
+int sweep_setup(SweepParams& p, const char* who, std::initializer_list<const void*> bufs, bool need_nbr,
+                const void* feat, const int32_t* nbr, const float* hom, const float* depth, int V, int C,
+                int D, int H, int W, int k, int layout, int ref_begin, int n_feat, bool per_pixel);
+// Grid of one CTA per tile_w x tile_h pixels, per 128*G-channel slice and per reference view; sets
+// p.tiles_x / tiles_y / slices.
+int sweep_grid(SweepParams& p, const char* who, int tile_w, int tile_h, int G, dim3& grid);
+
+// The run-merging backwards (plane_sweep_bwd_run.cu): the variance backward for k in {1, 2}, and the
+// group-wise correlation backward for bf16 features and k = 2.
+int launch_bwd_run(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st);
+int launch_bwd_run_corr(SweepParams& p, cudaStream_t st);
+
+// Calls f(std::bool_constant<b>...) for the run-time flags b...: a launcher's generic lambda is
+// compiled for every combination and states which kernel each one launches.  Everything inlines:
+// no std::function, no allocation.
+template <typename F>
+inline void with_flags(F&& f) { f(); }
+template <typename F, typename... Bs>
+inline void with_flags(F&& f, bool b, Bs... bs) {
+  if (b) with_flags([&](auto... c) { f(std::true_type{}, c...); }, bs...);
+  else with_flags([&](auto... c) { f(std::false_type{}, c...); }, bs...);
+}
+
+// One sweep kernel launch: the grid for tile_w x tile_h pixel CTAs (errors name `who`), then
+// launch(grid, G2, FULL, PX, extra...) with compile-time flags -- two channel groups per warp, C a
+// multiple of the warp's channels, per-pixel depth -- counted and checked as `name`.
+template <typename F, typename... Bs>
+int sweep_launch(SweepParams& p, const char* who, int tile_w, int tile_h, const char* name, F&& launch,
+                 Bs... extra) {
+  const int G = p.C > 128 ? 2 : 1;      // 128-channel groups per warp: all 256 FPN channels of a tap in one warp
+  dim3 grid;
+  if (int e = sweep_grid(p, who, tile_w, tile_h, G, grid)) return e;
+  with_flags([&](auto... c) { launch(grid, c...); }, G == 2, p.C % (128 * G) == 0, p.depth_per_pixel != 0,
+             extra...);
+  count_launch();
+  return check_launch(name);
+}
 
 }  // namespace mvsd

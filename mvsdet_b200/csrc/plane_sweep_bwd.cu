@@ -119,44 +119,20 @@ __global__ void __launch_bounds__(kSweepThreads) sweep_bwd_kernel(const SweepPar
   }
 }
 
-template <typename TIn, typename TG, bool WARP_ONLY>
+// The pixel-per-warp kernel: the variance backward for k = 0, 3, 4 (and every k through the test hook),
+// its deterministic form (TAcc = long long) and the stand-alone warp.  One instantiation per dtype and
+// channel-group count: every k <= 4 and ragged C handled by predication.
+template <typename TIn, typename TG, bool WARP_ONLY, typename TAcc>
 static int launch_bwd_k(SweepParams& p, cudaStream_t st) {
-  dim3 grid;
-  const int G = sweep_groups(p.C);
-  if (!sweep_grid(p, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: grid too large");
-  // generic fallback (k = 3, 4, the stand-alone warp, and the test hook): one instantiation per
-  // dtype and channel-group count, every k <= 4 and ragged C handled by predication
-#define MVSD_BWD(KM, GG, PX) sweep_bwd_kernel<TIn, TG, KM, GG, false, WARP_ONLY, float, PX><<<grid, kSweepThreads, 0, st>>>(p)
-  if constexpr (WARP_ONLY) {
-    if (G == 2) MVSD_BWD(1, 2, false); else MVSD_BWD(1, 1, false);
-  } else if (p.depth_per_pixel) {
-    if (G == 2) MVSD_BWD(4, 2, true); else MVSD_BWD(4, 1, true);
-  } else {
-    if (G == 2) MVSD_BWD(4, 2, false); else MVSD_BWD(4, 1, false);
-  }
-#undef MVSD_BWD
-  count_launch();
-  return check_launch("plane_sweep_bwd");
+  const char* name = sizeof(TAcc) == 8 ? "plane_sweep_bwd_det" : "plane_sweep_bwd";
+  return sweep_launch(p, name, kPatchW, kPatchH, name, [&](dim3 grid, auto G2, auto /*FULL*/, auto PX) {
+    constexpr int GG = G2 ? 2 : 1;
+    if constexpr (WARP_ONLY)              // reads either depth form (fill_samples<kDepthEither>)
+      sweep_bwd_kernel<TIn, TG, 1, GG, false, true><<<grid, kSweepThreads, 0, st>>>(p);
+    else
+      sweep_bwd_kernel<TIn, TG, 4, GG, false, false, TAcc, PX><<<grid, kSweepThreads, 0, st>>>(p);
+  });
 }
-
-// deterministic form: the pixel-per-warp kernel with 64-bit fixed-point integer REDs
-template <typename TIn, typename TG>
-static int launch_bwd_det(SweepParams& p, cudaStream_t st) {
-  dim3 grid;
-  const int G = sweep_groups(p.C);
-  if (!sweep_grid(p, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd_det: grid too large");
-#define MVSD_BWD_DET(GG, PX) sweep_bwd_kernel<TIn, TG, 4, GG, false, false, long long, PX><<<grid, kSweepThreads, 0, st>>>(p)
-  if (p.depth_per_pixel) {
-    if (G == 2) MVSD_BWD_DET(2, true); else MVSD_BWD_DET(1, true);
-  } else {
-    if (G == 2) MVSD_BWD_DET(2, false); else MVSD_BWD_DET(1, false);
-  }
-#undef MVSD_BWD_DET
-  count_launch();
-  return check_launch("plane_sweep_bwd_det");
-}
-
-int launch_bwd_run(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st);
 
 __global__ void fixed_to_float_kernel(const long long* __restrict__ src, float* __restrict__ dst, long long n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -167,56 +143,33 @@ __global__ void fixed_to_float_kernel(const long long* __restrict__ src, float* 
 
 using namespace mvsd;
 
-// per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133)
+// per_pixel: depth_values is [V,D,H,W] (homo_warping's per-pixel branch, module.py:130-133).
+// g_acc: dL/dfeat, fp32 (TAcc = float) or the deterministic form's 64-bit fixed point (TAcc = long long).
+template <typename TAcc>
 static int plane_sweep_bwd(const char* who, const void* g_out, int g_dtype, int g_layout, const void* feat,
                            int feat_dtype, const int32_t* nbr_ids, const float* hom,
-                           const float* depth_values, float* g_feat, int V, int C, int D, int H, int W,
+                           const float* depth_values, TAcc* g_acc, int V, int C, int D, int H, int W,
                            int k, int ref_begin, int n_feat_views, bool per_pixel, void* stream) {
-  if (int e = sweep_check(who, V, C, D, H, W, k, g_layout)) return e;
-  if (!g_out || !feat || !g_feat || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
-                who, ref_begin, ref_begin + V, n_feat_views);
-  SweepParams p{};
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
-  p.g_feat = g_feat;
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  p.depth_per_pixel = per_pixel ? 1 : 0;
+  constexpr bool det = std::is_same_v<TAcc, long long>;
+  SweepParams p;
+  if (int e = sweep_setup(p, who, {g_out, feat, g_acc}, k > 0, feat, nbr_ids, hom, depth_values, V, C, D, H, W,
+                          k, g_layout, ref_begin, n_feat_views, per_pixel))
+    return e;
+  p.g_out = g_out;
+  if constexpr (det) p.g_feat_q = g_acc;
+  else p.g_feat = g_acc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // Kernel selection.  k in {1, 2} (the reference uses k = min(2, V-1), mvsdet.py:432): the
   // run-merging kernels of plane_sweep_bwd_run.cu -- row hand-off + pipelined loads for bf16
-  // features, the lean kernel for fp32 features.  Any other k (and the stand-alone warp): the
+  // features, the lean kernel for fp32 features.  Any other k, and the deterministic form: the
   // pixel-per-warp kernel above.  mvsd_set_tuning(5, 1) is a TEST hook, never used on the product
   // path: it sends k in {1, 2} to the pixel kernel too.
-  if ((k == 1 || k == 2) && tuning(5) != 1) return launch_bwd_run(p, feat_dtype, g_dtype, st);
-  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_k<float, float, false>(p, st);
+  if (!det && (k == 1 || k == 2) && tuning(5) != 1) return launch_bwd_run(p, feat_dtype, g_dtype, st);
+  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_k<float, float, false, TAcc>(p, st);
   if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32)
-    return launch_bwd_k<__nv_bfloat16, float, false>(p, st);
+    return launch_bwd_k<__nv_bfloat16, float, false, TAcc>(p, st);
   if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16)
-    return launch_bwd_k<__nv_bfloat16, __nv_bfloat16, false>(p, st);
-  return fail(MVSD_ERR_UNSUPPORTED, "%s: dtype combination not built", who);
-}
-
-static int plane_sweep_bwd_det(const char* who, const void* g_out, int g_dtype, int g_layout, const void* feat,
-                               int feat_dtype, const int32_t* nbr_ids, const float* hom,
-                               const float* depth_values, int64_t* g_feat_q, int V, int C, int D, int H,
-                               int W, int k, int ref_begin, int n_feat_views, bool per_pixel, void* stream) {
-  if (int e = sweep_check(who, V, C, D, H, W, k, g_layout)) return e;
-  if (!g_out || !feat || !g_feat_q || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
-                who, ref_begin, ref_begin + V, n_feat_views);
-  SweepParams p{};
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
-  p.g_feat_q = reinterpret_cast<long long*>(g_feat_q);
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  p.depth_per_pixel = per_pixel ? 1 : 0;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_det<float, float>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32) return launch_bwd_det<__nv_bfloat16, float>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16) return launch_bwd_det<__nv_bfloat16, __nv_bfloat16>(p, st);
+    return launch_bwd_k<__nv_bfloat16, __nv_bfloat16, false, TAcc>(p, st);
   return fail(MVSD_ERR_UNSUPPORTED, "%s: dtype combination not built", who);
 }
 
@@ -243,8 +196,9 @@ extern "C" int mvsd_plane_sweep_bwd_det(const void* g_out, int g_dtype, int g_la
                                         const float* depth_values, int64_t* g_feat_q, int V, int C, int D,
                                         int H, int W, int k, int ref_begin, int n_feat_views,
                                         void* stream) {
-  return plane_sweep_bwd_det("plane_sweep_bwd_det", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
-                             depth_values, g_feat_q, V, C, D, H, W, k, ref_begin, n_feat_views, false, stream);
+  return plane_sweep_bwd("plane_sweep_bwd_det", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
+                         depth_values, reinterpret_cast<long long*>(g_feat_q), V, C, D, H, W, k, ref_begin,
+                         n_feat_views, false, stream);
 }
 
 extern "C" int mvsd_plane_sweep_bwd_det_px(const void* g_out, int g_dtype, int g_layout, const void* feat,
@@ -252,8 +206,9 @@ extern "C" int mvsd_plane_sweep_bwd_det_px(const void* g_out, int g_dtype, int g
                                            const float* depth_values, int64_t* g_feat_q, int V, int C, int D,
                                            int H, int W, int k, int ref_begin, int n_feat_views,
                                            void* stream) {
-  return plane_sweep_bwd_det("plane_sweep_bwd_det_px", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
-                             depth_values, g_feat_q, V, C, D, H, W, k, ref_begin, n_feat_views, true, stream);
+  return plane_sweep_bwd("plane_sweep_bwd_det_px", g_out, g_dtype, g_layout, feat, feat_dtype, nbr_ids, hom,
+                         depth_values, reinterpret_cast<long long*>(g_feat_q), V, C, D, H, W, k, ref_begin,
+                         n_feat_views, true, stream);
 }
 
 extern "C" int mvsd_fixed_to_float(const int64_t* src, float* dst, int64_t n, void* stream) {
@@ -270,16 +225,14 @@ extern "C" int mvsd_fixed_to_float(const int64_t* src, float* dst, int64_t n, vo
 extern "C" int mvsd_homo_warp_bwd(const void* g_out, int g_dtype, int g_layout, const float* hom,
                                   const float* depth_values, float* g_src, int B, int C, int D,
                                   int H, int W, int depth_per_pixel, void* stream) {
-  if (int e = sweep_check("homo_warp_bwd", B, C, D, H, W, 1, g_layout)) return e;
-  if (!g_out || !hom || !depth_values || !g_src)
-    return fail(MVSD_ERR_INVALID_ARG, "homo_warp_bwd: null pointer");
-  SweepParams p{};
-  p.feat = nullptr; p.nbr = nullptr; p.hom = hom; p.depth = depth_values; p.g_out = g_out;
+  SweepParams p;
+  if (int e = sweep_setup(p, "homo_warp_bwd", {g_out, hom, g_src}, false, nullptr, nullptr, hom, depth_values, B, C,
+                          D, H, W, 1, g_layout, 0, B, depth_per_pixel != 0))
+    return e;
+  p.g_out = g_out;
   p.g_feat = g_src;
-  p.V = B; p.C = C; p.D = D; p.H = H; p.W = W; p.k = 1; p.ref_begin = 0; p.n_feat = B;
-  p.depth_per_pixel = depth_per_pixel ? 1 : 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (g_dtype == MVSD_F32) return launch_bwd_k<float, float, true>(p, st);
-  if (g_dtype == MVSD_BF16) return launch_bwd_k<float, __nv_bfloat16, true>(p, st);
+  if (g_dtype == MVSD_F32) return launch_bwd_k<float, float, true, float>(p, st);
+  if (g_dtype == MVSD_BF16) return launch_bwd_k<float, __nv_bfloat16, true, float>(p, st);
   return fail(MVSD_ERR_INVALID_ARG, "homo_warp_bwd: bad dtype");
 }

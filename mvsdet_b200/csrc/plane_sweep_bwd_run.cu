@@ -808,96 +808,47 @@ __global__ void __launch_bounds__(kRunThreads, MINB) sweep_bwd_runs_kernel(const
   tmem_free_cta<kCols>(&s_tmem, warp);
 }
 
+// The hand-off kernel with two queue stages in dynamic shared memory.  The queue and the kernel's
+// static tables (its __shared__ declarations: samples, flag bytes, barriers, tensor-memory base) stay
+// within the 48 KB a launch gets without raising cudaFuncAttributeMaxDynamicSharedMemorySize.
+template <typename TIn, typename TG, int KMAX, int G, bool FULL, int MODE, bool PX>
+static void launch_runs(const SweepParams& p, dim3 grid, cudaStream_t st) {
+  constexpr size_t dyn = run_slot_bytes<KMAX, G, 2>();
+  constexpr size_t tables = sizeof(WarpSample) * kRunRows * 2 * 32 + kRunRows * 2 * 32 +
+                            sizeof(unsigned long long) * (kRunRows - 1) * KMAX * 2 * 2 + sizeof(uint32_t);
+  static_assert(dyn + tables <= 48 * 1024, "hand-off queue exceeds the default shared memory");
+  sweep_bwd_runs_kernel<TIn, TG, KMAX, G, FULL, kRunQMinBlocks, 2, MODE, PX><<<grid, kRunThreads, dyn, st>>>(p);
+}
+
 // k in {1,2} only (k*kRun <= 32 samples per plane); other k use the pixel kernel.
 // One run kernel is built per feature dtype: the hand-off kernel for bf16 features, the lean
 // kernel for fp32 features -- with fp32 features the raw loads of a pixel are 80 registers
 // instead of 44 and the pipelined kernel spills (ptxas: 160 B of stack).
-template <typename TIn, typename TG, bool PX>
+template <typename TIn, typename TG>
 static int launch_bwd_run_t(SweepParams& p, cudaStream_t st) {
-  const int G = sweep_groups(p.C);
-  p.tiles_x = (p.W + kRun - 1) / kRun;
-  p.tiles_y = (p.H + kRunRows - 1) / kRunRows;
-  p.slices = (p.C + 128 * G - 1) / (128 * G);
-  const long long blocks = (long long)p.V * p.slices * p.tiles_y * p.tiles_x;
-  if (blocks > 2147483647LL) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: grid too large");
-  dim3 grid((unsigned)blocks);
-  const bool full = p.C % (128 * G) == 0;
-#define MVSD_RUN(KM, GG, FU)                                                                \
-  do {                                                                                      \
-    if constexpr (sizeof(TIn) == 2) {                                                       \
-      auto kern = sweep_bwd_runs_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks, 2, 0, PX>;     \
-      constexpr size_t dyn = run_slot_bytes<KM, GG, 2>();                                   \
-      static bool attr_set = false;                                                         \
-      if (!attr_set) {                                                                      \
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);  \
-        attr_set = true;                                                                    \
-      }                                                                                     \
-      kern<<<grid, kRunThreads, dyn, st>>>(p);                                              \
-    } else {                                                                                \
-      sweep_bwd_runq_kernel<TIn, TG, KM, GG, FU, kRunQMinBlocks, PX><<<grid, kRunThreads, 0, st>>>(p); \
-    }                                                                                       \
-  } while (0)
-  if (p.k == 1) {
-    if (G == 2) { if (full) MVSD_RUN(1, 2, true); else MVSD_RUN(1, 2, false); }
-    else { if (full) MVSD_RUN(1, 1, true); else MVSD_RUN(1, 1, false); }
-  } else {
-    if (G == 2) { if (full) MVSD_RUN(2, 2, true); else MVSD_RUN(2, 2, false); }
-    else { if (full) MVSD_RUN(2, 1, true); else MVSD_RUN(2, 1, false); }
-  }
-#undef MVSD_RUN
-  count_launch();
-  return check_launch("plane_sweep_bwd(run)");
-}
-
-// Group-wise correlation backward (group_corr.cu) through the hand-off kernel: bf16 features, k = 2.
-// Returns -1 when this configuration is not built (the caller falls back to its pixel kernel).
-template <bool PX>
-static int launch_bwd_run_corr_t(SweepParams& p, cudaStream_t st) {
-  typedef __nv_bfloat16 TIn;
-  const int G = sweep_groups(p.C);
-  p.tiles_x = (p.W + kRun - 1) / kRun;
-  p.tiles_y = (p.H + kRunRows - 1) / kRunRows;
-  p.slices = (p.C + 128 * G - 1) / (128 * G);
-  const long long blocks = (long long)p.V * p.slices * p.tiles_y * p.tiles_x;
-  if (blocks > 2147483647LL) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_groupcorr_bwd: grid too large");
-  dim3 grid((unsigned)blocks);
-  const bool full = p.C % (128 * G) == 0;
-#define MVSD_RUNC(GG, FU)                                                                   \
-  do {                                                                                      \
-    auto kern = sweep_bwd_runs_kernel<TIn, float, 2, GG, FU, kRunQMinBlocks, 2, 1, PX>;     \
-    constexpr size_t dyn = run_slot_bytes<2, GG, 2>();                                      \
-    static bool attr_set = false;                                                           \
-    if (!attr_set) {                                                                        \
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);    \
-      attr_set = true;                                                                      \
-    }                                                                                       \
-    kern<<<grid, kRunThreads, dyn, st>>>(p);                                                \
-  } while (0)
-  if (G == 2) { if (full) MVSD_RUNC(2, true); else MVSD_RUNC(2, false); }
-  else { if (full) MVSD_RUNC(1, true); else MVSD_RUNC(1, false); }
-#undef MVSD_RUNC
-  count_launch();
-  return check_launch("plane_sweep_groupcorr_bwd(run)");
-}
-
-int launch_bwd_run_corr(SweepParams& p, int feat_dtype, cudaStream_t st) {
-  if (feat_dtype != MVSD_BF16 || p.k != 2) return -1;
-  return p.depth_per_pixel ? launch_bwd_run_corr_t<true>(p, st) : launch_bwd_run_corr_t<false>(p, st);
-}
-
-template <bool PX>
-static int launch_bwd_run_px(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st) {
-  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_run_t<float, float, PX>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16)
-    return launch_bwd_run_t<__nv_bfloat16, __nv_bfloat16, PX>(p, st);
-  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32)
-    return launch_bwd_run_t<__nv_bfloat16, float, PX>(p, st);
-  return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: dtype combination not built");
+  return sweep_launch(p, "plane_sweep_bwd", kRun, kRunRows, "plane_sweep_bwd(run)",
+                      [&](dim3 grid, auto G2, auto FULL, auto PX, auto K2) {
+    constexpr int KM = K2 ? 2 : 1, GG = G2 ? 2 : 1;
+    if constexpr (sizeof(TIn) == 2)
+      launch_runs<TIn, TG, KM, GG, FULL, 0, PX>(p, grid, st);
+    else
+      sweep_bwd_runq_kernel<TIn, TG, KM, GG, FULL, kRunQMinBlocks, PX><<<grid, kRunThreads, 0, st>>>(p);
+  }, p.k == 2);
 }
 
 int launch_bwd_run(SweepParams& p, int feat_dtype, int g_dtype, cudaStream_t st) {
-  return p.depth_per_pixel ? launch_bwd_run_px<true>(p, feat_dtype, g_dtype, st)
-                           : launch_bwd_run_px<false>(p, feat_dtype, g_dtype, st);
+  if (feat_dtype == MVSD_F32 && g_dtype == MVSD_F32) return launch_bwd_run_t<float, float>(p, st);
+  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_BF16) return launch_bwd_run_t<__nv_bfloat16, __nv_bfloat16>(p, st);
+  if (feat_dtype == MVSD_BF16 && g_dtype == MVSD_F32) return launch_bwd_run_t<__nv_bfloat16, float>(p, st);
+  return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_bwd: dtype combination not built");
+}
+
+// Group-wise correlation backward (group_corr.cu) through the hand-off kernel, MODE 1: bf16 features, k = 2.
+int launch_bwd_run_corr(SweepParams& p, cudaStream_t st) {
+  return sweep_launch(p, "plane_sweep_groupcorr_bwd", kRun, kRunRows, "plane_sweep_groupcorr_bwd(run)",
+                      [&](dim3 grid, auto G2, auto FULL, auto PX) {
+    launch_runs<__nv_bfloat16, float, 2, G2 ? 2 : 1, FULL, 1, PX>(p, grid, st);
+  });
 }
 
 }  // namespace mvsd

@@ -235,7 +235,9 @@ __global__ void __launch_bounds__(kFwdThreads, 8) sweep_fwd_p_kernel(const Sweep
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-int sweep_check(const char* who, int V, int C, int D, int H, int W, int k, int layout) {
+int sweep_setup(SweepParams& p, const char* who, std::initializer_list<const void*> bufs, bool need_nbr,
+                const void* feat, const int32_t* nbr, const float* hom, const float* depth, int V, int C,
+                int D, int H, int W, int k, int layout, int ref_begin, int n_feat, bool per_pixel) {
   if (V <= 0 || C <= 0 || D <= 0 || H <= 0 || W <= 0 || k < 0)
     return fail(MVSD_ERR_INVALID_ARG, "%s: non-positive dimension", who);
   if (C % 4 != 0 || C > MVSD_MAX_C)
@@ -245,64 +247,45 @@ int sweep_check(const char* who, int V, int C, int D, int H, int W, int k, int l
     return fail(MVSD_ERR_UNSUPPORTED, "%s: one feature map must stay below 2^31 elements", who);
   if (layout != MVSD_CHANNELS_LAST)
     return fail(MVSD_ERR_UNSUPPORTED, "%s: only MVSD_CHANNELS_LAST volumes are implemented", who);
+  bool null = !depth || (need_nbr && (!nbr || !hom));
+  for (const void* b : bufs) null = null || !b;
+  if (null) return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (ref_begin < 0 || (long long)ref_begin + V > n_feat)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
+                who, ref_begin, ref_begin + V, n_feat);
+  p = SweepParams{};
+  p.feat = feat; p.nbr = nbr; p.hom = hom; p.depth = depth;
+  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat;
+  p.depth_per_pixel = per_pixel ? 1 : 0;
   return MVSD_OK;
 }
 
-// Channel groups (of 128) per warp: 2 keeps all 256 FPN channels of a tap in one
-// warp (fewest instructions per byte).
-int sweep_groups(int C) { return C > 128 ? 2 : 1; }
-
-bool sweep_grid(SweepParams& p, int G, dim3& grid) {
-  p.tiles_x = (p.W + kPatchW - 1) / kPatchW;
-  p.tiles_y = (p.H + kPatchH - 1) / kPatchH;
+int sweep_grid(SweepParams& p, const char* who, int tile_w, int tile_h, int G, dim3& grid) {
+  p.tiles_x = (p.W + tile_w - 1) / tile_w;
+  p.tiles_y = (p.H + tile_h - 1) / tile_h;
   p.slices = (p.C + 128 * G - 1) / (128 * G);
   const long long blocks = (long long)p.V * p.slices * p.tiles_y * p.tiles_x;
-  if (blocks > 2147483647LL) return false;
+  if (blocks > 2147483647LL) return fail(MVSD_ERR_UNSUPPORTED, "%s: grid too large", who);
   grid = dim3((unsigned)blocks);
-  return true;
+  return MVSD_OK;
 }
 
 template <typename TIn, typename TOut, bool WARP_ONLY>
 static int launch_fwd_k(SweepParams& p, cudaStream_t st) {
-  dim3 grid;
-  const int G = sweep_groups(p.C);
-  if (!sweep_grid(p, G, grid)) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_fwd: grid too large");
-  if constexpr (!WARP_ONLY) {                 // the packed kernel has its own CTA patch
-    p.tiles_x = (p.W + kFwdPatchW - 1) / kFwdPatchW;
-    p.tiles_y = (p.H + kFwdPatchH - 1) / kFwdPatchH;
-    const long long blocks = (long long)p.V * p.slices * p.tiles_y * p.tiles_x;
-    if (blocks > 2147483647LL) return fail(MVSD_ERR_UNSUPPORTED, "plane_sweep_fwd: grid too large");
-    grid = dim3((unsigned)blocks);
-  }
-  const bool full = p.C % (128 * G) == 0;
-  const int kmax = WARP_ONLY ? 1 : (p.k <= 1 ? 1 : (p.k == 2 ? 2 : 4));
-#define MVSD_FWD(KM, GG, FU)                                                           \
-  do {                                                                                 \
-    if constexpr (WARP_ONLY)                                                           \
-      sweep_fwd_kernel<TIn, TOut, KM, GG, FU, true><<<grid, kSweepThreads, 0, st>>>(p); \
-    else if (p.depth_per_pixel)                                                        \
-      sweep_fwd_p_kernel<TIn, TOut, KM, GG, FU, true><<<grid, kFwdThreads, 0, st>>>(p); \
-    else                                                                               \
-      sweep_fwd_p_kernel<TIn, TOut, KM, GG, FU, false><<<grid, kFwdThreads, 0, st>>>(p); \
-  } while (0)
-#define MVSD_FWD_G(KM)                                                            \
-  do {                                                                            \
-    if (G == 2) { if (full) MVSD_FWD(KM, 2, true); else MVSD_FWD(KM, 2, false); } \
-    else { if (full) MVSD_FWD(KM, 1, true); else MVSD_FWD(KM, 1, false); }        \
-  } while (0)
-  if constexpr (WARP_ONLY) {
-    MVSD_FWD_G(1);                        // stand-alone warp: the scalar kernel, one source
-  } else {
+  return sweep_launch(p, "plane_sweep_fwd", WARP_ONLY ? kPatchW : kFwdPatchW, WARP_ONLY ? kPatchH : kFwdPatchH,
+                      "plane_sweep_fwd", [&](dim3 grid, auto G2, auto FULL, auto PX) {
+    constexpr int GG = G2 ? 2 : 1;
+    if constexpr (WARP_ONLY)              // stand-alone warp: the scalar kernel, one source, either depth form
+      sweep_fwd_kernel<TIn, TOut, 1, GG, FULL, true><<<grid, kSweepThreads, 0, st>>>(p);
     // k = 2 is the reference's configuration (mvsdet.py:432) and gets the un-predicated
     // instantiation; k = 0, 1 (one- and two-view scenes) and k = 3, 4 share the predicated ones
-    if (kmax == 2) MVSD_FWD_G(2);
-    else if (kmax == 1) { if (G == 2) MVSD_FWD(1, 2, false); else MVSD_FWD(1, 1, false); }
-    else { if (G == 2) MVSD_FWD(4, 2, false); else MVSD_FWD(4, 1, false); }
-  }
-#undef MVSD_FWD_G
-#undef MVSD_FWD
-  count_launch();
-  return check_launch("plane_sweep_fwd");
+    else if (p.k == 2)
+      sweep_fwd_p_kernel<TIn, TOut, 2, GG, FULL, PX><<<grid, kFwdThreads, 0, st>>>(p);
+    else if (p.k <= 1)
+      sweep_fwd_p_kernel<TIn, TOut, 1, GG, false, PX><<<grid, kFwdThreads, 0, st>>>(p);
+    else
+      sweep_fwd_p_kernel<TIn, TOut, 4, GG, false, PX><<<grid, kFwdThreads, 0, st>>>(p);
+  });
 }
 
 template <bool WARP_ONLY>
@@ -326,16 +309,11 @@ static int plane_sweep_fwd(const char* who, const void* feat, int feat_dtype, co
                            const float* hom, const float* depth_values, void* out, int out_dtype,
                            int out_layout, int V, int C, int D, int H, int W, int k, int ref_begin,
                            int n_feat_views, bool per_pixel, void* stream) {
-  if (int e = sweep_check(who, V, C, D, H, W, k, out_layout)) return e;
-  if (!feat || !out || !depth_values || (k > 0 && (!nbr_ids || !hom)))
-    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (ref_begin < 0 || (long long)ref_begin + V > n_feat_views)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: reference views [%d, %d) exceed the %d feature views",
-                who, ref_begin, ref_begin + V, n_feat_views);
-  SweepParams p{};
-  p.feat = feat; p.nbr = nbr_ids; p.hom = hom; p.depth = depth_values; p.out = out;
-  p.V = V; p.C = C; p.D = D; p.H = H; p.W = W; p.k = k; p.ref_begin = ref_begin; p.n_feat = n_feat_views;
-  p.depth_per_pixel = per_pixel ? 1 : 0;
+  SweepParams p;
+  if (int e = sweep_setup(p, who, {feat, out}, k > 0, feat, nbr_ids, hom, depth_values, V, C, D, H, W, k,
+                          out_layout, ref_begin, n_feat_views, per_pixel))
+    return e;
+  p.out = out;
   return launch_fwd<false>(p, feat_dtype, out_dtype, static_cast<cudaStream_t>(stream));
 }
 
@@ -359,12 +337,10 @@ extern "C" int mvsd_homo_warp_fwd(const void* src, int src_dtype, const float* h
                                   const float* depth_values, void* out, int out_dtype,
                                   int out_layout, int B, int C, int D, int H, int W,
                                   int depth_per_pixel, void* stream) {
-  if (int e = sweep_check("homo_warp_fwd", B, C, D, H, W, 1, out_layout)) return e;
-  if (!src || !hom || !depth_values || !out)
-    return fail(MVSD_ERR_INVALID_ARG, "homo_warp_fwd: null pointer");
-  SweepParams p{};
-  p.feat = src; p.nbr = nullptr; p.hom = hom; p.depth = depth_values; p.out = out;
-  p.V = B; p.C = C; p.D = D; p.H = H; p.W = W; p.k = 1; p.ref_begin = 0; p.n_feat = B;
-  p.depth_per_pixel = depth_per_pixel ? 1 : 0;
+  SweepParams p;
+  if (int e = sweep_setup(p, "homo_warp_fwd", {src, hom, out}, false, src, nullptr, hom, depth_values, B, C, D, H,
+                          W, 1, out_layout, 0, B, depth_per_pixel != 0))
+    return e;
+  p.out = out;
   return launch_fwd<true>(p, src_dtype, out_dtype, static_cast<cudaStream_t>(stream));
 }
