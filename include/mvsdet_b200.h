@@ -30,7 +30,9 @@
  * Additive symbols (no ABI version change; every earlier signature is unchanged):
  *   mvsd_plane_sweep_fwd_px, mvsd_plane_sweep_bwd_px, mvsd_plane_sweep_bwd_det_px,
  *   mvsd_plane_sweep_groupcorr_fwd_px, mvsd_plane_sweep_groupcorr_bwd_px --
- *   the fused sweeps with per-pixel depth hypotheses.
+ *   the fused sweeps with per-pixel depth hypotheses;
+ *   mvsd_depth_topk_fwd_px, mvsd_depth_topk_bwd_px -- the top-k epilogue over
+ *   per-pixel depth hypotheses.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -277,6 +279,43 @@ int mvsd_depth_topk_bwd(const float* cost_out, int64_t s_v, int64_t s_c,
                         float* g_cost_out,
                         float near, float interval, int raw,
                         int V, int D, int H, int W, int T, void* stream);
+/* The top-k epilogue over per-pixel depth hypotheses, e.g. the fine cost volume
+ * of a second sweep around est_depth (mvsd_plane_sweep_fwd_px).  Arguments as
+ * mvsd_depth_topk_fwd / _bwd, except that the planes d*interval + near are
+ * replaced by
+ *   depth_values  [V,D,H,W] fp32 contiguous (required): z_d of each pixel, in
+ *                 any order along D (est_idx indexes this axis)
+ *   interval_map  [V,H,W] fp32 contiguous offset scale I per pixel, or NULL:
+ *                 I = interval
+ * depth_d = z_d + off_d*I (two roundings).  Selection, NaN rule, expectation
+ * order and NVS epilogue are those of mvsd_depth_topk_fwd; a NaN z_d propagates
+ * into the depths that use it.  Planes z_d = fl(fl(d*interval) + near) with
+ * I = interval (scalar or constant map) give the per-view call's bits, forward
+ * and g_cost_out.
+ * Backward, in addition to g_cost_out (both optional, fully overwritten):
+ *   g_depth_values [V,D,H,W]  dL/dz_d = g_coding*p_d + sum_t [d == idx_t] g_est_depth_t
+ *   g_interval_map [V,H,W]    dL/dI = g_coding*sum_d p_d off_d + sum_t g_est_depth_t off_idx_t
+ *                             (requires interval_map)
+ * where g_coding and g_est_depth include the ray-depth terms. */
+int mvsd_depth_topk_fwd_px(const float* cost_out, int64_t s_v, int64_t s_c,
+                           int64_t s_d, int64_t s_p,
+                           const float* depth_values, const float* interval_map, float interval,
+                           float* prob_volume, float* off_pred, float* est_depth,
+                           float* est_dens, int64_t* est_idx, float* depth_coding,
+                           const float* ray_intrinsics, int ray_per_view,
+                           float* opacity, float* depth_scale, float* est_ray_depth,
+                           float* ray_depth_coding,
+                           int raw, int V, int D, int H, int W, int T, void* stream);
+int mvsd_depth_topk_bwd_px(const float* cost_out, int64_t s_v, int64_t s_c,
+                           int64_t s_d, int64_t s_p, const int64_t* est_idx,
+                           const float* depth_values, const float* interval_map, float interval,
+                           const float* g_prob_volume, const float* g_off_pred,
+                           const float* g_est_depth, const float* g_est_dens,
+                           const float* g_depth_coding,
+                           const float* ray_intrinsics, int ray_per_view,
+                           const float* g_est_ray_depth, const float* g_ray_depth_coding,
+                           float* g_cost_out, float* g_depth_values, float* g_interval_map,
+                           int raw, int V, int D, int H, int W, int T, void* stream);
 
 /* compute_depth_scale / compute_depth_scale_MultiIntrin alone (mvsdet.py:1158-1218):
  * depth_scale [V,H,W] from [4,4] or (per_view) [V,4,4] feature-level intrinsics. */

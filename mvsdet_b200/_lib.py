@@ -51,6 +51,10 @@ SIGNATURES = {
                              _f, _f, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_depth_topk_bwd": ([_p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p,
                              _f, _f, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_depth_topk_fwd_px": ([_p, _l, _l, _l, _l, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p,
+                                _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_depth_topk_bwd_px": ([_p, _l, _l, _l, _l, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p,
+                                _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_ray_depth_scale": ([_p, _i, _p, _i, _i, _i, _p], _i),
     "mvsd_rgb_downsample4": ([_p, _p, _i, _p, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_backproject_fwd": ([_p, _i, _i, _i, _p, _p, _p, _p, _l, _l, _l, _l, _f, _i, _p, _i,
@@ -188,25 +192,45 @@ def homo_warp_bwd(g, hom, depth_values, g_src):
          g_src.data_ptr(), b, c, depth_values.shape[1], h, w, int(depth_values.dim() == 4), _stream())
 
 
+def _interval(interval):
+    """-> (interval_map or None, scalar interval) for the *_px entry points"""
+    return (interval, 0.0) if isinstance(interval, torch.Tensor) else (None, float(interval))
+
+
 def depth_topk_fwd(cost_out, prob, off, est_depth, est_dens, est_idx, coding, *, near, interval, raw=False,
-                   ray_intr=None, nvs=(None,) * 4):
+                   ray_intr=None, nvs=(None,) * 4, depth_values=None):
     """cost_out [V,2,D,H,W] -> [V,D,H,W], [V,T,H,W] and [V,H,W] outputs (prob, off, coding may be
-    None); with ``ray_intr`` also ``nvs`` = (opacity, depth_scale, est_ray_depth, ray_depth_coding)"""
+    None); with ``ray_intr`` also ``nvs`` = (opacity, depth_scale, est_ray_depth, ray_depth_coding).
+    ``depth_values`` [V,D,H,W]: per-pixel hypotheses (mvsd_depth_topk_fwd_px); ``near`` is then unused
+    and ``interval`` is a float or an [V,H,W] map."""
     v, _, d, h, w = cost_out.shape
     sv, sc, sd, _, sp = cost_out.stride()
-    call("mvsd_depth_topk_fwd", cost_out.data_ptr(), sv, sc, sd, sp, _ptr(prob), _ptr(off), est_depth.data_ptr(),
-         est_dens.data_ptr(), est_idx.data_ptr(), _ptr(coding), _ptr(ray_intr), _per_view(ray_intr),
-         *map(_ptr, nvs), float(near), float(interval), int(raw), v, d, h, w, est_depth.shape[1], _stream())
+    outs = (_ptr(prob), _ptr(off), est_depth.data_ptr(), est_dens.data_ptr(), est_idx.data_ptr(), _ptr(coding),
+            _ptr(ray_intr), _per_view(ray_intr), *map(_ptr, nvs))
+    dims = (int(raw), v, d, h, w, est_depth.shape[1], _stream())
+    if depth_values is None:
+        call("mvsd_depth_topk_fwd", cost_out.data_ptr(), sv, sc, sd, sp, *outs, float(near), float(interval), *dims)
+    else:
+        imap, ival = _interval(interval)
+        call("mvsd_depth_topk_fwd_px", cost_out.data_ptr(), sv, sc, sd, sp, depth_values.data_ptr(), _ptr(imap),
+             ival, *outs, *dims)
 
 
 def depth_topk_bwd(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, g_cost, *, near, interval,
-                   raw=False, ray_intr=None, g_ray_depth=None, g_ray_coding=None):
+                   raw=False, ray_intr=None, g_ray_depth=None, g_ray_coding=None, depth_values=None,
+                   g_depth_values=None, g_interval_map=None):
     v, _, d, h, w = cost_out.shape
     sv, sc, sd, _, sp = cost_out.stride()
-    call("mvsd_depth_topk_bwd", cost_out.data_ptr(), sv, sc, sd, sp, est_idx.data_ptr(), _ptr(g_prob), _ptr(g_off),
-         _ptr(g_depth), _ptr(g_dens), _ptr(g_coding), _ptr(ray_intr), _per_view(ray_intr), _ptr(g_ray_depth),
-         _ptr(g_ray_coding), g_cost.data_ptr(), float(near), float(interval), int(raw), v, d, h, w,
-         est_idx.shape[1], _stream())
+    grads = (_ptr(g_prob), _ptr(g_off), _ptr(g_depth), _ptr(g_dens), _ptr(g_coding), _ptr(ray_intr),
+             _per_view(ray_intr), _ptr(g_ray_depth), _ptr(g_ray_coding), g_cost.data_ptr())
+    dims = (int(raw), v, d, h, w, est_idx.shape[1], _stream())
+    if depth_values is None:
+        call("mvsd_depth_topk_bwd", cost_out.data_ptr(), sv, sc, sd, sp, est_idx.data_ptr(), *grads, float(near),
+             float(interval), *dims)
+    else:
+        imap, ival = _interval(interval)
+        call("mvsd_depth_topk_bwd_px", cost_out.data_ptr(), sv, sc, sd, sp, est_idx.data_ptr(),
+             depth_values.data_ptr(), _ptr(imap), ival, *grads, _ptr(g_depth_values), _ptr(g_interval_map), *dims)
 
 
 def ray_depth_scale(intrinsics, out):

@@ -102,10 +102,24 @@ class MVSDetHotPath(nn.Module):
                                         out_dtype=self.variance_dtype, ref_begin=ref_begin,
                                         grad_sink=grad_sink)
 
-    def hypotheses(self, cost_out: torch.Tensor, k_feat: Optional[torch.Tensor] = None):
+    def hypotheses(self, cost_out: torch.Tensor, k_feat: Optional[torch.Tensor] = None,
+                   depth_values: Optional[torch.Tensor] = None, interval=None):
         """(prob_volume, off_pred, est_depth, est_densities, est_idx, depth_coding); with the
         feature-level intrinsics ``k_feat`` also the NVS-branch outputs (opacity, depth_scale,
-        est_ray_depth, ray_depth_coding) from the same kernel (mvsdet.py:494, :579, :583)."""
+        est_ray_depth, ray_depth_coding) from the same kernel (mvsdet.py:494, :579, :583).
+        ``depth_values`` [V,D,Hf,Wf]: the per-pixel planes the cost volume was swept over (a second
+        sweep, ``variance(..., depth_values=)``), with ``interval`` their offset scale -- a float or
+        an [V,Hf,Wf] map; the scene's interval is no default for them.  Both may carry gradients."""
+        if depth_values is not None:
+            if interval is None:
+                raise ValueError("per-pixel depth_values need their own interval (a float or an [V,H,W] map)")
+            if k_feat is not None:
+                return ops.depth_topk_nvs(cost_out, 0.0, interval, self.topk, k_feat, depth_values=depth_values)
+            if self.dispatcher_ops:
+                if isinstance(interval, torch.Tensor):
+                    return library.depth_topk_px(cost_out, depth_values, interval, 0.0, self.topk)
+                return library.depth_topk_px(cost_out, depth_values, None, float(interval), self.topk)
+            return ops.depth_topk(cost_out, 0.0, interval, self.topk, depth_values=depth_values)
         if k_feat is not None:
             return ops.depth_topk_nvs(cost_out, self.near_far_range[0], self.depth_interval, self.topk, k_feat)
         if self.dispatcher_ops:

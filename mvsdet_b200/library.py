@@ -25,6 +25,9 @@ Operators (reference lines as in ``ops.py``):
   depth_topk(cost_out, near, interval, topk, raw=False)
       -> (prob_volume, off_pred, est_depth, est_densities, est_idx, depth_coding)
       mvsdet.py:470-482, :266-283, :298-317
+  depth_topk_px(cost_out, depth_values, interval_map, interval, topk, raw=False) -> the same six
+      over per-pixel hypotheses [V,D,H,W] with an [V,H,W] interval map (or None: the scalar);
+      its backward also gives dL/ddepth_values and dL/dinterval_map
   backproject_aggregate(feat, points, projection, est_depth, est_dens, vs_z, height, width,
                         sum_only=False, channels_first=True) -> (volume, count)
       mvsdet.py:1372-1492, :511-515, :681-682 (sum_only: the multi-GPU partials)
@@ -40,8 +43,8 @@ from torch import Tensor
 from . import ops as _ops
 from ._lib import BP_MEAN, BP_SUM
 
-__all__ = ["plane_sweep_variance", "plane_sweep_group_correlation", "depth_topk", "backproject_aggregate",
-           "voxel_normalize"]
+__all__ = ["plane_sweep_variance", "plane_sweep_group_correlation", "depth_topk", "depth_topk_px",
+           "backproject_aggregate", "voxel_normalize"]
 
 _NS = "mvsdet_b200"
 
@@ -143,6 +146,15 @@ plane_sweep_group_correlation.register_autograd(_corr_backward, setup_context=_c
 # --------------------------------------------------------------------------
 # softmax / sigmoid / top-k / expectation
 # --------------------------------------------------------------------------
+def _topk_outputs(cost_out, topk):
+    v, _, d, h, w = cost_out.shape
+    f32 = dict(dtype=torch.float32, device=cost_out.device)
+    return (torch.empty((v, d, h, w), **f32), torch.empty((v, d, h, w), **f32),
+            torch.empty((v, topk, h, w), **f32), torch.empty((v, topk, h, w), **f32),
+            torch.empty((v, topk, h, w), dtype=torch.int64, device=cost_out.device),
+            torch.empty((v, h, w), **f32))
+
+
 @torch.library.custom_op(f"{_NS}::depth_topk", mutates_args=(), device_types="cuda")
 def depth_topk(cost_out: Tensor, near: float, interval: float, topk: int,
                raw: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
@@ -153,12 +165,7 @@ def depth_topk(cost_out: Tensor, near: float, interval: float, topk: int,
 
 @depth_topk.register_fake
 def _(cost_out, near, interval, topk, raw=False):
-    v, _, d, h, w = cost_out.shape
-    f32 = dict(dtype=torch.float32, device=cost_out.device)
-    return (torch.empty((v, d, h, w), **f32), torch.empty((v, d, h, w), **f32),
-            torch.empty((v, topk, h, w), **f32), torch.empty((v, topk, h, w), **f32),
-            torch.empty((v, topk, h, w), dtype=torch.int64, device=cost_out.device),
-            torch.empty((v, h, w), **f32))
+    return _topk_outputs(cost_out, topk)
 
 
 @torch.library.custom_op(f"{_NS}::depth_topk_bwd", mutates_args=(), device_types="cuda")
@@ -192,6 +199,68 @@ def _topk_backward(ctx, g_prob, g_off, g_depth, g_dens, _g_idx, g_coding):
 
 
 depth_topk.register_autograd(_topk_backward, setup_context=_topk_setup)
+
+
+@torch.library.custom_op(f"{_NS}::depth_topk_px", mutates_args=(), device_types="cuda")
+def depth_topk_px(cost_out: Tensor, depth_values: Tensor, interval_map: Optional[Tensor], interval: float,
+                  topk: int, raw: bool = False) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    iv = interval if interval_map is None else interval_map
+    _ops._check_topk_px("cost_out", cost_out, depth_values, iv)
+    _, outs = _ops._topk_fwd_raw(cost_out, None, iv if interval_map is None else interval_map.contiguous(),
+                                 int(topk), int(raw), depth_values=depth_values.contiguous())
+    return outs
+
+
+@depth_topk_px.register_fake
+def _(cost_out, depth_values, interval_map, interval, topk, raw=False):
+    return _topk_outputs(cost_out, topk)
+
+
+@torch.library.custom_op(f"{_NS}::depth_topk_px_bwd", mutates_args=(), device_types="cuda")
+def depth_topk_px_bwd(cost_out: Tensor, est_idx: Tensor, depth_values: Tensor, interval_map: Optional[Tensor],
+                      g_prob: Optional[Tensor], g_off: Optional[Tensor], g_depth: Optional[Tensor],
+                      g_dens: Optional[Tensor], g_coding: Optional[Tensor], interval: float,
+                      raw: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """-> (dL/dcost_out, dL/ddepth_values, dL/dinterval_map: [V,H,W], or [0] without a map)"""
+    depth_values = depth_values.contiguous()
+    g_dv = torch.empty_like(depth_values)
+    if interval_map is None:
+        g_im = torch.empty((0,), dtype=torch.float32, device=cost_out.device)
+        iv = interval
+    else:
+        iv = interval_map.contiguous()
+        g_im = torch.empty_like(iv)
+    g_cost = _ops._topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, None, iv, int(raw),
+                                depth_values=depth_values, g_depth_values=g_dv,
+                                g_interval_map=None if interval_map is None else g_im)
+    return g_cost, g_dv, g_im
+
+
+@depth_topk_px_bwd.register_fake
+def _(cost_out, est_idx, depth_values, interval_map, g_prob, g_off, g_depth, g_dens, g_coding, interval, raw):
+    v, _, d, h, w = cost_out.shape
+    f32 = dict(dtype=torch.float32, device=cost_out.device)
+    return (torch.empty((v, 2, d, h, w), **f32), torch.empty((v, d, h, w), **f32),
+            torch.empty((0,) if interval_map is None else (v, h, w), **f32))
+
+
+def _topk_px_setup(ctx, inputs, output):
+    cost_out, depth_values, interval_map, interval, topk, raw = inputs
+    ctx.save_for_backward(cost_out, output[4], depth_values, interval_map)
+    ctx.consts = (float(interval), bool(raw))
+
+
+def _topk_px_backward(ctx, g_prob, g_off, g_depth, g_dens, _g_idx, g_coding):
+    cost_out, est_idx, depth_values, interval_map = ctx.saved_tensors
+    interval, raw = ctx.consts
+    g_cost, g_dv, g_im = depth_topk_px_bwd(cost_out, est_idx, depth_values, interval_map, g_prob, g_off, g_depth,
+                                           g_dens, g_coding, interval, raw)
+    if g_cost.dtype != cost_out.dtype:
+        g_cost = g_cost.to(cost_out.dtype)
+    return g_cost, g_dv, (None if interval_map is None else g_im), None, None, None
+
+
+depth_topk_px.register_autograd(_topk_px_backward, setup_context=_topk_px_setup)
 
 
 # --------------------------------------------------------------------------

@@ -14,6 +14,7 @@ kernels (and cuDNN's Conv3d after them) want.
 """
 from __future__ import annotations
 
+import numbers
 from typing import Optional, Tuple
 
 import torch
@@ -430,9 +431,10 @@ def _ray_intr(ray_intr, v):
     raise ValueError(f"ray intrinsics must be [4,4] or [{v},4,4], got {tuple(ray_intr.shape)}")
 
 
-def _topk_fwd_raw(cost_out, near, interval, topk, raw, ray_intr=None):
+def _topk_fwd_raw(cost_out, near, interval, topk, raw, ray_intr=None, depth_values=None):
     """-> (cost_out as the kernel read it, the six outputs, and with ``ray_intr`` the four NVS
-    outputs opacity, depth_scale, est_ray_depth, ray_depth_coding)"""
+    outputs opacity, depth_scale, est_ray_depth, ray_depth_coding).  ``depth_values``: per-pixel
+    hypotheses [V,D,H,W] (``interval`` a float or an [V,H,W] map, ``near`` unused)."""
     cost_out = _as_cost(cost_out)
     v, _, d, h, w = cost_out.shape
     dev = cost_out.device
@@ -449,13 +451,17 @@ def _topk_fwd_raw(cost_out, near, interval, topk, raw, ray_intr=None):
         nvs = (torch.empty((v, h, w), **f32), torch.empty((v, h, w), **f32),
                torch.empty((v, topk, h, w), **f32), torch.empty((v, h, w), **f32))
     _lib.depth_topk_fwd(cost_out, prob, off, est_depth, est_dens, est_idx, coding, near=near,
-                        interval=interval, raw=raw, ray_intr=kmat, nvs=nvs or (None,) * 4)
+                        interval=interval, raw=raw, ray_intr=kmat, nvs=nvs or (None,) * 4,
+                        depth_values=depth_values)
     return cost_out, (prob, off, est_depth, est_dens, est_idx, coding) + nvs
 
 
 def _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, near, interval,
-                  raw, ray_intr=None, g_ray_depth=None, g_ray_coding=None):
-    """-> dL/dcost_out (any of the upstream gradients may be None)"""
+                  raw, ray_intr=None, g_ray_depth=None, g_ray_coding=None, depth_values=None,
+                  g_depth_values=None, g_interval_map=None):
+    """-> dL/dcost_out (any of the upstream gradients may be None).  With per-pixel
+    ``depth_values`` the kernel also overwrites the given ``g_depth_values`` [V,D,H,W] and
+    ``g_interval_map`` [V,H,W] buffers."""
     cost_out = _as_cost(cost_out)
 
     def prep(g):
@@ -466,7 +472,8 @@ def _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, n
     g_cost = torch.empty(cost_out.shape, dtype=torch.float32, device=cost_out.device)
     _lib.depth_topk_bwd(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, g_cost, near=near,
                         interval=interval, raw=raw, ray_intr=kmat, g_ray_depth=g_ray_depth,
-                        g_ray_coding=g_ray_coding)
+                        g_ray_coding=g_ray_coding, depth_values=depth_values, g_depth_values=g_depth_values,
+                        g_interval_map=g_interval_map)
     return g_cost
 
 
@@ -474,6 +481,24 @@ def _check_cost(name, cost_out) -> None:
     _need_cuda(name, cost_out)
     if cost_out.dim() != 5 or cost_out.shape[1] != 2:
         raise ValueError(f"{name} must be [V,2,D,H,W]")
+
+
+def _check_topk_px(name, cost_out, depth_values, interval) -> None:
+    """the top-k over per-pixel hypotheses: depth_values fp32 CUDA [V,D,H,W] with the cost volume's
+    V, D, H, W; interval a number or an fp32 CUDA [V,H,W] map"""
+    _check_cost(name, cost_out)
+    _need_cuda("depth_values", depth_values)
+    v, _, d, h, w = cost_out.shape
+    if depth_values.dtype != torch.float32 or tuple(depth_values.shape) != (v, d, h, w):
+        raise ValueError(f"depth_values must be float32 [V,D,H,W] = {[v, d, h, w]} (the cost volume's), "
+                         f"got {depth_values.dtype} {list(depth_values.shape)}")
+    if isinstance(interval, torch.Tensor):
+        _need_cuda("interval", interval)
+        if interval.dtype != torch.float32 or tuple(interval.shape) != (v, h, w):
+            raise ValueError(f"an interval map must be float32 [V,H,W] = {[v, h, w]}, "
+                             f"got {interval.dtype} {list(interval.shape)}")
+    elif not isinstance(interval, numbers.Real):
+        raise ValueError("interval must be a number or an [V,H,W] tensor")
 
 
 class _DepthTopk(torch.autograd.Function):
@@ -519,17 +544,64 @@ class _DepthTopkNVS(torch.autograd.Function):
         return g_cost, None, None, None, None
 
 
-def depth_topk(cost_out: torch.Tensor, near: float, interval: float, topk: int):
+class _DepthTopkPX(torch.autograd.Function):
+    """depth_topk (``ray_intr`` None) or depth_topk_nvs over per-pixel hypotheses: z_d =
+    depth_values[v,d,y,x] and I = interval_map[v,y,x] (or the scalar ``interval``) in place of
+    d*interval + near and interval.  Gradients also reach depth_values and the interval map."""
+
+    @staticmethod
+    def forward(ctx, cost_out, depth_values, interval_map, interval, topk, raw, ray_intr):
+        iv = interval if interval_map is None else interval_map
+        cost_out, outs = _topk_fwd_raw(cost_out, None, iv, topk, raw, ray_intr, depth_values)
+        ctx.save_for_backward(cost_out, outs[4], depth_values, interval_map, ray_intr)
+        ctx.consts = (float(interval), int(raw))
+        ctx.mark_non_differentiable(*outs[4:5], *outs[7:8])
+        return outs
+
+    @staticmethod
+    def backward(ctx, g_prob, g_off, g_depth, g_dens, _g_idx, g_coding, g_opacity=None, _g_scale=None,
+                 g_ray_depth=None, g_ray_coding=None):
+        cost_out, est_idx, depth_values, interval_map, ray_intr = ctx.saved_tensors
+        interval, raw = ctx.consts
+        if g_opacity is not None:                      # opacity == est_dens[:, 0]
+            g_dens = torch.zeros_like(est_idx, dtype=torch.float32) if g_dens is None else g_dens.clone()
+            g_dens[:, 0] += g_opacity
+        g_dv = torch.empty_like(depth_values) if ctx.needs_input_grad[1] else None
+        g_im = torch.empty_like(interval_map) if ctx.needs_input_grad[2] else None
+        g_cost = _topk_bwd_raw(cost_out, est_idx, g_prob, g_off, g_depth, g_dens, g_coding, None,
+                               interval if interval_map is None else interval_map, raw, ray_intr, g_ray_depth,
+                               g_ray_coding, depth_values, g_dv, g_im)
+        return g_cost, g_dv, g_im, None, None, None, None
+
+
+def _depth_topk_px(name, cost_out, depth_values, interval, topk, raw, kmat=None):
+    _check_topk_px(name, cost_out, depth_values, interval)
+    imap = interval.contiguous() if isinstance(interval, torch.Tensor) else None
+    return _DepthTopkPX.apply(cost_out, depth_values.contiguous(), imap, 0.0 if imap is not None else float(interval),
+                              int(topk), raw, kmat)
+
+
+def depth_topk(cost_out: torch.Tensor, near: float, interval, topk: int,
+               depth_values: Optional[torch.Tensor] = None):
     """Fused mvsdet.py:470-482 + sample_depth_prob (:266-283) + compute_avg_depth
     (:298-317).  cost_out [V,2,D,H,W] -> (prob_volume [V,D,H,W], off_pred
     [V,D,H,W], est_depth [V,T,H,W], est_densities [V,T,H,W], est_idx int64
-    [V,T,H,W], depth_coding [V,H,W])."""
+    [V,T,H,W], depth_coding [V,H,W]).
+
+    ``depth_values`` [V,D,H,W] fp32: per-pixel hypotheses (e.g. the planes of a second sweep around
+    ``est_depth``) in place of the planes d*interval + near.  Hypothesis d of pixel (x, y) then lies at
+    depth_values[v,d,y,x] + off_pred * I, with I = ``interval`` (a float, or an fp32 [V,H,W] map of
+    per-pixel spacings); ``near`` is ignored and ``est_idx`` indexes the D axis of depth_values, which
+    need not be sorted.  Gradients reach depth_values and an interval map, so planes built from an
+    earlier ``est_depth`` may stay attached."""
+    if depth_values is not None:
+        return _depth_topk_px("cost_out", cost_out, depth_values, interval, topk, 0)
     _check_cost("cost_out", cost_out)
     return _DepthTopk.apply(cost_out, near, interval, int(topk), 0)
 
 
-def depth_topk_nvs(cost_out: torch.Tensor, near: float, interval: float, topk: int,
-                   k_feat: torch.Tensor):
+def depth_topk_nvs(cost_out: torch.Tensor, near: float, interval, topk: int,
+                   k_feat: torch.Tensor, depth_values: Optional[torch.Tensor] = None):
     """``depth_topk`` with the NVS-branch consumers computed in the same kernel (SURVEY.md 8f
     rank 3).  ``k_feat``: feature-level intrinsics [4,4] or [V,4,4].  Returns the six outputs of
     ``depth_topk`` followed by
@@ -537,9 +609,12 @@ def depth_topk_nvs(cost_out: torch.Tensor, near: float, interval: float, topk: i
       depth_scale [V,H,W]       compute_depth_scale[_MultiIntrin]          mvsdet.py:1158-1218
       est_ray_depth [V,T,H,W]   est_depth / (depth_scale + 1e-8)           mvsdet.py:494
       ray_depth_coding [V,H,W]  depth_coding / (depth_scale + 1e-8)        mvsdet.py:583
-    (full, un-cropped maps; the caller crops / reshapes as it does est_depth)."""
+    (full, un-cropped maps; the caller crops / reshapes as it does est_depth).
+    ``depth_values``, ``interval``: per-pixel hypotheses as in ``depth_topk``."""
     _check_cost("cost_out", cost_out)
     kmat = _ray_intr(k_feat, cost_out.shape[0])
+    if depth_values is not None:
+        return _depth_topk_px("cost_out", cost_out, depth_values, interval, topk, 0, kmat)
     return _DepthTopkNVS.apply(cost_out, near, interval, int(topk), kmat)
 
 
@@ -572,10 +647,14 @@ def rgb_downsample4(rgb: torch.Tensor, src_ids, height: int, width: int) -> torc
     return out
 
 
-def topk_hypotheses(prob_off: torch.Tensor, near: float, interval: float, topk: int):
+def topk_hypotheses(prob_off: torch.Tensor, near: float, interval, topk: int,
+                    depth_values: Optional[torch.Tensor] = None):
     """Stand-alone form of ``depth_topk`` for inputs that are already
     probabilities / offsets: prob_off [V,2,D,H,W] = stack(prob_volume, off_pred).
-    Same six outputs (the first two are pass-through copies)."""
+    Same six outputs (the first two are pass-through copies); ``depth_values`` and
+    ``interval`` as in ``depth_topk``."""
+    if depth_values is not None:
+        return _depth_topk_px("prob_off", prob_off, depth_values, interval, topk, 1)
     _check_cost("prob_off", prob_off)
     return _DepthTopk.apply(prob_off, near, interval, int(topk), 1)
 
