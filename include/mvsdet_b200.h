@@ -25,14 +25,16 @@
  * format.  Volumes with layout MVSD_CHANNELS_LAST are [V][D][H][W][C]
  * (torch.channels_last_3d of logical [V,C,D,H,W]).  C must be a multiple of 4
  * and at most 512.  Accumulation is always fp32 (64-bit fixed point in the
- * bit-reproducible *_det forms of the two scatter backwards).
+ * bit-reproducible *_det forms of the scatter backwards).
  *
  * Additive symbols (no ABI version change; every earlier signature is unchanged):
  *   mvsd_plane_sweep_fwd_px, mvsd_plane_sweep_bwd_px, mvsd_plane_sweep_bwd_det_px,
  *   mvsd_plane_sweep_groupcorr_fwd_px, mvsd_plane_sweep_groupcorr_bwd_px --
  *   the fused sweeps with per-pixel depth hypotheses;
  *   mvsd_depth_topk_fwd_px, mvsd_depth_topk_bwd_px -- the top-k epilogue over
- *   per-pixel depth hypotheses.
+ *   per-pixel depth hypotheses;
+ *   mvsd_plane_sweep_groupcorr_bwd_det, mvsd_plane_sweep_groupcorr_bwd_det_px --
+ *   the deterministic group-correlation backward.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -220,6 +222,23 @@ int mvsd_plane_sweep_groupcorr_bwd_px(const float* g_out, const void* feat, int 
                                       const float* depth_values, float* g_feat,
                                       int V, int C, int D, int H, int W, int k, int num_groups,
                                       int ref_begin, int n_feat_views, void* stream);
+/* Deterministic form of mvsd_plane_sweep_groupcorr_bwd / _bwd_px (bit-reproducible
+ * gradients), as mvsd_plane_sweep_bwd_det is for the variance: same arguments and
+ * checks, except that the contributions are added as signed 64-bit fixed point with
+ * 32 fractional bits (resolution 2.3e-10, |values| < 2^31; integer REDs are
+ * order-independent) into g_feat_q (nhwc int64, extent of feat, caller zero-fills);
+ * mvsd_fixed_to_float converts the sums back.  Always the un-merged pixel-per-warp
+ * scatter with scalar 64-bit REDs: opt-in reproducibility mode, not the fast path. */
+int mvsd_plane_sweep_groupcorr_bwd_det(const float* g_out, const void* feat, int feat_dtype,
+                                       const int32_t* nbr_ids, const float* hom,
+                                       const float* depth_values, int64_t* g_feat_q,
+                                       int V, int C, int D, int H, int W, int k, int num_groups,
+                                       int ref_begin, int n_feat_views, void* stream);
+int mvsd_plane_sweep_groupcorr_bwd_det_px(const float* g_out, const void* feat, int feat_dtype,
+                                          const int32_t* nbr_ids, const float* hom,
+                                          const float* depth_values, int64_t* g_feat_q,
+                                          int V, int C, int D, int H, int W, int k, int num_groups,
+                                          int ref_begin, int n_feat_views, void* stream);
 
 /* ---- a3 alone: homo_warping (mvs_models/module.py:105-146) --------------- *
  *   src  nhwc [B,H,W,C]; hom [B,12]; out [B,D,H,W,C];

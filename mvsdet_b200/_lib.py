@@ -45,6 +45,9 @@ SIGNATURES = {
     "mvsd_plane_sweep_groupcorr_bwd": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_groupcorr_fwd_px": ([_p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_plane_sweep_groupcorr_bwd_px": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_groupcorr_bwd_det": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_plane_sweep_groupcorr_bwd_det_px": ([_p, _p, _i, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p],
+                                              _i),
     "mvsd_homo_warp_fwd": ([_p, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_homo_warp_bwd": ([_p, _i, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_depth_topk_fwd": ([_p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p,
@@ -169,13 +172,22 @@ def plane_sweep_groupcorr_fwd(feat, nbr_ids, hom, depth_values, out, *, ref_begi
          vf, _stream())
 
 
-def plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, *, ref_begin=0):
-    """fp32 g laid out as the forward's out -> RED into the fp32 g_feat"""
+def _corr_bwd(name, g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin):
     vf, c, h, w = feat.shape
     v, k = nbr_ids.shape
-    call(_sweep_entry("mvsd_plane_sweep_groupcorr_bwd", depth_values), g.data_ptr(), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
+    call(_sweep_entry(name, depth_values), g.data_ptr(), feat.data_ptr(), _code(feat.dtype), nbr_ids.data_ptr(),
          hom.data_ptr(), depth_values.data_ptr(), g_feat.data_ptr(), v, c, depth_values.shape[1], h, w, k,
          g.shape[2], ref_begin, vf, _stream())
+
+
+def plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, *, ref_begin=0):
+    """fp32 g laid out as the forward's out -> RED into the fp32 g_feat"""
+    _corr_bwd("mvsd_plane_sweep_groupcorr_bwd", g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin)
+
+
+def plane_sweep_groupcorr_bwd_det(g, feat, nbr_ids, hom, depth_values, g_feat_q, *, ref_begin=0):
+    """``plane_sweep_groupcorr_bwd`` into an int64 fixed-point accumulator"""
+    _corr_bwd("mvsd_plane_sweep_groupcorr_bwd_det", g, feat, nbr_ids, hom, depth_values, g_feat_q, ref_begin)
 
 
 def homo_warp_fwd(src, hom, depth_values, out):

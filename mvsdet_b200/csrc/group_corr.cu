@@ -17,7 +17,8 @@
 // Backward: d ref += sum_j sum_d g_j / cg * warped_j ; d warped_j = g_j / cg * ref -> bilinear
 // scatter with fp32 vector REDs: for bf16 features and k = 2 through the run-merging hand-off kernel of
 // the variance backward (plane_sweep_bwd_run.cu, MODE 1: same gather, column merging and row hand-off,
-// the correlation algebra in the pixel body), otherwise the un-merged pixel-per-warp kernel below.
+// the correlation algebra in the pixel body), otherwise the un-merged pixel-per-warp kernel below.  The
+// deterministic form (*_bwd_det) is always that pixel kernel, with 64-bit fixed-point integer REDs.
 #include "plane_sweep.cuh"
 
 namespace mvsd {
@@ -163,17 +164,17 @@ __global__ void __launch_bounds__(kCorrThreads, 8) corr_fwd_kernel(const CorrPar
   }
 }
 
-template <int G, bool FULL>
-__device__ __forceinline__ void corr_red_tap(float* dst, unsigned off, const float4 (&gw)[G], float w,
-                                             int c0, int C) {
-  if (w == 0.f) return;                         // clamped (outside) tap: contributes nothing
-  float* a = at(dst, off);
-#pragma unroll
-  for (int g = 0; g < G; ++g)
-    if (group_on<FULL>(c0, g, C)) red_add_f32x4(a + 128 * g, f4scale(gw[g], w));
+// The gradient accumulator of the TAcc form, read where it is used: a pointer hoisted to the top of
+// corr_bwd_kernel changed the register allocation of the fp32-RED kernels.
+template <typename TAcc>
+__device__ __forceinline__ TAcc* acc_ptr(const SweepParams& p) {
+  if constexpr (sizeof(TAcc) == 8) return p.g_feat_q;
+  else return p.g_feat;
 }
 
-template <typename TIn, int G, bool FULL, bool PX = false>
+// TAcc = float: fp32 vector REDs into p.g_feat; TAcc = long long: the deterministic form, fixed-point
+// integer REDs into p.g_feat_q (common.cuh)
+template <typename TIn, int G, bool FULL, typename TAcc = float, bool PX = false>
 __global__ void __launch_bounds__(kSweepThreads) corr_bwd_kernel(const CorrParams q) {
   const SweepParams& p = q.s;
   __shared__ WarpSample s_tab[kSweepWarps][kSlots];
@@ -212,18 +213,18 @@ __global__ void __launch_bounds__(kSweepThreads) corr_bwd_kernel(const CorrParam
           gref[g] = f4fma(wv[g], gq, gref[g]);
           gw[g] = f4scale(ref[g], gq);
         }
-        float* dst = p.g_feat + (size_t)n * HW * C + c.c0;
-        corr_red_tap<G, FULL>(dst, s.p00, gw, s.w00, c.c0, C);
-        corr_red_tap<G, FULL>(dst, s.p01, gw, s.w01, c.c0, C);
-        corr_red_tap<G, FULL>(dst, s.p10, gw, s.w10, c.c0, C);
-        corr_red_tap<G, FULL>(dst, s.p11, gw, s.w11, c.c0, C);
+        TAcc* dst = acc_ptr<TAcc>(p) + (size_t)n * HW * C + c.c0;
+        red_tap<G, FULL, TAcc>(dst, s.p00, gw, s.w00, c.c0, C);
+        red_tap<G, FULL, TAcc>(dst, s.p01, gw, s.w01, c.c0, C);
+        red_tap<G, FULL, TAcc>(dst, s.p10, gw, s.w10, c.c0, C);
+        red_tap<G, FULL, TAcc>(dst, s.p11, gw, s.w11, c.c0, C);
       }
     }
   }
-  float* dst = p.g_feat + ref_off;
+  TAcc* dst = acc_ptr<TAcc>(p) + ref_off;
 #pragma unroll
   for (int g = 0; g < G; ++g)
-    if (group_on<FULL>(c.c0, g, C)) red_add_f32x4(dst + 128 * g, gref[g]);
+    if (group_on<FULL>(c.c0, g, C)) red_vec(dst + 128 * g, gref[g]);
 }
 
 static int corr_setup(const char* who, CorrParams& q, int num_groups) {
@@ -245,23 +246,28 @@ static int corr_setup(const char* who, CorrParams& q, int num_groups) {
   return MVSD_OK;
 }
 
-template <bool BWD, typename TIn>
+// TAcc = long long: the deterministic backward, built with FULL = false only (ragged C by predication), as
+// the variance's deterministic kernel is
+template <bool BWD, typename TIn, typename TAcc>
 static int corr_launch_t(CorrParams& q, cudaStream_t st) {
-  // the forward has its own CTA patch
-  return sweep_launch(q.s, "plane_sweep_groupcorr", BWD ? kPatchW : kCorrPatchW, BWD ? kPatchH : kCorrPatchH,
-                      BWD ? "plane_sweep_groupcorr_bwd" : "plane_sweep_groupcorr_fwd",
-                      [&](dim3 grid, auto G2, auto FULL, auto PX) {
+  constexpr bool det = std::is_same_v<TAcc, long long>;
+  const char* name = det ? "plane_sweep_groupcorr_bwd_det"
+                         : BWD ? "plane_sweep_groupcorr_bwd" : "plane_sweep_groupcorr_fwd";
+  // the forward has its own CTA patch; grid errors name the family, or the deterministic kernel
+  return sweep_launch(q.s, det ? name : "plane_sweep_groupcorr", BWD ? kPatchW : kCorrPatchW,
+                      BWD ? kPatchH : kCorrPatchH, name, [&](dim3 grid, auto G2, auto FULL, auto PX) {
     constexpr int GG = G2 ? 2 : 1;
-    if constexpr (BWD) corr_bwd_kernel<TIn, GG, FULL, PX><<<grid, kSweepThreads, 0, st>>>(q);
+    if constexpr (det) corr_bwd_kernel<TIn, GG, false, TAcc, PX><<<grid, kSweepThreads, 0, st>>>(q);
+    else if constexpr (BWD) corr_bwd_kernel<TIn, GG, FULL, TAcc, PX><<<grid, kSweepThreads, 0, st>>>(q);
     else if (q.s.k == 2) corr_fwd_kernel<TIn, 2, GG, FULL, PX><<<grid, kCorrThreads, 0, st>>>(q);
     else corr_fwd_kernel<TIn, 4, GG, FULL, PX><<<grid, kCorrThreads, 0, st>>>(q);
   });
 }
 
-template <bool BWD>
+template <bool BWD, typename TAcc = float>
 static int corr_launch(CorrParams& q, const char* who, int feat_dtype, cudaStream_t st) {
-  if (feat_dtype == MVSD_F32) return corr_launch_t<BWD, float>(q, st);
-  if (feat_dtype == MVSD_BF16) return corr_launch_t<BWD, __nv_bfloat16>(q, st);
+  if (feat_dtype == MVSD_F32) return corr_launch_t<BWD, float, TAcc>(q, st);
+  if (feat_dtype == MVSD_BF16) return corr_launch_t<BWD, __nv_bfloat16, TAcc>(q, st);
   return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
 }
 
@@ -279,23 +285,27 @@ static int groupcorr_fwd(const char* who, const void* feat, int feat_dtype, cons
   return corr_launch<false>(q, who, feat_dtype, static_cast<cudaStream_t>(stream));
 }
 
+// g_acc: dL/dfeat, fp32 (TAcc = float) or the deterministic form's 64-bit fixed point (TAcc = long long)
+template <typename TAcc>
 static int groupcorr_bwd(const char* who, const float* g_out, const void* feat, int feat_dtype,
-                         const int32_t* nbr_ids, const float* hom, const float* depth_values, float* g_feat,
+                         const int32_t* nbr_ids, const float* hom, const float* depth_values, TAcc* g_acc,
                          int V, int C, int D, int H, int W, int k, int num_groups, int ref_begin,
                          int n_feat_views, bool per_pixel, void* stream) {
+  constexpr bool det = std::is_same_v<TAcc, long long>;
   CorrParams q{};
-  if (int e = sweep_setup(q.s, who, {g_out, feat, g_feat}, true, feat, nbr_ids, hom, depth_values, V, C, D, H, W,
+  if (int e = sweep_setup(q.s, who, {g_out, feat, g_acc}, true, feat, nbr_ids, hom, depth_values, V, C, D, H, W,
                           k, MVSD_CHANNELS_LAST, ref_begin, n_feat_views, per_pixel))
     return e;
   q.s.g_out = g_out;
-  q.s.g_feat = g_feat;
+  if constexpr (det) q.s.g_feat_q = g_acc;
+  else q.s.g_feat = g_acc;
   if (int e = corr_setup(who, q, num_groups)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // bf16 features, k = 2: the run-merging hand-off kernel of the variance backward with the correlation
-  // algebra in its pixel body (same gather, same merged scatter); anything else (and the test hook
-  // mvsd_set_tuning(5, 1)): the pixel-per-warp kernel above
-  if (feat_dtype == MVSD_BF16 && k == 2 && tuning(5) != 1) return launch_bwd_run_corr(q.s, st);
-  return corr_launch<true>(q, who, feat_dtype, st);
+  // algebra in its pixel body (same gather, same merged scatter); anything else, the deterministic form
+  // and the test hook mvsd_set_tuning(5, 1): the pixel-per-warp kernel above
+  if (!det && feat_dtype == MVSD_BF16 && k == 2 && tuning(5) != 1) return launch_bwd_run_corr(q.s, st);
+  return corr_launch<true, TAcc>(q, who, feat_dtype, st);
 }
 
 }  // namespace mvsd
@@ -334,4 +344,24 @@ extern "C" int mvsd_plane_sweep_groupcorr_bwd_px(const float* g_out, const void*
                                                  int n_feat_views, void* stream) {
   return groupcorr_bwd("plane_sweep_groupcorr_bwd_px", g_out, feat, feat_dtype, nbr_ids, hom, depth_values,
                        g_feat, V, C, D, H, W, k, num_groups, ref_begin, n_feat_views, true, stream);
+}
+
+extern "C" int mvsd_plane_sweep_groupcorr_bwd_det(const float* g_out, const void* feat, int feat_dtype,
+                                                  const int32_t* nbr_ids, const float* hom,
+                                                  const float* depth_values, int64_t* g_feat_q, int V, int C,
+                                                  int D, int H, int W, int k, int num_groups, int ref_begin,
+                                                  int n_feat_views, void* stream) {
+  return groupcorr_bwd("plane_sweep_groupcorr_bwd_det", g_out, feat, feat_dtype, nbr_ids, hom, depth_values,
+                       reinterpret_cast<long long*>(g_feat_q), V, C, D, H, W, k, num_groups, ref_begin,
+                       n_feat_views, false, stream);
+}
+
+extern "C" int mvsd_plane_sweep_groupcorr_bwd_det_px(const float* g_out, const void* feat, int feat_dtype,
+                                                     const int32_t* nbr_ids, const float* hom,
+                                                     const float* depth_values, int64_t* g_feat_q, int V,
+                                                     int C, int D, int H, int W, int k, int num_groups,
+                                                     int ref_begin, int n_feat_views, void* stream) {
+  return groupcorr_bwd("plane_sweep_groupcorr_bwd_det_px", g_out, feat, feat_dtype, nbr_ids, hom, depth_values,
+                       reinterpret_cast<long long*>(g_feat_q), V, C, D, H, W, k, num_groups, ref_begin,
+                       n_feat_views, true, stream);
 }

@@ -314,6 +314,21 @@ __device__ __forceinline__ bool group_on(int c0, int g, int C) {
   return FULL || (c0 + 128 * g < C);
 }
 
+// The scatter of the pixel-per-warp backwards (variance: plane_sweep_bwd.cu, correlation: group_corr.cu).
+// TAcc = float: fp32 vector REDs; TAcc = long long: the deterministic fixed-point form (common.cuh)
+__device__ __forceinline__ void red_vec(float* a, float4 v) { red_add_f32x4(a, v); }
+__device__ __forceinline__ void red_vec(long long* a, float4 v) { red_add_fixed4(a, v); }
+
+template <int G, bool FULL, typename TAcc>
+__device__ __forceinline__ void red_tap(TAcc* dst, unsigned off, const float4 (&gw)[G], float w,
+                                        int c0, int C) {
+  if (w == 0.f) return;                         // clamped (outside) tap: contributes nothing
+  TAcc* a = at(dst, off);
+#pragma unroll
+  for (int g = 0; g < G; ++g)
+    if (group_on<FULL>(c0, g, C)) red_vec(a + 128 * g, f4scale(gw[g], w));
+}
+
 // The bilinear sample of one neighbour: nw*w00 + ne*w01 + sw*w10 + se*w11, the
 // order ATen's sampler uses.  All 4*G loads are issued before the first FMA.
 template <typename TIn, int G, bool FULL>

@@ -9,20 +9,6 @@
 
 namespace mvsd {
 
-// TAcc = float: fp32 vector REDs; TAcc = long long: the deterministic fixed-point form (common.cuh)
-__device__ __forceinline__ void red_vec(float* a, float4 v) { red_add_f32x4(a, v); }
-__device__ __forceinline__ void red_vec(long long* a, float4 v) { red_add_fixed4(a, v); }
-
-template <int G, bool FULL, typename TAcc>
-__device__ __forceinline__ void red_tap(TAcc* dst, unsigned off, const float4 (&gw)[G], float w,
-                                        int c0, int C) {
-  if (w == 0.f) return;                         // clamped (outside) tap: contributes nothing
-  TAcc* a = at(dst, off);
-#pragma unroll
-  for (int g = 0; g < G; ++g)
-    if (group_on<FULL>(c0, g, C)) red_vec(a + 128 * g, f4scale(gw[g], w));
-}
-
 // PX: per-pixel depth hypotheses [V,D,H,W] (the *_px entry points)
 template <typename TIn, typename TG, int KMAX, int G, bool FULL, bool WARP_ONLY, typename TAcc = float,
           bool PX = false>

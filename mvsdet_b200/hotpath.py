@@ -59,10 +59,11 @@ class MVSDetHotPath(nn.Module):
         # True: hand the cost-regularisation net the variance in the reference's strict NCDHW
         # contiguous memory (one extra transpose pass) instead of channels_last_3d
         self.strict_ncdhw_variance = bool(strict_ncdhw_variance)
-        # True: bit-reproducible feature / cost gradients -- the backward kernels accumulate in 64-bit
-        # fixed point with integer REDs (order-independent) instead of fp32 REDs.  A scene's forward +
-        # backward takes 7.3 ms instead of 1.2 ms (un-merged scatter, scalar 64-bit REDs): a
-        # reproducibility mode, not the fast path; the forward is deterministic either way.
+        # True: bit-reproducible feature / cost gradients -- the backward kernels (variance or group-
+        # correlation sweep, back-projection) accumulate in 64-bit fixed point with integer REDs
+        # (order-independent) instead of fp32 REDs.  A scene's forward + backward with the variance
+        # takes 7.3 ms instead of 1.2 ms (un-merged scatter, scalar 64-bit REDs): a reproducibility
+        # mode, not the fast path; the forward is deterministic either way.
         self.deterministic = bool(deterministic)
         # "variance" (the reference, mvsdet.py:439-467) or "group_correlation": hand the cost-regularisation
         # net the k group-wise correlation volumes [V,k,num_groups,D,H,W] instead (SURVEY 8f rank 4; the
@@ -71,8 +72,6 @@ class MVSDetHotPath(nn.Module):
             raise ValueError("cost_volume must be 'variance' or 'group_correlation'")
         self.cost_volume = cost_volume
         self.num_groups = int(num_groups)
-        if cost_volume == "group_correlation" and deterministic:
-            raise ValueError("the group-correlation backward has no deterministic form")
         if self.deterministic and self.dispatcher_ops:
             raise ValueError("deterministic=True uses the shared gradient accumulator of the autograd.Function "
                              "layer; it is not available with dispatcher_ops=True")

@@ -322,12 +322,13 @@ def _corr_fwd_raw(feat, nbr_ids, hom, depth_values, num_groups, ref_begin):
 
 
 def _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, ref_begin, acc=None):
-    """-> dL/dfeat in feat's dtype (channels_last), or None when it was accumulated into the fp32
-    accumulator ``acc`` (FeatureGradSink)"""
+    """-> dL/dfeat in feat's dtype (channels_last), or None when it was accumulated into the
+    accumulator ``acc`` (FeatureGradSink: fp32, or int64 fixed point for the deterministic form)"""
     # no copy when it arrives in the forward's layout
     g = g.float().permute(0, 1, 3, 4, 5, 2).contiguous().permute(0, 1, 5, 2, 3, 4)
-    if acc is not None and acc.dtype != torch.float32:
-        raise ValueError("the group-correlation backward has no deterministic form")
+    if acc is not None and acc.dtype == torch.int64:        # deterministic sink: fixed-point integer REDs
+        _lib.plane_sweep_groupcorr_bwd_det(g, feat, nbr_ids, hom, depth_values, acc, ref_begin=ref_begin)
+        return None
     g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
     _lib.plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin=ref_begin)
     return None if acc is not None else g_feat.to(feat.dtype)
