@@ -34,7 +34,9 @@
  *   mvsd_depth_topk_fwd_px, mvsd_depth_topk_bwd_px -- the top-k epilogue over
  *   per-pixel depth hypotheses;
  *   mvsd_plane_sweep_groupcorr_bwd_det, mvsd_plane_sweep_groupcorr_bwd_det_px --
- *   the deterministic group-correlation backward.
+ *   the deterministic group-correlation backward;
+ *   mvsd_homo_warp_bwd_det, mvsd_backproject_bwd_det_mode -- the deterministic
+ *   backwards of the stand-alone warp and of the SUM / PER_VIEW back-projection.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -252,6 +254,16 @@ int mvsd_homo_warp_bwd(const void* g_out, int g_dtype, int g_layout,
                        const float* hom, const float* depth_values,
                        float* g_src, int B, int C, int D, int H, int W,
                        int depth_per_pixel, void* stream);
+/* Deterministic form of mvsd_homo_warp_bwd (bit-reproducible gradients): same arguments
+ * and checks (messages name mvsd_homo_warp_bwd_det), both depth forms, fp32 or bf16
+ * g_out, except that the contributions are added as signed 64-bit fixed point with 32
+ * fractional bits (resolution 2.3e-10, |values| < 2^31; integer REDs are
+ * order-independent) into g_src_q (nhwc int64, extent of src, caller zero-fills);
+ * mvsd_fixed_to_float converts the sums back. */
+int mvsd_homo_warp_bwd_det(const void* g_out, int g_dtype, int g_layout,
+                           const float* hom, const float* depth_values,
+                           int64_t* g_src_q, int B, int C, int D, int H, int W,
+                           int depth_per_pixel, void* stream);
 
 /* ---- a5-a7: softmax / sigmoid / top-k / depth expectation ---------------- *
  * Replaces mvsdet.py:470-482, sample_depth_prob (:266-283) and
@@ -396,6 +408,22 @@ int mvsd_backproject_bwd_det(const float* g_out, int g_layout, const int32_t* co
                              int64_t dp_sv, int64_t dp_sy, int64_t dp_sx, int64_t dp_st,
                              float vs_z, int64_t* g_feat_q, int64_t* g_pn_q,
                              int V, int C, int h, int w, int T, int N, void* stream);
+/* Deterministic form of mvsd_backproject_bwd for MVSD_BP_SUM (either layout) and
+ * MVSD_BP_PER_VIEW (channels-last): same arguments and checks (messages name
+ * mvsd_backproject_bwd_det_mode; count is unused), except that g_feat_q (nhwc int64,
+ * extent of feat) and g_pn_q (int64, prob's strides, may be NULL) take the
+ * contributions as signed 64-bit fixed point with 32 fractional bits (resolution
+ * 2.3e-10, |values| < 2^31; integer REDs are order-independent); the caller
+ * zero-fills both and converts them with mvsd_fixed_to_float.  MVSD_BP_MEAN is
+ * MVSD_ERR_UNSUPPORTED here: its deterministic form is mvsd_backproject_bwd_det. */
+int mvsd_backproject_bwd_det_mode(const float* g_out, int g_layout, int mode,
+                                  const int32_t* count,
+                                  const void* feat, int feat_dtype, int feat_h, int feat_w,
+                                  const float* points, const float* projection,
+                                  const float* depth, const float* prob,
+                                  int64_t dp_sv, int64_t dp_sy, int64_t dp_sx, int64_t dp_st,
+                                  float vs_z, int64_t* g_feat_q, int64_t* g_pn_q,
+                                  int V, int C, int h, int w, int T, int N, void* stream);
 int mvsd_prob_norm_bwd(const float* prob, const float* g_pn, float* g_prob,
                        int64_t dp_sv, int64_t dp_sy, int64_t dp_sx, int64_t dp_st,
                        int V, int h, int w, int T, void* stream);

@@ -50,6 +50,7 @@ SIGNATURES = {
                                               _i),
     "mvsd_homo_warp_fwd": ([_p, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_homo_warp_bwd": ([_p, _i, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_homo_warp_bwd_det": ([_p, _i, _i, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_depth_topk_fwd": ([_p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p,
                              _f, _f, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_depth_topk_bwd": ([_p, _l, _l, _l, _l, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p,
@@ -64,6 +65,8 @@ SIGNATURES = {
                               _p, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_backproject_bwd": ([_p, _i, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _l, _l, _l, _l,
                               _f, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
+    "mvsd_backproject_bwd_det_mode": ([_p, _i, _i, _p, _p, _i, _i, _i, _p, _p, _p, _p, _l, _l, _l, _l,
+                                       _f, _p, _p, _i, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_prob_norm_bwd": ([_p, _p, _p, _l, _l, _l, _l, _i, _i, _i, _i, _p], _i),
     "mvsd_voxel_normalize": ([_p, _p, _p, _i, _i, _i, _p], _i),
     "mvsd_voxel_reduce_p2p": ([_p, _p, _p, _i, _i, _i, _i, _i, _p], _i),
@@ -198,10 +201,19 @@ def homo_warp_fwd(src, hom, depth_values, out):
          int(depth_values.dim() == 4), _stream())
 
 
-def homo_warp_bwd(g, hom, depth_values, g_src):
+def _homo_warp_bwd(name, g, hom, depth_values, g_src):
     b, c, h, w = g_src.shape
-    call("mvsd_homo_warp_bwd", g.data_ptr(), _code(g.dtype), CHANNELS_LAST, hom.data_ptr(), depth_values.data_ptr(),
+    call(name, g.data_ptr(), _code(g.dtype), CHANNELS_LAST, hom.data_ptr(), depth_values.data_ptr(),
          g_src.data_ptr(), b, c, depth_values.shape[1], h, w, int(depth_values.dim() == 4), _stream())
+
+
+def homo_warp_bwd(g, hom, depth_values, g_src):
+    _homo_warp_bwd("mvsd_homo_warp_bwd", g, hom, depth_values, g_src)
+
+
+def homo_warp_bwd_det(g, hom, depth_values, g_src_q):
+    """``homo_warp_bwd`` into an int64 fixed-point accumulator"""
+    _homo_warp_bwd("mvsd_homo_warp_bwd_det", g, hom, depth_values, g_src_q)
 
 
 def _interval(interval):
@@ -269,16 +281,29 @@ def backproject_fwd(feat, points, projection, depth, prob, out, *, vs_z, mode, h
          _layout(channels_first), _ptr(count), _ptr(valid), None, v, c, height, width, t, out.shape[-1], _stream())
 
 
-def backproject_bwd(g_out, feat, points, projection, depth, prob, g_feat, g_pn, *, vs_z, mode, height, width,
-                    channels_first=False, count=None):
-    """g_out shaped as ``backproject_fwd``'s out -> RED into g_feat and g_pn (prob's strides)"""
+def _backproject_bwd(name, g_out, feat, points, projection, depth, prob, g_feat, g_pn, vs_z, mode, height, width,
+                     channels_first, count):
     _, c, fh, fw = feat.shape
     v, t = depth.shape[:2]
     sv, st, sy, sx = depth.stride()
-    call("mvsd_backproject_bwd", g_out.data_ptr(), _layout(channels_first), mode, _ptr(count), feat.data_ptr(),
+    call(name, g_out.data_ptr(), _layout(channels_first), mode, _ptr(count), feat.data_ptr(),
          _code(feat.dtype), fh, fw, points.data_ptr(), projection.data_ptr(), depth.data_ptr(), prob.data_ptr(),
          sv, sy, sx, st, float(vs_z), g_feat.data_ptr(), g_pn.data_ptr(), v, c, height, width, t,
          g_out.shape[-1], _stream())
+
+
+def backproject_bwd(g_out, feat, points, projection, depth, prob, g_feat, g_pn, *, vs_z, mode, height, width,
+                    channels_first=False, count=None):
+    """g_out shaped as ``backproject_fwd``'s out -> RED into g_feat and g_pn (prob's strides)"""
+    _backproject_bwd("mvsd_backproject_bwd", g_out, feat, points, projection, depth, prob, g_feat, g_pn, vs_z,
+                     mode, height, width, channels_first, count)
+
+
+def backproject_bwd_det_mode(g_out, feat, points, projection, depth, prob, g_feat_q, g_pn_q, *, vs_z, mode,
+                             height, width, channels_first=False):
+    """``backproject_bwd`` (SUM or PER_VIEW) into int64 fixed-point accumulators"""
+    _backproject_bwd("mvsd_backproject_bwd_det_mode", g_out, feat, points, projection, depth, prob, g_feat_q,
+                     g_pn_q, vs_z, mode, height, width, channels_first, None)
 
 
 def backproject_bwd_det(g_out, count, feat, points, projection, depth, prob, g_feat_q, g_pn_q, *, vs_z, height,

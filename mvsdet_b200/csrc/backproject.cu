@@ -500,6 +500,54 @@ extern "C" int mvsd_backproject_bwd_det(const float* g_out, int g_layout, const 
   return fail(MVSD_ERR_INVALID_ARG, "backproject_bwd_det: bad dtype");
 }
 
+// Deterministic form of the SUM and PER_VIEW backwards (the MEAN mode stays with mvsd_backproject_bwd_det):
+// SUM in both volume layouts, PER_VIEW channels-last only, as in the fp32 form.
+template <typename TIn, int G>
+static int launch_bp_bwd_det_mode(const BpParams& p, int mode, bool cfirst, cudaStream_t st) {
+  dim3 grid((p.N + kBpVox - 1) / kBpVox);
+  if (mode == MVSD_BP_PER_VIEW)
+    backproject_bwd_kernel<TIn, G, MVSD_BP_PER_VIEW, false, 16, true><<<grid, 16 * 32, 0, st>>>(p);
+  else if (cfirst) backproject_bwd_kernel<TIn, G, MVSD_BP_SUM, true, 16, true><<<grid, 16 * 32, 0, st>>>(p);
+  else backproject_bwd_kernel<TIn, G, MVSD_BP_SUM, false, 16, true><<<grid, 16 * 32, 0, st>>>(p);
+  count_launch();
+  return check_launch("backproject_bwd_det_mode");
+}
+
+extern "C" int mvsd_backproject_bwd_det_mode(const float* g_out, int g_layout, int mode,
+                                             const int32_t* count, const void* feat, int feat_dtype,
+                                             int feat_h, int feat_w, const float* points,
+                                             const float* projection, const float* depth, const float* prob,
+                                             int64_t dp_sv, int64_t dp_sy, int64_t dp_sx, int64_t dp_st,
+                                             float vs_z, int64_t* g_feat_q, int64_t* g_pn_q, int V, int C,
+                                             int h, int w, int T, int N, void* stream) {
+  const char* who = "backproject_bwd_det_mode";
+  if (int e = check_bp(who, V, C, h, w, T, N, feat_h, feat_w, mode, g_layout)) return e;
+  if (!g_out || !feat || !points || !projection || !depth || !prob || !g_feat_q)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (mode == MVSD_BP_MEAN)
+    return fail(MVSD_ERR_UNSUPPORTED, "%s: the MEAN mode's deterministic backward is mvsd_backproject_bwd_det", who);
+  BpParams p{};
+  p.feat = feat; p.points = points; p.proj = projection; p.depth = depth; p.prob = prob;
+  p.sv = dp_sv; p.sy = dp_sy; p.sx = dp_sx; p.st = dp_st; p.vs_z = vs_z;
+  p.g_out = g_out; p.count_in = count;
+  p.g_feat_q = reinterpret_cast<long long*>(g_feat_q); p.g_pn_q = reinterpret_cast<long long*>(g_pn_q);
+  p.V = V; p.C = C; p.h = h; p.w = w; p.T = T; p.N = N; p.feat_h = feat_h; p.feat_w = feat_w;
+  const bool cfirst = g_layout == MVSD_CHANNELS_FIRST;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int G = (C + 127) / 128;
+  if (feat_dtype == MVSD_F32) {
+    if (G == 1) return launch_bp_bwd_det_mode<float, 1>(p, mode, cfirst, st);
+    if (G == 2) return launch_bp_bwd_det_mode<float, 2>(p, mode, cfirst, st);
+    return launch_bp_bwd_det_mode<float, 4>(p, mode, cfirst, st);
+  }
+  if (feat_dtype == MVSD_BF16) {
+    if (G == 1) return launch_bp_bwd_det_mode<__nv_bfloat16, 1>(p, mode, cfirst, st);
+    if (G == 2) return launch_bp_bwd_det_mode<__nv_bfloat16, 2>(p, mode, cfirst, st);
+    return launch_bp_bwd_det_mode<__nv_bfloat16, 4>(p, mode, cfirst, st);
+  }
+  return fail(MVSD_ERR_INVALID_ARG, "%s: bad dtype", who);
+}
+
 extern "C" int mvsd_prob_norm_bwd(const float* prob, const float* g_pn, float* g_prob,
                                   int64_t dp_sv, int64_t dp_sy, int64_t dp_sx, int64_t dp_st,
                                   int V, int h, int w, int T, void* stream) {

@@ -106,15 +106,16 @@ __global__ void __launch_bounds__(kSweepThreads) sweep_bwd_kernel(const SweepPar
 }
 
 // The pixel-per-warp kernel: the variance backward for k = 0, 3, 4 (and every k through the test hook),
-// its deterministic form (TAcc = long long) and the stand-alone warp.  One instantiation per dtype and
-// channel-group count: every k <= 4 and ragged C handled by predication.
+// its deterministic form (TAcc = long long) and the stand-alone warp (either accumulator).  One
+// instantiation per dtype and channel-group count: every k <= 4 and ragged C handled by predication.
 template <typename TIn, typename TG, bool WARP_ONLY, typename TAcc>
 static int launch_bwd_k(SweepParams& p, cudaStream_t st) {
-  const char* name = sizeof(TAcc) == 8 ? "plane_sweep_bwd_det" : "plane_sweep_bwd";
+  const char* name = sizeof(TAcc) == 8 ? (WARP_ONLY ? "homo_warp_bwd_det" : "plane_sweep_bwd_det")
+                                       : "plane_sweep_bwd";
   return sweep_launch(p, name, kPatchW, kPatchH, name, [&](dim3 grid, auto G2, auto /*FULL*/, auto PX) {
     constexpr int GG = G2 ? 2 : 1;
     if constexpr (WARP_ONLY)              // reads either depth form (fill_samples<kDepthEither>)
-      sweep_bwd_kernel<TIn, TG, 1, GG, false, true><<<grid, kSweepThreads, 0, st>>>(p);
+      sweep_bwd_kernel<TIn, TG, 1, GG, false, true, TAcc><<<grid, kSweepThreads, 0, st>>>(p);
     else
       sweep_bwd_kernel<TIn, TG, 4, GG, false, false, TAcc, PX><<<grid, kSweepThreads, 0, st>>>(p);
   });
@@ -221,4 +222,21 @@ extern "C" int mvsd_homo_warp_bwd(const void* g_out, int g_dtype, int g_layout, 
   if (g_dtype == MVSD_F32) return launch_bwd_k<float, float, true, float>(p, st);
   if (g_dtype == MVSD_BF16) return launch_bwd_k<float, __nv_bfloat16, true, float>(p, st);
   return fail(MVSD_ERR_INVALID_ARG, "homo_warp_bwd: bad dtype");
+}
+
+// Deterministic form of mvsd_homo_warp_bwd: the same scatter into a 64-bit fixed-point accumulator
+// (common.cuh), whose integer REDs do not depend on the order the warps arrive in.
+extern "C" int mvsd_homo_warp_bwd_det(const void* g_out, int g_dtype, int g_layout, const float* hom,
+                                      const float* depth_values, int64_t* g_src_q, int B, int C, int D,
+                                      int H, int W, int depth_per_pixel, void* stream) {
+  SweepParams p;
+  if (int e = sweep_setup(p, "homo_warp_bwd_det", {g_out, hom, g_src_q}, false, nullptr, nullptr, hom,
+                          depth_values, B, C, D, H, W, 1, g_layout, 0, B, depth_per_pixel != 0))
+    return e;
+  p.g_out = g_out;
+  p.g_feat_q = reinterpret_cast<long long*>(g_src_q);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (g_dtype == MVSD_F32) return launch_bwd_k<float, float, true, long long>(p, st);
+  if (g_dtype == MVSD_BF16) return launch_bwd_k<float, __nv_bfloat16, true, long long>(p, st);
+  return fail(MVSD_ERR_INVALID_ARG, "homo_warp_bwd_det: bad dtype");
 }

@@ -63,7 +63,9 @@ class MVSDetHotPath(nn.Module):
         # correlation sweep, back-projection) accumulate in 64-bit fixed point with integer REDs
         # (order-independent) instead of fp32 REDs.  A scene's forward + backward with the variance
         # takes 7.3 ms instead of 1.2 ms (un-merged scatter, scalar 64-bit REDs): a reproducibility
-        # mode, not the fast path; the forward is deterministic either way.
+        # mode, not the fast path; the forward is deterministic either way.  The backwards use the same kernels
+        # whenever torch.use_deterministic_algorithms(True) is in force (ops._deterministic), also with
+        # already-packed features and dispatcher_ops=True.
         self.deterministic = bool(deterministic)
         # "variance" (the reference, mvsdet.py:439-467) or "group_correlation": hand the cost-regularisation
         # net the k group-wise correlation volumes [V,k,num_groups,D,H,W] instead (SURVEY 8f rank 4; the
@@ -74,7 +76,8 @@ class MVSDetHotPath(nn.Module):
         self.num_groups = int(num_groups)
         if self.deterministic and self.dispatcher_ops:
             raise ValueError("deterministic=True uses the shared gradient accumulator of the autograd.Function "
-                             "layer; it is not available with dispatcher_ops=True")
+                             "layer; it is not available with dispatcher_ops=True.  "
+                             "torch.use_deterministic_algorithms(True) makes the dispatcher route deterministic")
 
     def geometry(self, img_meta: dict, device, view_slice=None, prologue=None) -> SceneGeometry:
         """Per-scene parameter block (mvsdet.py:407-450).  ``prologue``: "device" (default: two
@@ -158,7 +161,8 @@ class MVSDetHotPath(nn.Module):
             raise ValueError("a cost_regularization callable is required (mvsdet.py:470)")
         geo = geometry or self.geometry(img_meta, feature.device)
         # one fp32 gradient accumulator shared by the two consumers of the packed features
-        # (ops.FeatureGradSink); the torch.library route keeps plain functional autograd
+        # (ops.FeatureGradSink; int64 fixed point when deterministic or under the flag); the torch.library
+        # route keeps plain functional autograd
         feat_cl, sink = ops.pack_features(feature, self.feature_dtype, sink=True, deterministic=self.deterministic)
         if self.dispatcher_ops:
             sink = None

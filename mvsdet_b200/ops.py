@@ -15,6 +15,7 @@ kernels (and cuDNN's Conv3d after them) want.
 from __future__ import annotations
 
 import numbers
+import warnings
 from typing import Optional, Tuple
 
 import torch
@@ -35,6 +36,29 @@ def _need_cuda(name: str, t: torch.Tensor) -> None:
         raise ValueError(f"{name} must be a tensor")
     if not t.is_cuda:
         raise ValueError(f"{name} must be a CUDA tensor: mvsdet_b200 has no CPU path")
+
+
+def _deterministic(explicit: bool = False) -> bool:
+    """The one policy of the scatter backwards: the fixed-point (``*_det``) kernels when the caller asks
+    for them or ``torch.use_deterministic_algorithms(True)`` is in force.  Read when a backward runs, as
+    ATen reads the flag; the forwards are deterministic either way and never look at it."""
+    return bool(explicit) or torch.are_deterministic_algorithms_enabled()
+
+
+def _alert_not_deterministic(name: str) -> None:
+    """For a route with no deterministic backward under ``torch.use_deterministic_algorithms(True)``:
+    raise RuntimeError, or warn with ``warn_only=True`` -- what ATen does for such an op.  Host-side, so
+    call it before enqueueing anything."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{name} does not have a deterministic implementation, but you set "
+           "'torch.use_deterministic_algorithms(True)'. You can turn off determinism just for this operation, "
+           "or you can use the 'warn_only=True' option, if that's acceptable for your application. "
+           "MVSDetHotPath runs the same kernels with deterministic backwards.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg)
+    else:
+        raise RuntimeError(msg)
 
 
 def _is_nhwc(t: torch.Tensor) -> bool:
@@ -99,17 +123,19 @@ class FeatureGradSink:
         """the accumulator (logical [V,C,H,W], channels-last memory), zero-filled on first use.
         (Pre-filling it at forward time on a side stream was measured: the cross-stream
         ``record_stream`` defeats the caching allocator's block reuse, 820 -> 692 scenes/s.)
-        ``deterministic``: int64 fixed point (32 fractional bits) for the ``*_det`` kernels, whose
-        integer REDs make the sum independent of the order the warps arrive in."""
+        Deterministic (``_deterministic(self.deterministic)``, decided here, i.e. in the first
+        backward): int64 fixed point (32 fractional bits) for the ``*_det`` kernels, whose integer
+        REDs make the sum independent of the order the warps arrive in."""
         if self.buf is None:
             v, c, h, w = self.shape
-            self.buf = _zeros_nhwc(v, c, h, w, torch.int64 if self.deterministic else torch.float32, self.device)
+            dtype = torch.int64 if _deterministic(self.deterministic) else torch.float32
+            self.buf = _zeros_nhwc(v, c, h, w, dtype, self.device)
         return self.buf
 
     def take(self) -> Optional[torch.Tensor]:
         """-> the fp32 accumulator (converted once from fixed point in the deterministic form)"""
         buf, self.buf = self.buf, None
-        if buf is not None and self.deterministic:
+        if buf is not None and buf.dtype == torch.int64:
             buf = fixed_to_float(buf)
         return buf
 
@@ -159,6 +185,26 @@ class _PackFeaturesSink(torch.autograd.Function):
         return _unpack(acc), None, None
 
 
+class _PackedSink(torch.autograd.Function):
+    """A tensor that is already channels-last, handed to the sink's consumers with ``deterministic=True``:
+    the gradient is the sink's accumulator, cast once to the input's dtype."""
+
+    @staticmethod
+    def forward(ctx, x: torch.Tensor, dtype: torch.dtype, sink: FeatureGradSink):
+        ctx.sink = sink
+        ctx.in_dtype = x.dtype
+        ctx.set_materialize_grads(False)
+        return x.view_as(x) if x.dtype == dtype else x.to(dtype)
+
+    @staticmethod
+    def backward(ctx, g):
+        acc = ctx.sink.take()
+        if g is not None:                   # a consumer that does not know the sink
+            g = g.float()
+            acc = g if acc is None else acc.add_(g)
+        return (None if acc is None else acc.to(ctx.in_dtype)), None, None
+
+
 class _PackFeatures(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x: torch.Tensor, dtype: torch.dtype):
@@ -180,11 +226,17 @@ def pack_features(x: torch.Tensor, dtype: torch.dtype = torch.float32, sink: boo
 
     ``sink=True`` returns ``(packed, FeatureGradSink | None)``: when ``x`` needs a gradient and goes
     through the transpose kernel, the sink collects the fp32 gradients of the consumers that are
-    given it (``plane_sweep_variance(..., grad_sink=)``, ``backproject_aggregate(..., grad_sink=)``)."""
+    given it (``plane_sweep_variance(..., grad_sink=)``, ``backproject_aggregate(..., grad_sink=)``).
+    ``deterministic=True`` makes that accumulator int64 fixed point, and also gives a sink to an
+    already channels-last ``x`` that needs a gradient; ``torch.use_deterministic_algorithms(True)``
+    makes every sink fixed point, and every backward without one too."""
     _need_cuda("features", x)
     if x.dim() != 4:
         raise ValueError("features must be [V,C,H,W]")
     if _is_nhwc(x) and x.shape[1] > 1:
+        if sink and deterministic and x.requires_grad and torch.is_grad_enabled():
+            gs = FeatureGradSink(x.shape, x.device, True)
+            return _PackedSink.apply(x, dtype, gs), gs
         out = x if x.dtype == dtype else x.to(dtype)
         return (out, None) if sink else out
     if x.dtype != torch.float32 or not x.is_contiguous():
@@ -239,14 +291,29 @@ def _sweep_fwd_raw(feat, nbr_ids, hom, depth_values, out_dtype, ref_begin):
     return out
 
 
+def _fixed_acc(acc, feat) -> Optional[torch.Tensor]:
+    """The int64 fixed-point accumulator a scatter backward adds into, or None for the fp32-RED form:
+    the sink's (its dtype is the policy, fixed at its first use), or without a sink a private zero-filled
+    one when ``_deterministic()``."""
+    if acc is not None:
+        return acc if acc.dtype == torch.int64 else None
+    return _zeros_nhwc(*feat.shape, torch.int64, feat.device) if _deterministic() else None
+
+
+def _fixed_result(q, acc, feat):
+    """after a ``*_det`` launch into q: None into a sink, else dL/dfeat in feat's dtype"""
+    return None if acc is not None else fixed_to_float(q).to(feat.dtype)
+
+
 def _sweep_bwd_raw(g, feat, nbr_ids, hom, depth_values, ref_begin, acc=None):
     """-> dL/dfeat in feat's dtype, channels_last.  ``acc``: an fp32 channels-last accumulator to
     RED into instead (FeatureGradSink); returns None then."""
     gdt = torch.bfloat16 if (g.dtype == torch.bfloat16 and feat.dtype == torch.bfloat16) else torch.float32
     g = _as_ndhwc(g, gdt)
-    if acc is not None and acc.dtype == torch.int64:        # deterministic sink: fixed-point integer REDs
-        _lib.plane_sweep_bwd_det(g, feat, nbr_ids, hom, depth_values, acc, ref_begin=ref_begin)
-        return None
+    q = _fixed_acc(acc, feat)
+    if q is not None:                                       # fixed-point integer REDs
+        _lib.plane_sweep_bwd_det(g, feat, nbr_ids, hom, depth_values, q, ref_begin=ref_begin)
+        return _fixed_result(q, acc, feat)
     g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
     _lib.plane_sweep_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin=ref_begin)
     return None if acc is not None else g_feat.to(feat.dtype)
@@ -326,9 +393,10 @@ def _corr_bwd_raw(g, feat, nbr_ids, hom, depth_values, ref_begin, acc=None):
     accumulator ``acc`` (FeatureGradSink: fp32, or int64 fixed point for the deterministic form)"""
     # no copy when it arrives in the forward's layout
     g = g.float().permute(0, 1, 3, 4, 5, 2).contiguous().permute(0, 1, 5, 2, 3, 4)
-    if acc is not None and acc.dtype == torch.int64:        # deterministic sink: fixed-point integer REDs
-        _lib.plane_sweep_groupcorr_bwd_det(g, feat, nbr_ids, hom, depth_values, acc, ref_begin=ref_begin)
-        return None
+    q = _fixed_acc(acc, feat)
+    if q is not None:                                       # fixed-point integer REDs
+        _lib.plane_sweep_groupcorr_bwd_det(g, feat, nbr_ids, hom, depth_values, q, ref_begin=ref_begin)
+        return _fixed_result(q, acc, feat)
     g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
     _lib.plane_sweep_groupcorr_bwd(g, feat, nbr_ids, hom, depth_values, g_feat, ref_begin=ref_begin)
     return None if acc is not None else g_feat.to(feat.dtype)
@@ -388,6 +456,10 @@ class _HomoWarp(torch.autograd.Function):
         hom, depth_values = ctx.saved_tensors
         shape, sdtype = ctx.src_meta
         g = _as_ndhwc(g, torch.float32 if g.dtype != torch.bfloat16 else torch.bfloat16)
+        if _deterministic():                                # fixed-point integer REDs
+            q = _zeros_nhwc(*shape, torch.int64, g.device)
+            _lib.homo_warp_bwd_det(g, hom, depth_values, q)
+            return fixed_to_float(q).to(sdtype), None, None, None
         g_src = _zeros_nhwc(*shape, torch.float32, g.device)
         _lib.homo_warp_bwd(g, hom, depth_values, g_src)
         return g_src.to(sdtype), None, None, None
@@ -669,6 +741,19 @@ def _zeros_strided_like(t: torch.Tensor) -> torch.Tensor:
     return torch.empty_strided(t.size(), t.stride(), dtype=t.dtype, device=t.device).zero_()
 
 
+def _fixed_zeros_strided_like(t: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """-> (base, view): an int64 fixed-point accumulator with t's sizes and strides (the kernels address
+    it with prob's strides) as a view of a zero-filled flat base that spans its whole extent, gaps included"""
+    extent = 1 + sum((n - 1) * s for n, s in zip(t.shape, t.stride())) if t.numel() else 0
+    base = torch.zeros(extent, dtype=torch.int64, device=t.device)
+    return base, base.as_strided(t.size(), t.stride())
+
+
+def _fixed_to_float_strided(base: torch.Tensor, view: torch.Tensor) -> torch.Tensor:
+    """the fp32 values of ``_fixed_zeros_strided_like``'s accumulator, with the view's sizes and strides"""
+    return fixed_to_float(base).as_strided(view.size(), view.stride())
+
+
 def _bp_fwd_raw(feat, points, projection, est_depth, est_dens, vs_z, h, w, mode, channels_first,
                 out=None, count=None):
     """aggregating modes; -> (volume logical [C,N], count)"""
@@ -696,17 +781,19 @@ def _bp_bwd_raw(g_out, feat, points, projection, est_depth, est_dens, count, vs_
     (FeatureGradSink accumulator) the feature gradient is RED-added there and None is returned"""
     g_out = g_out.float()
     g_mem = g_out.contiguous() if channels_first else g_out.t().contiguous().t()
-    if acc is not None and acc.dtype == torch.int64:        # deterministic sink (MEAN mode only)
-        if mode != BP_MEAN:
-            raise ValueError("the deterministic backward is built for the mean aggregation only")
-        g_pn_q = torch.zeros(est_dens.shape, dtype=torch.int64, device=feat.device)
+    q = _fixed_acc(acc, feat)
+    if q is not None:                                       # fixed-point integer REDs
+        g_pn_base, g_pn_q = _fixed_zeros_strided_like(est_dens)
         g_prob = _zeros_strided_like(est_dens)
-        if g_pn_q.stride() != est_depth.stride():           # g_pn_q: contiguous [V,T,fh,fw]
-            raise ValueError("the deterministic backward needs contiguous [V,T,H,W] hypotheses")
-        _lib.backproject_bwd_det(g_mem, count, feat, points, projection, est_depth, est_dens, acc, g_pn_q,
-                                 vs_z=vs_z, height=h, width=w, channels_first=channels_first)
-        _lib.prob_norm_bwd(est_dens, fixed_to_float(g_pn_q), g_prob, height=h, width=w)
-        return None, g_prob
+        args = (g_mem, feat, points, projection, est_depth, est_dens)
+        if mode == BP_MEAN:
+            _lib.backproject_bwd_det(g_mem, count, *args[1:], q, g_pn_q, vs_z=vs_z, height=h, width=w,
+                                     channels_first=channels_first)
+        else:
+            _lib.backproject_bwd_det_mode(*args, q, g_pn_q, vs_z=vs_z, mode=mode, height=h, width=w,
+                                          channels_first=channels_first)
+        _lib.prob_norm_bwd(est_dens, _fixed_to_float_strided(g_pn_base, g_pn_q), g_prob, height=h, width=w)
+        return _fixed_result(q, acc, feat), g_prob
     g_feat = acc if acc is not None else _zeros_nhwc(*feat.shape, torch.float32, feat.device)
     g_pn = _zeros_strided_like(est_dens)
     g_prob = _zeros_strided_like(est_dens)
@@ -830,12 +917,18 @@ class _BackprojectPerView(torch.autograd.Function):
         feat, points, projection, depth, prob = ctx.saved_tensors
         vs_z, h, w = ctx.consts
         g_mem = g_out.float().permute(0, 2, 1).contiguous().permute(0, 2, 1)
-        g_feat = _zeros_nhwc(*feat.shape, torch.float32, feat.device)
-        g_pn = _zeros_strided_like(prob)
         g_prob = _zeros_strided_like(prob)
         prob_t = _per_view_hyp(prob, h, w)
-        _lib.backproject_bwd(g_mem, feat, points, projection, _per_view_hyp(depth, h, w), prob_t, g_feat, g_pn,
-                             vs_z=vs_z, mode=BP_PER_VIEW, height=h, width=w)
+        args = (g_mem, feat, points, projection, _per_view_hyp(depth, h, w), prob_t)
+        if _deterministic():                                # fixed-point integer REDs
+            q = _zeros_nhwc(*feat.shape, torch.int64, feat.device)
+            g_pn_base, g_pn_q = _fixed_zeros_strided_like(prob)
+            _lib.backproject_bwd_det_mode(*args, q, g_pn_q, vs_z=vs_z, mode=BP_PER_VIEW, height=h, width=w)
+            _lib.prob_norm_bwd(prob_t, _fixed_to_float_strided(g_pn_base, g_pn_q), g_prob, height=h, width=w)
+            return fixed_to_float(q).to(feat.dtype), None, None, None, g_prob, None, None, None
+        g_feat = _zeros_nhwc(*feat.shape, torch.float32, feat.device)
+        g_pn = _zeros_strided_like(prob)
+        _lib.backproject_bwd(*args, g_feat, g_pn, vs_z=vs_z, mode=BP_PER_VIEW, height=h, width=w)
         _lib.prob_norm_bwd(prob_t, g_pn, g_prob, height=h, width=w)
         return g_feat.to(feat.dtype), None, None, None, g_prob, None, None, None
 

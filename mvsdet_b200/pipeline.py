@@ -28,7 +28,7 @@ from typing import Dict, Optional
 
 import torch
 
-from . import _lib
+from . import _lib, ops
 from ._lib import BP_MEAN
 from .geometry import SceneGeometry
 from .scene import SceneConfig
@@ -132,6 +132,8 @@ class ScenePipeline:
         geo = self.geo
         if geo is None:
             raise RuntimeError("set_geometry() first")
+        # its backward kernels RED in fp32, in an order that varies from run to run
+        ops._alert_not_deterministic("ScenePipeline.step")
         cfg = self.cfg
         h, w = geo.height, geo.width
         near, interval = cfg.near_far_range[0], cfg.depth_interval

@@ -556,6 +556,8 @@ class ShardedScenePipeline:
         ``g_variance`` logical [Vb,C,D,Hf,Wf] in channels_last_3d for this rank's reference views (rows in
         the order of ``self.view_ids``).
         -> (g_feature [Vb,C,Hf,Wf] fp32 for the rank's own views ``self.view_ids``, g_cost_out [Vb,2,D,Hf,Wf])."""
+        # its backward kernels RED in fp32, in an order that varies from run to run
+        ops._alert_not_deterministic("ShardedScenePipeline.backward")
         cfg, lg, geo = self.cfg, self.lg, self.lg.geo
         dev = self.device
         vl, vb, c, n = self.vl, self.vb, self.c, self.n
