@@ -36,7 +36,9 @@
  *   mvsd_plane_sweep_groupcorr_bwd_det, mvsd_plane_sweep_groupcorr_bwd_det_px --
  *   the deterministic group-correlation backward;
  *   mvsd_homo_warp_bwd_det, mvsd_backproject_bwd_det_mode -- the deterministic
- *   backwards of the stand-alone warp and of the SUM / PER_VIEW back-projection.
+ *   backwards of the stand-alone warp and of the SUM / PER_VIEW back-projection;
+ *   mvsd_halo_reduce_p2p_fixed -- the halo pull of a view-sharded scene over the
+ *   64-bit fixed-point accumulators of the deterministic backwards.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -457,6 +459,15 @@ int mvsd_voxel_reduce_p2p(const void* const* part_ptrs, void* const* out_ptrs,
 int mvsd_halo_reduce_p2p(void* const* g_ptrs, const int32_t* pull_offsets,
                          const int32_t* pull_sources, int world, int rank, int n_own,
                          int64_t view_elems, void* stream);
+/* The same pull over the int64 fixed-point accumulators of the deterministic backwards
+ * (mvsd_plane_sweep_bwd_det, mvsd_backproject_bwd_det; 32 fractional bits): same arguments,
+ * checks and grid (messages name halo_reduce_p2p_fixed), except that the peer buffers are
+ * int64 [V_local][view_elems] and the owner adds its peers' rows with integer adds.  Integer
+ * addition does not depend on order, so after mvsd_fixed_to_float the owned rows are the bits
+ * of the single-GPU deterministic gradient, whatever the number of ranks and the split.     */
+int mvsd_halo_reduce_p2p_fixed(void* const* g_ptrs, const int32_t* pull_offsets,
+                               const int32_t* pull_sources, int world, int rank, int n_own,
+                               int64_t view_elems, void* stream);
 
 #ifdef __cplusplus
 }

@@ -71,6 +71,7 @@ SIGNATURES = {
     "mvsd_voxel_normalize": ([_p, _p, _p, _i, _i, _i, _p], _i),
     "mvsd_voxel_reduce_p2p": ([_p, _p, _p, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_halo_reduce_p2p": ([_p, _p, _p, _i, _i, _i, _l, _p], _i),
+    "mvsd_halo_reduce_p2p_fixed": ([_p, _p, _p, _i, _i, _i, _l, _p], _i),
 }
 
 
@@ -335,9 +336,18 @@ def voxel_reduce_p2p(part_ptrs, out_ptrs, count_local, *, world, rank, channels,
          channels, count_local.numel(), _stream())
 
 
+def _halo_reduce(name, g_ptrs, pull_offsets, pull_sources, world, rank, view_elems):
+    call(name, g_ptrs, pull_offsets.data_ptr(), pull_sources.data_ptr(), world, rank, pull_offsets.numel() - 1,
+         view_elems, _stream())
+
+
 def halo_reduce_p2p(g_ptrs, pull_offsets, pull_sources, *, world, rank, view_elems):
-    call("mvsd_halo_reduce_p2p", g_ptrs, pull_offsets.data_ptr(), pull_sources.data_ptr(), world, rank,
-         pull_offsets.numel() - 1, view_elems, _stream())
+    _halo_reduce("mvsd_halo_reduce_p2p", g_ptrs, pull_offsets, pull_sources, world, rank, view_elems)
+
+
+def halo_reduce_p2p_fixed(g_ptrs, pull_offsets, pull_sources, *, world, rank, view_elems):
+    """``halo_reduce_p2p`` over int64 fixed-point accumulators"""
+    _halo_reduce("mvsd_halo_reduce_p2p_fixed", g_ptrs, pull_offsets, pull_sources, world, rank, view_elems)
 
 
 def fixed_to_float(src, dst):

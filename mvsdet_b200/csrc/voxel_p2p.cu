@@ -96,30 +96,82 @@ __global__ void __launch_bounds__(256) p2p_reduce_kernel(const P2PParams p) {
 // pointers, one CTA column per (owned view, 16-byte chunk), sources in table order -> the same
 // summation order on every run (deterministic).  pulls: CSR over the owned views --
 // offs[d] .. offs[d+1] index (src_rank, src_local_view) pairs.
+// The element type is fp32 (mvsd_halo_reduce_p2p) or the 64-bit fixed point of the *_det scatter
+// backwards (mvsd_halo_reduce_p2p_fixed, common.cuh), whose integer adds make the owner's sum
+// independent of how the views were split over the ranks.  Both move 16 bytes per peer load.
+template <typename T>
 struct HaloParams {
-  float* const* g;            // device array [world]: peers' gradient buffers [V_local][view_elems] fp32
+  T* const* g;                // device array [world]: peers' gradient buffers [V_local][view_elems]
   const int32_t* offs;        // [n_own + 1]
   const int32_t* src;         // [n_pull][2]
   int rank, n_own;
   size_t view_elems;          // H*W*C, multiple of 4
 };
 
-__global__ void __launch_bounds__(256) halo_reduce_kernel(const HaloParams p) {
+template <typename T> struct HaloVec;
+template <> struct HaloVec<float> {                 // one float4
+  using V16 = float4;
+  static constexpr int kElems = 4;
+  static __device__ __forceinline__ float4 ld_peer(const float* p) { return ld_peer4(p); }
+  static __device__ __forceinline__ float4 add(float4 s, float4 t) {
+    s.x = __fadd_rn(s.x, t.x); s.y = __fadd_rn(s.y, t.y);
+    s.z = __fadd_rn(s.z, t.z); s.w = __fadd_rn(s.w, t.w);
+    return s;
+  }
+};
+template <> struct HaloVec<long long> {             // two long long
+  using V16 = longlong2;
+  static constexpr int kElems = 2;
+  static __device__ __forceinline__ longlong2 ld_peer(const long long* p) {
+    return __ldcv(reinterpret_cast<const longlong2*>(p));
+  }
+  static __device__ __forceinline__ longlong2 add(longlong2 s, longlong2 t) {
+    // two's-complement wrap-around: exact whenever the true sum fits, whatever the order
+    s.x = (long long)((unsigned long long)s.x + (unsigned long long)t.x);
+    s.y = (long long)((unsigned long long)s.y + (unsigned long long)t.y);
+    return s;
+  }
+};
+
+template <typename T>
+__global__ void __launch_bounds__(256) halo_reduce_kernel(const HaloParams<T> p) {
+  using Vec = HaloVec<T>;
+  using V16 = typename Vec::V16;
+  constexpr int kE = Vec::kElems;
   const int d = blockIdx.y;
   const int b = p.offs[d], e = p.offs[d + 1];
   if (b == e) return;
-  float* mine = p.g[p.rank] + (size_t)d * p.view_elems;
-  const size_t n4 = p.view_elems >> 2;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
-    float4 s = *reinterpret_cast<const float4*>(mine + (i << 2));
+  T* mine = p.g[p.rank] + (size_t)d * p.view_elems;
+  const size_t nv = p.view_elems / kE;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (size_t)gridDim.x * blockDim.x) {
+    V16 s = *reinterpret_cast<const V16*>(mine + i * kE);
     for (int q = b; q < e; ++q) {
-      const float* peer = p.g[p.src[2 * q]] + (size_t)p.src[2 * q + 1] * p.view_elems;
-      const float4 t = ld_peer4(peer + (i << 2));
-      s.x = __fadd_rn(s.x, t.x); s.y = __fadd_rn(s.y, t.y);
-      s.z = __fadd_rn(s.z, t.z); s.w = __fadd_rn(s.w, t.w);
+      const T* peer = p.g[p.src[2 * q]] + (size_t)p.src[2 * q + 1] * p.view_elems;
+      s = Vec::add(s, Vec::ld_peer(peer + i * kE));
     }
-    *reinterpret_cast<float4*>(mine + (i << 2)) = s;
+    *reinterpret_cast<V16*>(mine + i * kE) = s;
   }
+}
+
+// one CTA column per owned view, at most 64 CTAs (of 256 threads, one 16-byte vector each) across a view
+template <typename T>
+int halo_reduce(const char* who, void* const* g_ptrs, const int32_t* pull_offsets, const int32_t* pull_sources,
+                int world, int rank, int n_own, int64_t view_elems, void* stream) {
+  if (!g_ptrs || !pull_offsets || !pull_sources)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (world < 1 || world > kMaxPeers || rank < 0 || rank >= world)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: bad world/rank (%d/%d)", who, rank, world);
+  if (n_own <= 0 || n_own > 65535 || view_elems <= 0 || (view_elems & 3))
+    return fail(MVSD_ERR_INVALID_ARG, "%s: bad view count / size", who);
+  HaloParams<T> p;
+  p.g = reinterpret_cast<T* const*>(g_ptrs);
+  p.offs = pull_offsets; p.src = pull_sources; p.rank = rank; p.n_own = n_own;
+  p.view_elems = (size_t)view_elems;
+  const size_t want = ((size_t)view_elems / HaloVec<T>::kElems + 255) / 256;
+  dim3 grid((unsigned)(want < 64 ? want : 64), (unsigned)n_own);
+  halo_reduce_kernel<T><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
+  count_launch();
+  return check_launch(who);
 }
 
 }  // namespace
@@ -130,21 +182,15 @@ using namespace mvsd;
 extern "C" int mvsd_halo_reduce_p2p(void* const* g_ptrs, const int32_t* pull_offsets,
                                     const int32_t* pull_sources, int world, int rank, int n_own,
                                     int64_t view_elems, void* stream) {
-  if (!g_ptrs || !pull_offsets || !pull_sources)
-    return fail(MVSD_ERR_INVALID_ARG, "halo_reduce_p2p: null pointer");
-  if (world < 1 || world > kMaxPeers || rank < 0 || rank >= world)
-    return fail(MVSD_ERR_INVALID_ARG, "halo_reduce_p2p: bad world/rank (%d/%d)", rank, world);
-  if (n_own <= 0 || n_own > 65535 || view_elems <= 0 || (view_elems & 3))
-    return fail(MVSD_ERR_INVALID_ARG, "halo_reduce_p2p: bad view count / size");
-  HaloParams p;
-  p.g = reinterpret_cast<float* const*>(g_ptrs);
-  p.offs = pull_offsets; p.src = pull_sources; p.rank = rank; p.n_own = n_own;
-  p.view_elems = (size_t)view_elems;
-  const size_t want = ((size_t)view_elems / 4 + 255) / 256;
-  dim3 grid((unsigned)(want < 64 ? want : 64), (unsigned)n_own);
-  halo_reduce_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
-  count_launch();
-  return check_launch("halo_reduce_p2p");
+  return halo_reduce<float>("halo_reduce_p2p", g_ptrs, pull_offsets, pull_sources, world, rank, n_own,
+                            view_elems, stream);
+}
+
+extern "C" int mvsd_halo_reduce_p2p_fixed(void* const* g_ptrs, const int32_t* pull_offsets,
+                                          const int32_t* pull_sources, int world, int rank, int n_own,
+                                          int64_t view_elems, void* stream) {
+  return halo_reduce<long long>("halo_reduce_p2p_fixed", g_ptrs, pull_offsets, pull_sources, world, rank,
+                                n_own, view_elems, stream);
 }
 
 extern "C" int mvsd_voxel_reduce_p2p(const void* const* part_ptrs, void* const* out_ptrs,

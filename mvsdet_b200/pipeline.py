@@ -21,6 +21,12 @@ allocator, and can therefore be captured once into a CUDA graph and replayed:
 It also provides the host-buffer form of the same call (``run_host``): pinned
 host inputs are copied in, the step runs, results are copied out -- the
 end-to-end path bench.py reports as ``e2e``.
+
+``deterministic=True`` gives the bit-reproducible form of the same step: the two
+scatter backwards (voxels bwd, sweep bwd) add into int64 fixed-point accumulators
+(``*_det`` kernels, integer REDs) that ``mvsd_fixed_to_float`` converts once, so
+``g_feature`` and ``g_cost_out`` are the bits of ``MVSDetHotPath(deterministic=True)``
+on every run.  It is the form that runs under ``torch.use_deterministic_algorithms(True)``.
 """
 from __future__ import annotations
 
@@ -39,10 +45,12 @@ __all__ = ["ScenePipeline"]
 class ScenePipeline:
     INPUTS = ("feature", "cost_out", "g_volume_mean", "g_variance")
     OUTPUTS = ("volume_mean", "count", "g_feature", "g_cost_out")
+    deterministic = False          # fp32-RED backward (the default, fastest form)
 
     def __init__(self, cfg: SceneConfig, device="cuda", feature_dtype=torch.bfloat16,
-                 variance_dtype=torch.float32, pack_input: bool = True):
+                 variance_dtype=torch.float32, pack_input: bool = True, deterministic: bool = False):
         self.cfg = cfg
+        self.deterministic = bool(deterministic)
         self.device = torch.device(device)
         self.feature_dtype = feature_dtype
         self.variance_dtype = variance_dtype
@@ -70,6 +78,11 @@ class ScenePipeline:
         self.g_pn = torch.empty((v, t, hf, wf), **f32)
         self.g_est_dens = torch.zeros((v, t, hf, wf), **f32)
         self.g_feat_cl = torch.empty((v, hf, wf, c), **f32)
+        if self.deterministic:
+            # the fixed-point accumulators of the *_det kernels; g_feat_cl and g_pn take their conversions
+            self.g_feat_q = torch.empty((v, hf, wf, c), dtype=torch.int64, device=dev)
+            self.g_pn_q = torch.empty((v, t, hf, wf), dtype=torch.int64, device=dev)
+            self._g_feat_q = self.g_feat_q.permute(0, 3, 1, 2)
         # outputs
         self.volume_mean = torch.empty((c, n), **f32)
         self.count = torch.empty((n,), dtype=torch.int32, device=dev)
@@ -111,7 +124,7 @@ class ScenePipeline:
         bv = self.variance.element_size()
         feat = v * c * hf * wf
         vol = v * c * d * hf * wf
-        return {
+        out = {
             "pack": feat * 4 + feat * bf,
             "plane_sweep_fwd": feat * bf + vol * bv,
             "depth_topk_fwd": 2 * v * d * hf * wf * 4 + 2 * v * d * hf * wf * 4
@@ -123,6 +136,13 @@ class ScenePipeline:
             "plane_sweep_bwd": vol * bv + feat * bf + feat * 4,
             "unpack": feat * 4 * 2,
         }
+        if self.deterministic:
+            # the scatter backwards write 8-byte fixed-point accumulators, each converted once (read 8, write 4)
+            out["backproject_bwd_det"] = out.pop("backproject_bwd") + v * c * h * w * 4 + v * h * w * t * 4
+            out["plane_sweep_bwd_det"] = out.pop("plane_sweep_bwd") + feat * 4
+            out["fixed_to_float_pn"] = v * t * hf * wf * (8 + 4)
+            out["fixed_to_float_feat"] = feat * (8 + 4)
+        return out
 
     # ------------------------------------------------------------------
     def step(self, timers: Optional[Dict] = None) -> None:
@@ -132,8 +152,10 @@ class ScenePipeline:
         geo = self.geo
         if geo is None:
             raise RuntimeError("set_geometry() first")
-        # its backward kernels RED in fp32, in an order that varies from run to run
-        ops._alert_not_deterministic("ScenePipeline.step")
+        det = self.deterministic
+        if not det:
+            # its backward kernels RED in fp32, in an order that varies from run to run
+            ops._alert_not_deterministic("ScenePipeline.step")
         cfg = self.cfg
         h, w = geo.height, geo.width
         near, interval = cfg.near_far_range[0], cfg.depth_interval
@@ -158,7 +180,13 @@ class ScenePipeline:
                 run("backproject_fwd", _lib.backproject_fwd, *hyp, self.volume_mean, **bp)
                 # ---- backward
                 aux.wait_stream(self._side)
-                run("backproject_bwd", _lib.backproject_bwd, self.g_volume_mean, *hyp, self._g_feat, self.g_pn, **bp)
+                if det:
+                    run("backproject_bwd_det", _lib.backproject_bwd_det, self.g_volume_mean, self.count, *hyp,
+                        self._g_feat_q, self.g_pn_q, vs_z=cfg.voxel_size[2], height=h, width=w, channels_first=True)
+                    run("fixed_to_float_pn", _lib.fixed_to_float, self.g_pn_q, self.g_pn)
+                else:
+                    run("backproject_bwd", _lib.backproject_bwd, self.g_volume_mean, *hyp, self._g_feat, self.g_pn,
+                        **bp)
                 run("prob_norm_bwd", _lib.prob_norm_bwd, self.est_dens, self.g_pn, self.g_est_dens, height=h,
                     width=w)
                 run("depth_topk_bwd", _lib.depth_topk_bwd, self.cost_out, self.est_idx, None, None, None,
@@ -169,8 +197,10 @@ class ScenePipeline:
         #   _aux   top-k fwd -> voxels fwd -> voxels bwd -> pn bwd -> top-k bwd
         #          small latency-bound kernels (2-3 waves, L2-resident operands) that depend only
         #          on pack; they run under the sweep kernels at higher stream priority.  The two
-        #          backward kernels accumulate into g_feat_cl with commutative REDs.
-        #   _side  zero-fills of the gradient accumulators (98 MB + 1 MB), no producer
+        #          backward kernels accumulate into g_feat_cl with commutative REDs -- with
+        #          ``deterministic`` into g_feat_q with integer REDs, which also commute (and
+        #          associate), so the overlap leaves the fixed-point sums' bits unchanged.
+        #   _side  zero-fills of the gradient accumulators (98 MB + 1 MB; int64: twice that), no producer
         # With ``timers`` the kernels run back to back on ``cur`` so each can be timed alone.
         cur = torch.cuda.current_stream()
         overlap = timers is None and self.overlap_small
@@ -181,8 +211,12 @@ class ScenePipeline:
         # next to a 98 MB memset) and run under the forward sweep instead
         self._side.wait_stream(cur)
         with torch.cuda.stream(self._side):
-            self.g_feat_cl.zero_()
-            self.g_pn.zero_()
+            if det:
+                self.g_feat_q.zero_()
+                self.g_pn_q.zero_()
+            else:
+                self.g_feat_cl.zero_()
+                self.g_pn.zero_()
         if overlap:
             aux.wait_stream(cur)
             small_kernels()
@@ -191,9 +225,14 @@ class ScenePipeline:
             cur.wait_stream(self._side)
         else:
             small_kernels()
-        run("plane_sweep_bwd", _lib.plane_sweep_bwd, self._g_variance, *sweep, self._g_feat)
+        if det:
+            run("plane_sweep_bwd_det", _lib.plane_sweep_bwd_det, self._g_variance, *sweep, self._g_feat_q)
+        else:
+            run("plane_sweep_bwd", _lib.plane_sweep_bwd, self._g_variance, *sweep, self._g_feat)
         if overlap:
             cur.wait_stream(aux)
+        if det:
+            run("fixed_to_float_feat", _lib.fixed_to_float, self.g_feat_q, self.g_feat_cl)
         run("unpack", _lib.unpack, self._g_feat, self.g_feature)
 
     # ------------------------------------------------------------------

@@ -394,13 +394,21 @@ class ShardedScenePipeline:
     back-projection / prob-norm / top-k / sweep backward run locally into one fp32 accumulator
     over block + halo views, then each owner pulls its peers' halo contributions over NVLink
     (``mvsd_halo_reduce_p2p``): the result is dL/dfeature for the rank's own block -- a
-    reduce-scatter of the scene's feature gradient with 2-4 views of traffic per rank."""
+    reduce-scatter of the scene's feature gradient with 2-4 views of traffic per rank.
+
+    A hot path with ``deterministic=True`` makes the backward deterministic, as it makes the hot path's
+    own: the scatter backwards add into an int64 fixed-point accumulator (``*_det`` kernels) and the
+    owners pull with ``mvsd_halo_reduce_p2p_fixed``.  Every contribution to a view is then summed as an
+    integer, in no particular order, so a rank's ``g_feature`` rows are the bits of the single-GPU
+    deterministic gradient of those views, for any number of ranks and any split of the views."""
+    deterministic = False          # fp32-RED backward
 
     def __init__(self, hot_path, cfg, device, group=None):
         import torch.distributed._symmetric_memory as symm
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("ShardedScenePipeline needs an initialised process group")
         self.hot, self.cfg, self.device = hot_path, cfg, torch.device(device)
+        self.deterministic = bool(hot_path.deterministic)
         self.group = group if group is not None else dist.group.WORLD
         self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
         self._symm = symm
@@ -556,19 +564,24 @@ class ShardedScenePipeline:
         ``g_variance`` logical [Vb,C,D,Hf,Wf] in channels_last_3d for this rank's reference views (rows in
         the order of ``self.view_ids``).
         -> (g_feature [Vb,C,Hf,Wf] fp32 for the rank's own views ``self.view_ids``, g_cost_out [Vb,2,D,Hf,Wf])."""
-        # its backward kernels RED in fp32, in an order that varies from run to run
-        ops._alert_not_deterministic("ShardedScenePipeline.backward")
+        det = self.deterministic
+        if not det:
+            # its backward kernels RED in fp32, in an order that varies from run to run
+            ops._alert_not_deterministic("ShardedScenePipeline.backward")
         cfg, lg, geo = self.cfg, self.lg, self.lg.geo
         dev = self.device
         vl, vb, c, n = self.vl, self.vb, self.c, self.n
         d, t = cfg.num_depth, cfg.topk
         hf, wf = cfg.feat_hw
+        view_elems = hf * wf * c
         if self._g_feat is None:
-            view_elems = hf * wf * c
             # every rank allocates for the same (maximum) number of local views: symmetric allocation
             vl_max = torch.tensor([vl], device=dev)
             dist.all_reduce(vl_max, op=dist.ReduceOp.MAX, group=self.group)
-            self._g_feat = self._symm.empty(int(vl_max.item()) * view_elems, dtype=torch.float32, device=dev)
+            # deterministic: the accumulator is int64 fixed point, g_pn_q too; the owned rows of the
+            # accumulator are converted into g_feat_own after the pull (the halo rows are scratch)
+            acc_dtype = torch.int64 if det else torch.float32
+            self._g_feat = self._symm.empty(int(vl_max.item()) * view_elems, dtype=acc_dtype, device=dev)
             self._h_g = self._symm.rendezvous(self._g_feat, self.group)
             offs, src = halo_pull_table(self.nbr_full, self.world, self.rank)
             self._pull_offs, self._pull_src = offs.to(dev), src.to(dev)
@@ -577,6 +590,9 @@ class ShardedScenePipeline:
             self.g_est_dens = torch.zeros((vb, t, hf, wf), dtype=torch.float32, device=dev)
             self.g_cost_out = torch.empty((vb, 2, d, hf, wf), dtype=torch.float32, device=dev)
             self.g_feature = torch.empty((vb, c, hf, wf), dtype=torch.float32, device=dev)
+            if det:
+                self.g_pn_q = torch.empty((vb, t, hf, wf), dtype=torch.int64, device=dev)
+                self.g_feat_own = torch.empty(vb * view_elems, dtype=torch.float32, device=dev)
         slot = self._last_slot
         g_vol = g_volume_mean.reshape(c, n).float().contiguous()
         gv = g_variance if g_variance.permute(0, 2, 3, 4, 1).is_contiguous() else \
@@ -588,18 +604,24 @@ class ShardedScenePipeline:
             cur = torch.cuda.current_stream()
             hyp = (self.feat_cl, geo.points, geo.projection, self.est_depth, self.est_dens)
             self._g_feat.zero_()
-            self.g_pn.zero_()
+            (self.g_pn_q if det else self.g_pn).zero_()
             # the three small kernels run on a higher-priority side stream under the sweep backward
             # (all of them RED into the same accumulator: the order does not matter)
             self.s_aux.wait_stream(cur)
             with torch.cuda.stream(self.s_aux):
-                _lib.backproject_bwd(g_vol, *hyp, self._g_feat, self.g_pn, vs_z=cfg.voxel_size[2], mode=BP_MEAN,
-                                     height=geo.height, width=geo.width, channels_first=True,
-                                     count=self._red[slot].count_local)
+                count = self._red[slot].count_local
+                if det:
+                    _lib.backproject_bwd_det(g_vol, count, *hyp, self._g_feat, self.g_pn_q, vs_z=cfg.voxel_size[2],
+                                             height=geo.height, width=geo.width, channels_first=True)
+                    _lib.fixed_to_float(self.g_pn_q, self.g_pn)
+                else:
+                    _lib.backproject_bwd(g_vol, *hyp, self._g_feat, self.g_pn, vs_z=cfg.voxel_size[2], mode=BP_MEAN,
+                                         height=geo.height, width=geo.width, channels_first=True, count=count)
                 _lib.prob_norm_bwd(self.est_dens, self.g_pn, self.g_est_dens, height=geo.height, width=geo.width)
                 _lib.depth_topk_bwd(self.cost_out, self.est_idx, None, None, None, self.g_est_dens, None,
                                     self.g_cost_out, near=cfg.near_far_range[0], interval=cfg.depth_interval)
-            _lib.plane_sweep_bwd(gv, self.feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self._g_feat)
+            sweep_bwd = _lib.plane_sweep_bwd_det if det else _lib.plane_sweep_bwd
+            sweep_bwd(gv, self.feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self._g_feat)
             cur.wait_stream(self.s_aux)
 
         # the local chain is replayed as one CUDA graph while the caller keeps handing in the same
@@ -626,10 +648,15 @@ class ShardedScenePipeline:
         # owners pull the halo contributions of their peers
         self._h_g.barrier(channel=0)
         if self._n_pull:
-            _lib.halo_reduce_p2p(self._h_g.buffer_ptrs_dev, self._pull_offs, self._pull_src, world=self.world,
-                                 rank=self.rank, view_elems=hf * wf * c)
+            pull = _lib.halo_reduce_p2p_fixed if det else _lib.halo_reduce_p2p
+            pull(self._h_g.buffer_ptrs_dev, self._pull_offs, self._pull_src, world=self.world, rank=self.rank,
+                 view_elems=view_elems)
         self._h_g.barrier(channel=0)
-        _lib.unpack(self._g_feat, self.g_feature)
+        if det:
+            _lib.fixed_to_float(self._g_feat[:vb * view_elems], self.g_feat_own)
+            _lib.unpack(self.g_feat_own, self.g_feature)
+        else:
+            _lib.unpack(self._g_feat, self.g_feature)
         return self.g_feature, self.g_cost_out
 
     def close(self) -> None:
