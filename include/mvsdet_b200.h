@@ -38,7 +38,9 @@
  *   mvsd_homo_warp_bwd_det, mvsd_backproject_bwd_det_mode -- the deterministic
  *   backwards of the stand-alone warp and of the SUM / PER_VIEW back-projection;
  *   mvsd_halo_reduce_p2p_fixed -- the halo pull of a view-sharded scene over the
- *   64-bit fixed-point accumulators of the deterministic backwards.
+ *   64-bit fixed-point accumulators of the deterministic backwards;
+ *   mvsd_halo_gather_p2p -- the forward's halo exchange of a view-sharded scene:
+ *   each rank copies its halo views' packed maps from their owners.
  */
 #ifndef MVSDET_B200_H_
 #define MVSDET_B200_H_
@@ -468,6 +470,20 @@ int mvsd_halo_reduce_p2p(void* const* g_ptrs, const int32_t* pull_offsets,
 int mvsd_halo_reduce_p2p_fixed(void* const* g_ptrs, const int32_t* pull_offsets,
                                const int32_t* pull_sources, int world, int rank, int n_own,
                                int64_t view_elems, void* stream);
+
+/* Forward of a view-sharded scene whose ranks each hold the feature maps of their OWN views only: the
+ * forward counterpart of mvsd_halo_reduce_p2p.  feat_ptrs: DEVICE array of `world` peer pointers to the
+ * ranks' packed channels-last feature buffers [V_local][view_bytes] (own views first, then halo views;
+ * 16-byte aligned, e.g. torch symmetric memory).  For j in [0, n_halo) the row gather_sources[2*j+1] of
+ * peer gather_sources[2*j] is copied into this rank's row n_own + j; nothing else is written.  The rows
+ * are opaque bytes (bf16 or fp32 maps alike); view_bytes must be a positive multiple of 8 (every
+ * C % 4 == 0 map is), rows that are not multiples of 16 bytes move 8 bytes per load.  Checks and grid
+ * are those of mvsd_halo_reduce_p2p (messages name halo_gather_p2p; n_own and n_halo in [1, 65535]).
+ * The caller puts a cross-rank barrier before this call (every owner has packed its rows) and must not
+ * overwrite its own rows until every peer has finished its gather (a later barrier).             */
+int mvsd_halo_gather_p2p(void* const* feat_ptrs, const int32_t* gather_sources,
+                         int world, int rank, int n_own, int n_halo,
+                         int64_t view_bytes, void* stream);
 
 #ifdef __cplusplus
 }

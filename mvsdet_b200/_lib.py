@@ -72,6 +72,7 @@ SIGNATURES = {
     "mvsd_voxel_reduce_p2p": ([_p, _p, _p, _i, _i, _i, _i, _i, _p], _i),
     "mvsd_halo_reduce_p2p": ([_p, _p, _p, _i, _i, _i, _l, _p], _i),
     "mvsd_halo_reduce_p2p_fixed": ([_p, _p, _p, _i, _i, _i, _l, _p], _i),
+    "mvsd_halo_gather_p2p": ([_p, _p, _i, _i, _i, _i, _l, _p], _i),
 }
 
 
@@ -348,6 +349,12 @@ def halo_reduce_p2p(g_ptrs, pull_offsets, pull_sources, *, world, rank, view_ele
 def halo_reduce_p2p_fixed(g_ptrs, pull_offsets, pull_sources, *, world, rank, view_elems):
     """``halo_reduce_p2p`` over int64 fixed-point accumulators"""
     _halo_reduce("mvsd_halo_reduce_p2p_fixed", g_ptrs, pull_offsets, pull_sources, world, rank, view_elems)
+
+
+def halo_gather_p2p(feat_ptrs, gather_sources, *, world, rank, n_own, view_bytes):
+    """gather_sources [n_halo,2] int32 -> rows n_own.. of this rank's packed buffer from their owners"""
+    call("mvsd_halo_gather_p2p", feat_ptrs, gather_sources.data_ptr(), world, rank, n_own, gather_sources.shape[0],
+         view_bytes, _stream())
 
 
 def fixed_to_float(src, dst):

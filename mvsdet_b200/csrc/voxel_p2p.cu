@@ -153,22 +153,55 @@ __global__ void __launch_bounds__(256) halo_reduce_kernel(const HaloParams<T> p)
   }
 }
 
-// one CTA column per owned view, at most 64 CTAs (of 256 threads, one 16-byte vector each) across a view
+// Forward of a view-sharded scene from each rank's own feature maps: every rank packs the views it owns
+// into rows [0, n_own) of its peer-mapped buffer; after a cross-rank barrier it copies its halo views (the
+// neighbours of its reference views that other ranks own) from their owners into rows n_own + j.  The rows
+// are opaque bytes (bf16 or fp32 channels-last maps), moved in 16-byte vectors, or in 8-byte ones when a row
+// is not a multiple of 16 bytes (bf16 with H*W odd and C % 8 == 4: rows packed back to back then start
+// 8-byte aligned).  src[2j], src[2j+1] = (owner rank, row in the owner's buffer) of halo row j.
+struct GatherParams {
+  char* const* feat;          // device array [world]: peers' packed buffers [V_local][view_bytes]
+  const int32_t* src;         // [n_halo][2]
+  int rank, n_own;
+  size_t view_bytes;
+};
+
+template <typename V>           // uint4 or uint2
+__global__ void __launch_bounds__(256) halo_gather_kernel(const GatherParams p) {
+  const int j = blockIdx.y;
+  const V* peer = reinterpret_cast<const V*>(p.feat[p.src[2 * j]] + (size_t)p.src[2 * j + 1] * p.view_bytes);
+  V* mine = reinterpret_cast<V*>(p.feat[p.rank] + (size_t)(p.n_own + j) * p.view_bytes);
+  const size_t nv = p.view_bytes / sizeof(V);
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (size_t)gridDim.x * blockDim.x)
+    mine[i] = __ldcv(peer + i);                                  // never from a stale L1 line
+}
+
+// the rules and the grid both halo kernels follow: at most kMaxPeers ranks, one CTA column per row of
+// this rank they write, at most 64 CTAs (of 256 threads, one vector each) across a row
+int check_world(const char* who, int world, int rank) {
+  if (world < 1 || world > kMaxPeers || rank < 0 || rank >= world)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: bad world/rank (%d/%d)", who, rank, world);
+  return MVSD_OK;
+}
+
+dim3 halo_grid(size_t vecs_per_row, int rows) {
+  const size_t want = (vecs_per_row + 255) / 256;
+  return dim3((unsigned)(want < 64 ? want : 64), (unsigned)rows);
+}
+
 template <typename T>
 int halo_reduce(const char* who, void* const* g_ptrs, const int32_t* pull_offsets, const int32_t* pull_sources,
                 int world, int rank, int n_own, int64_t view_elems, void* stream) {
   if (!g_ptrs || !pull_offsets || !pull_sources)
     return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
-  if (world < 1 || world > kMaxPeers || rank < 0 || rank >= world)
-    return fail(MVSD_ERR_INVALID_ARG, "%s: bad world/rank (%d/%d)", who, rank, world);
+  if (int e = check_world(who, world, rank)) return e;
   if (n_own <= 0 || n_own > 65535 || view_elems <= 0 || (view_elems & 3))
     return fail(MVSD_ERR_INVALID_ARG, "%s: bad view count / size", who);
   HaloParams<T> p;
   p.g = reinterpret_cast<T* const*>(g_ptrs);
   p.offs = pull_offsets; p.src = pull_sources; p.rank = rank; p.n_own = n_own;
   p.view_elems = (size_t)view_elems;
-  const size_t want = ((size_t)view_elems / HaloVec<T>::kElems + 255) / 256;
-  dim3 grid((unsigned)(want < 64 ? want : 64), (unsigned)n_own);
+  const dim3 grid = halo_grid((size_t)view_elems / HaloVec<T>::kElems, n_own);
   halo_reduce_kernel<T><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
   count_launch();
   return check_launch(who);
@@ -191,6 +224,27 @@ extern "C" int mvsd_halo_reduce_p2p_fixed(void* const* g_ptrs, const int32_t* pu
                                           int64_t view_elems, void* stream) {
   return halo_reduce<long long>("halo_reduce_p2p_fixed", g_ptrs, pull_offsets, pull_sources, world, rank,
                                 n_own, view_elems, stream);
+}
+
+extern "C" int mvsd_halo_gather_p2p(void* const* feat_ptrs, const int32_t* gather_sources, int world, int rank,
+                                    int n_own, int n_halo, int64_t view_bytes, void* stream) {
+  const char* who = "halo_gather_p2p";
+  if (!feat_ptrs || !gather_sources)
+    return fail(MVSD_ERR_INVALID_ARG, "%s: null pointer", who);
+  if (int e = check_world(who, world, rank)) return e;
+  if (n_own <= 0 || n_own > 65535 || n_halo <= 0 || n_halo > 65535 || view_bytes <= 0 || (view_bytes & 7))
+    return fail(MVSD_ERR_INVALID_ARG, "%s: bad view count / size", who);
+  GatherParams p;
+  p.feat = reinterpret_cast<char* const*>(feat_ptrs);
+  p.src = gather_sources; p.rank = rank; p.n_own = n_own;
+  p.view_bytes = (size_t)view_bytes;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (view_bytes & 15)
+    halo_gather_kernel<uint2><<<halo_grid((size_t)view_bytes / 8, n_halo), 256, 0, st>>>(p);
+  else
+    halo_gather_kernel<uint4><<<halo_grid((size_t)view_bytes / 16, n_halo), 256, 0, st>>>(p);
+  count_launch();
+  return check_launch(who);
 }
 
 extern "C" int mvsd_voxel_reduce_p2p(const void* const* part_ptrs, void* const* out_ptrs,

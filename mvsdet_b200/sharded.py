@@ -17,11 +17,21 @@ scene, giving replicas that are bit-identical across ranks.  Two combines exist:
   ``mvsd_voxel_normalize`` on every rank.  The counts travel as fp32 in the same
   buffer: they are integers <= V <= 2^24, so the sum is exact.
 
-The FPN feature maps of all V views are resident on every rank (the k=2 pose
-neighbours of a local view may belong to another rank, SURVEY.md 8e caveat 1);
-only the reference-view work is partitioned: a rank packs (fp32 NCHW -> channels-last
-bf16/fp32) just its own block plus the few neighbour views outside it ("halo"), and
-the neighbour ids are re-based onto that compact buffer.
+A rank sweeps its block of reference views against their k=2 pose neighbours, and some
+of those neighbours belong to another rank: the "halo" views.  The rank packs (fp32 NCHW
+-> channels-last bf16/fp32) its block plus its halo views into one compact buffer, and
+the neighbour ids are re-based onto it.  Two ways to fill that buffer:
+
+* ``ShardedSceneForward.__call__`` / ``ShardedScenePipeline.load`` take the FPN maps of
+  ALL V views on every rank and pack the block and the halo views from them;
+* ``ShardedSceneForward.forward_own`` / ``ShardedScenePipeline.load_own`` take the maps
+  of the rank's OWN views only (``owned_views`` names them before the backbone runs):
+  every rank packs its own rows into a peer-mapped buffer, a cross-rank barrier makes
+  them visible, and ``mvsd_halo_gather_p2p`` copies each halo view's packed map from its
+  owner over NVLink (``HaloExchange``; rows listed by ``halo_gather_table``).  The packed
+  buffer then holds the bits the first form packs, and the chain runs unchanged on it.
+  A rank must not re-pack its own rows while a peer may still be reading them: see
+  ``HaloExchange``.
 
 The partition / packing / all-reduce helpers are device-agnostic host logic and
 are exercised with a world-size-2 gloo group on CPU (tests/test_sharded_cpu.py);
@@ -38,9 +48,9 @@ import torch.distributed as dist
 from . import _lib, ops
 from ._lib import BP_MEAN, BP_SUM
 
-__all__ = ["partition_views", "halo_views", "halo_pull_table", "halo_counts", "pose_order", "permute_img_meta",
-           "pack_partials", "unpack_partials", "allreduce_partials", "LocalGeometry", "ShardedSceneForward",
-           "ShardedScenePipeline"]
+__all__ = ["partition_views", "halo_views", "halo_pull_table", "halo_gather_table", "halo_counts", "pose_order",
+           "permute_img_meta", "owned_views", "pack_partials", "unpack_partials", "allreduce_partials",
+           "LocalGeometry", "HaloExchange", "ShardedSceneForward", "ShardedScenePipeline"]
 
 
 def halo_views(neighbor_ids: torch.Tensor, begin: int, end: int) -> Tuple[List[int], torch.Tensor]:
@@ -86,6 +96,27 @@ def halo_pull_table(neighbor_ids: torch.Tensor, world: int, rank: int):
         offs.append(len(src))
     return (torch.tensor(offs, dtype=torch.int32),
             torch.tensor(src, dtype=torch.int32).reshape(-1, 2))
+
+
+def halo_gather_table(neighbor_ids: torch.Tensor, world: int, rank: int) -> torch.Tensor:
+    """Forward of a view-sharded scene whose ranks hold their own views only: where each halo view of
+    this rank lives.  ``neighbor_ids`` [V,k] are the FULL scene's ids (every rank computes the same tables
+    from them).  Returns int32 [n_halo,2] = (owner rank, row in the owner's buffer, whose rows are its own
+    views first), one row per halo view in the order ``halo_views`` puts them after the block: row j fills
+    local row ``n_own + j`` (``mvsd_halo_gather_p2p``).  The counterpart of ``halo_pull_table``.  Pure host
+    logic (tested on CPU)."""
+    nbr = neighbor_ids.to(torch.int64).cpu()
+    v = nbr.shape[0]
+    begin, end = partition_views(v, world, rank)
+    if end <= begin:
+        return torch.zeros((0, 2), dtype=torch.int32)
+    order, _ = halo_views(nbr[begin:end], begin, end)
+    blocks = [partition_views(v, world, q) for q in range(world)]
+    src = []
+    for g in order[end - begin:]:
+        q = next(q for q, (qb, qe) in enumerate(blocks) if qb <= g < qe)
+        src.append((q, g - blocks[q][0]))
+    return torch.tensor(src, dtype=torch.int32).reshape(-1, 2)
 
 
 def halo_counts(neighbor_ids: torch.Tensor, world: int, order: Optional[List[int]] = None) -> List[int]:
@@ -142,6 +173,40 @@ def permute_img_meta(img_meta: dict, order: List[int]) -> dict:
     out = dict(img_meta)
     out["lidar2img"] = l2i
     return out
+
+
+def _view_plan(hot_path, img_meta: dict, world: int, pose_clustered: bool):
+    """-> (order, img_meta with its views in that order, whole-scene neighbour ids [V,k] in that order's
+    numbering): rank r owns the views ``order[begin_r:end_r]`` of ``partition_views``."""
+    geo_full = hot_path.geometry(img_meta, "cpu", prologue="host")        # ids of the whole scene
+    v_all = geo_full.neighbor_ids_host.shape[0]
+    order = list(range(v_all))
+    if pose_clustered:
+        order = pose_order(img_meta["lidar2img"]["extrinsic"], geo_full.neighbor_ids_host, world)
+        if order != list(range(v_all)):
+            img_meta = permute_img_meta(img_meta, order)
+            geo_full = hot_path.geometry(img_meta, "cpu", prologue="host")   # ids in the permuted numbering
+    return order, img_meta, geo_full.neighbor_ids_host
+
+
+def owned_views(hot_path, img_meta: dict, world: int, rank: int,
+                pose_clustered: bool = True) -> Tuple[List[int], torch.Tensor]:
+    """The views rank ``rank`` of ``world`` owns in a view-sharded scene, known from the scene's poses
+    alone, so a detector can run its backbone and FPN on those images only and hand the maps to
+    ``ShardedSceneForward.forward_own`` / ``ShardedScenePipeline.load_own``.  ``pose_clustered``: the
+    blocks are pose clusters (``pose_order``) instead of index ranges.  Returns (order, view_ids int64
+    [Vb]): the scene's views in sharded order, and the rank's own views, in the row order the own-view
+    entry points take.  Every rank computes the same order from the same inputs.  Host logic."""
+    order, _, _ = _view_plan(hot_path, img_meta, world, pose_clustered)
+    begin, end = partition_views(len(order), world, rank)
+    return order, torch.tensor(order[begin:end], dtype=torch.int64)
+
+
+def _max_local_views(neighbor_ids: torch.Tensor, world: int) -> int:
+    """the largest block + halo view count over the ranks (the same on every rank)"""
+    v = neighbor_ids.shape[0]
+    return max(e - b + h for (b, e), h in zip((partition_views(v, world, r) for r in range(world)),
+                                              halo_counts(neighbor_ids, world)))
 
 
 @dataclass
@@ -250,6 +315,77 @@ class P2PVoxelReducer:
         return vol, self.out[self.total:].view(torch.int32)
 
 
+class HaloExchange:
+    """The forward halo exchange of a view-sharded scene whose ranks hold the feature maps of their own
+    views only.  Per call, on the current stream:
+
+    1. pack the own maps (fp32 NCHW) into rows [0, n_own) of this rank's peer-mapped packed buffer;
+    2. cross-rank barrier: every owner's rows are written and visible;
+    3. ``mvsd_halo_gather_p2p``: copy each halo view's packed map from its owner (``halo_gather_table``)
+       into rows n_own + j;
+
+    and the caller runs its chain on the returned buffer.  Every rank calls it, a rank without halo views
+    (its peers read from it) or without views too, so the barriers line up.  Buffers are torch symmetric
+    memory, allocated collectively with the same size on every rank (the largest local view count of the
+    group, all-reduced here); ``n_buffers`` buffers are used in turn by the caller.
+
+        xchg = HaloExchange(n_rows, (C, H, W), torch.bfloat16, device, group)
+        feat_cl = xchg(feature_own, gather_src)          # [n_own + n_halo, C, H, W] channels-last
+
+    REUSE: a rank must not pack into a buffer while a peer may still be gathering from it.  The caller
+    guarantees that a cross-rank barrier (or collective) follows every peer's gather before it reuses a
+    buffer: ``ShardedSceneForward`` uses one buffer, because the combine that follows the gather in stream
+    order is a barrier (p2p) or an all-reduce (NCCL); ``ShardedScenePipeline`` uses one buffer per slot,
+    because its combine runs on another stream, so the buffer of scene i+2 is packed only after the
+    exchange barrier of scene i+1, which every peer enters after its gather of scene i."""
+
+    def __init__(self, n_rows: int, view_shape: Tuple[int, int, int], dtype, device, group=None,
+                 n_buffers: int = 1):
+        import torch.distributed._symmetric_memory as symm
+        if not (dist.is_available() and dist.is_initialized()):
+            raise RuntimeError("HaloExchange needs an initialised process group")
+        self.group = group if group is not None else dist.group.WORLD
+        self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
+        dev = torch.device(device)
+        rows = torch.tensor([int(n_rows)], device=dev)
+        dist.all_reduce(rows, op=dist.ReduceOp.MAX, group=self.group)        # symmetric allocation
+        self.capacity = int(rows.item())
+        self.view_shape, self.dtype = tuple(int(x) for x in view_shape), dtype
+        c, h, w = self.view_shape
+        self.view_bytes = c * h * w * torch.empty((), dtype=dtype).element_size()
+        self._bufs, self._handles = [], []
+        for _ in range(n_buffers):
+            buf = symm.empty(max(self.capacity, 1) * h * w * c, dtype=dtype, device=dev)
+            hdl = symm.rendezvous(buf, self.group)
+            if hdl.buffer_ptrs[self.rank] != buf.data_ptr():
+                raise RuntimeError("symmetric buffer does not start at its peer pointer")
+            self._bufs.append(buf)
+            self._handles.append(hdl)
+
+    def fits(self, n_rows: int, view_shape, dtype) -> bool:
+        return n_rows <= self.capacity and tuple(view_shape) == self.view_shape and dtype == self.dtype
+
+    def rows(self, n: int, i: int = 0) -> torch.Tensor:
+        """the first ``n`` rows of buffer ``i`` as logical [n,C,H,W] in channels_last memory"""
+        c, h, w = self.view_shape
+        return self._bufs[i][:n * h * w * c].view(n, h, w, c).permute(0, 3, 1, 2)
+
+    def __call__(self, feature_own: torch.Tensor, gather_src: torch.Tensor, i: int = 0) -> torch.Tensor:
+        """feature_own fp32 NCHW [n_own,C,H,W], gather_src int32 [n_halo,2] on the device -> buffer ``i``'s
+        rows [n_own + n_halo] with the own maps packed and the halo maps gathered"""
+        n_own, n_halo = feature_own.shape[0], gather_src.shape[0]
+        if n_own + n_halo > self.capacity:
+            raise ValueError(f"{n_own + n_halo} local views exceed the exchange's {self.capacity}")
+        out = self.rows(n_own + n_halo, i)
+        if n_own:
+            _lib.pack(feature_own, out[:n_own])
+        self._handles[i].barrier(channel=0)          # every owner's rows are complete and visible
+        if n_halo:
+            _lib.halo_gather_p2p(self._handles[i].buffer_ptrs_dev, gather_src, world=self.world, rank=self.rank,
+                                 n_own=n_own, view_bytes=self.view_bytes)
+        return out
+
+
 class ShardedSceneForward:
     """Forward of one scene with the reference views split over the group.
 
@@ -260,13 +396,17 @@ class ShardedSceneForward:
     ``feature`` holds ALL views on every rank.  The all-reduce runs on the
     current stream right after the local back-projection (there is nothing left
     to overlap it with inside one scene; a multi-scene caller overlaps it with
-    the next scene's sweep by calling from a side stream)."""
+    the next scene's sweep by calling from a side stream).
+
+    ``forward_own`` is the form whose ranks hold their OWN views' maps only (``owned_views``): the halo
+    maps come from their owners over NVLink (``HaloExchange``), and the result is the same."""
 
     def __init__(self, hot_path, group=None, p2p: bool = True):
         self.hot = hot_path
         self.group = group
         self.p2p = p2p                 # combine over NVLink peer memory (default); False = NCCL all-reduce
         self._reducer = None
+        self._xchg: Optional[HaloExchange] = None
 
     def _world(self) -> Tuple[int, int]:
         if dist.is_available() and dist.is_initialized():
@@ -323,41 +463,108 @@ class ShardedSceneForward:
                 geo = hot.geometry(img_meta, dev, view_slice=slice(begin, end), prologue="host")
                 views, nbr_local = halo_views(geo.neighbor_ids_host, begin, end)
                 lg = LocalGeometry(geo, views, nbr_local.to(dev), begin, end)
-            geo = lg.geo
             feat_cl = self._pack_local(feature, lg)            # block + halo only
-            variance = ops.plane_sweep_variance(feat_cl, lg.neighbor_ids_local, geo.hom,
-                                                geo.depth_values, out_dtype=hot.variance_dtype,
-                                                ref_begin=0)
-            cost_out = cost_net(variance)
-            _, _, est_depth, est_dens, est_idx, _ = hot.hypotheses(cost_out)
-            vol_sum, count = ops.backproject_aggregate(
-                feat_cl[:end - begin], geo.points, geo.projection, est_depth, est_dens,
-                hot.voxel_size[2], geo.height, geo.width, mode="sum",
-                channels_first=hot.channels_first_volume,
-                out=None if partial_out is None else partial_out[0],
-                count_out=None if partial_out is None else partial_out[1])
+            vol_sum, count = self._chain(feat_cl, lg, cost_net, partial_out)
         else:                                   # more ranks than views: contribute zeros
-            shape = (c, n) if hot.channels_first_volume else (n, c)
-            vol_sum = torch.zeros(shape, dtype=torch.float32, device=dev)
-            vol_sum = vol_sum if hot.channels_first_volume else vol_sum.t()
-            count = torch.zeros(n, dtype=torch.int32, device=dev)
+            vol_sum, count = self._zero_partials(c, dev)
         return vol_sum, count, (begin, end)
+
+    def _chain(self, feat_cl: torch.Tensor, lg: LocalGeometry, cost_net: Callable, partial_out):
+        """sweep -> cost net -> top-k -> back-projection(SUM) of the rank's reference views over its packed
+        block + halo buffer -> (volume_sum logical [C,N], count int32 [N])"""
+        hot, geo = self.hot, lg.geo
+        variance = ops.plane_sweep_variance(feat_cl, lg.neighbor_ids_local, geo.hom,
+                                            geo.depth_values, out_dtype=hot.variance_dtype,
+                                            ref_begin=0)
+        cost_out = cost_net(variance)
+        _, _, est_depth, est_dens, est_idx, _ = hot.hypotheses(cost_out)
+        return ops.backproject_aggregate(
+            feat_cl[:lg.end - lg.begin], geo.points, geo.projection, est_depth, est_dens,
+            hot.voxel_size[2], geo.height, geo.width, mode="sum",
+            channels_first=hot.channels_first_volume,
+            out=None if partial_out is None else partial_out[0],
+            count_out=None if partial_out is None else partial_out[1])
+
+    def _zero_partials(self, c: int, dev):
+        hot = self.hot
+        nx, ny, nz = hot.n_voxels
+        n = nx * ny * nz
+        shape = (c, n) if hot.channels_first_volume else (n, c)
+        vol_sum = torch.zeros(shape, dtype=torch.float32, device=dev)
+        vol_sum = vol_sum if hot.channels_first_volume else vol_sum.t()
+        return vol_sum, torch.zeros(n, dtype=torch.int32, device=dev)
+
+    def _cost_net(self, cost_regularization):
+        cost_net = cost_regularization or self.hot.cost_regularization
+        if cost_net is None:
+            raise ValueError("a cost_regularization callable is required (mvsdet.py:470)")
+        return cost_net
+
+    def _partial_out(self, c: int, device):
+        """the p2p reducer's peer-mapped partial buffers, or None for the NCCL combine / a single rank"""
+        if not (self.p2p and self._world()[1] > 1):
+            return None
+        if self._reducer is None:
+            nx, ny, nz = self.hot.n_voxels
+            self._reducer = P2PVoxelReducer(c, nx * ny * nz, self.hot.channels_first_volume, device, self.group)
+        return self._reducer.partial_buffers()
 
     def __call__(self, feature: torch.Tensor, img_meta: dict,
                  cost_regularization: Optional[Callable] = None, geometry=None) -> Dict[str, torch.Tensor]:
+        cost_net = self._cost_net(cost_regularization)
+        partial_out = self._partial_out(feature.shape[1], feature.device)
+        vol_sum, count, (begin, end) = self.local_partials(feature, img_meta, cost_net, geometry,
+                                                           partial_out=partial_out)
+        return self._combine(vol_sum, count, partial_out is not None, (begin, end))
+
+    def forward_own(self, feature_own: torch.Tensor, img_meta: dict,
+                    cost_regularization: Optional[Callable] = None,
+                    pose_clustered: bool = True) -> Dict[str, torch.Tensor]:
+        """``__call__`` from the maps of this rank's OWN views: ``feature_own`` [Vb,C,H,W] (fp32 FPN maps) of
+        the views ``owned_views(hot, img_meta, world, rank, pose_clustered)`` names, in that order.  The rank
+        packs them, and pulls the packed maps of its halo views from their owners over NVLink
+        (``HaloExchange``) instead of packing them from a replicated input.  ``cost_regularization`` gets the
+        variance of the own views, in the same order.  Every rank of the group must call it (the exchange
+        has a barrier), a rank without views too (then with ``feature_own`` of 0 rows).  Returns the dict of
+        ``__call__`` plus ``view_ids``; with ``pose_clustered=False`` its values are the bits of ``__call__``
+        on the whole scene's maps.  ``view_range`` is the rank's block in the sharded order."""
         hot = self.hot
-        cost_net = cost_regularization or hot.cost_regularization
-        if cost_net is None:
-            raise ValueError("a cost_regularization callable is required (mvsdet.py:470)")
-        c = feature.shape[1]
+        cost_net = self._cost_net(cost_regularization)
+        rank, world = self._world()
+        order, img_meta, nbr_full = _view_plan(hot, img_meta, world, pose_clustered)
+        v_all = len(order)
+        begin, end = partition_views(v_all, world, rank)
+        if feature_own.dim() != 4 or feature_own.shape[0] != end - begin:
+            raise ValueError(f"feature_own must hold the rank's {end - begin} own views [Vb,C,H,W], "
+                             f"got {tuple(feature_own.shape)}")
+        dev = feature_own.device
+        c, h, w = feature_own.shape[1:]
+        feature_own = feature_own.to(torch.float32).contiguous()
+        partial_out = self._partial_out(c, dev)
+        n_rows = _max_local_views(nbr_full, world)
+        if self._xchg is None or not self._xchg.fits(n_rows, (c, h, w), hot.feature_dtype):
+            # every rank takes this branch together: n_rows comes from the same whole-scene table
+            self._xchg = None
+            self._xchg = HaloExchange(n_rows, (c, h, w), hot.feature_dtype, dev, self.group)
+        lg = self.local_geometry(img_meta, v_all, dev)
+        src = halo_gather_table(nbr_full, world, rank).to(dev)
+        # one packed buffer: the combine below follows this rank's gather in stream order and is a barrier
+        # (p2p) or an all-reduce (NCCL) that every peer enters after its own gather, so the next scene's
+        # pack cannot overwrite rows a peer is still reading
+        feat_cl = self._xchg(feature_own, src)
+        if lg is not None:
+            vol_sum, count = self._chain(feat_cl, lg, cost_net, partial_out)
+        else:
+            vol_sum, count = self._zero_partials(c, dev)
+        out = self._combine(vol_sum, count, partial_out is not None, (begin, end))
+        out["view_ids"] = torch.tensor(order[begin:end], dtype=torch.int64)
+        return out
+
+    def _combine(self, vol_sum, count, use_p2p: bool, view_range) -> Dict[str, torch.Tensor]:
+        hot = self.hot
+        c = vol_sum.shape[0]
         nx, ny, nz = hot.n_voxels
         n = nx * ny * nz
-        use_p2p = self.p2p and self._world()[1] > 1
-        if use_p2p and self._reducer is None:
-            self._reducer = P2PVoxelReducer(c, n, hot.channels_first_volume, feature.device, self.group)
-        vol_sum, count, (begin, end) = self.local_partials(
-            feature, img_meta, cost_net, geometry,
-            partial_out=self._reducer.partial_buffers() if use_p2p else None)
         if use_p2p:
             # the reducer's result buffers are peer-mapped and reused by the next scene (peers store
             # into them): hand the caller its own copy, as the NCCL branch does (the reference
@@ -372,17 +579,23 @@ class ShardedSceneForward:
         vm = (volume_mean.view(c, nx, ny, nz) if volume_mean.is_contiguous()
               else volume_mean.unflatten(1, (nx, ny, nz)))
         return dict(volume_mean=vm, valid=count.view(1, nx, ny, nz).float(), count=count,
-                    view_range=(begin, end))
+                    view_range=view_range)
 
 
 class ShardedScenePipeline:
     """Pre-allocated view-sharded forward (+ backward) of ONE large scene per rank -- the
     multi-GPU counterpart of ``pipeline.ScenePipeline`` (BASELINE.json configs[2] / [3]).
 
-    Per rank: the fp32 FPN maps of its block of reference views plus the halo views (the pose
-    neighbours it does not own) are resident ("pre-placed halos", SURVEY.md 8e caveat 1); the
+    Per rank, after ``load``: the fp32 FPN maps of its block of reference views plus the halo views (the
+    pose neighbours it does not own) are resident ("pre-placed halos", SURVEY.md 8e caveat 1); the
     chain  pack -> plane sweep -> top-k -> back-projection(SUM)  writes the partial voxel sums and
-    counts straight into a peer-mapped buffer and is replayed as ONE CUDA graph; the combine
+    counts straight into a peer-mapped buffer and is replayed as ONE CUDA graph.  After ``load_own`` only
+    the rank's own maps are resident: each forward packs them into the slot's peer-mapped packed buffer,
+    and, after a cross-rank barrier, gathers the halo views' packed maps from their owners
+    (``HaloExchange``; both outside the graph, which then replays sweep -> top-k -> back-projection).
+    The packed buffers are per slot, so the pack of scene i+2 comes after the exchange barrier of scene
+    i+1, which every peer enters only after its gather of scene i (the combine runs on another stream
+    and orders nothing on the compute stream).  The two forms give the same bits.  The combine
     (sum over ranks + ``sum / (count + 1e-8)``, mvsdet.py:511-515, :681-682) is either
     ``mvsd_voxel_reduce_p2p`` over NVLink peer pointers between two symmetric-memory barriers
     ("p2p") or NCCL all-reduces + ``mvsd_voxel_normalize`` ("nccl").  Partial and result buffers are
@@ -426,6 +639,7 @@ class ShardedScenePipeline:
         self._ev_free = [None, None]      # slot's partial buffer consumed by the combine (comm stream)
         self._graphs = [None, None]
         self.lg: Optional[LocalGeometry] = None
+        self._xchg: Optional[HaloExchange] = None     # own-view input (load_own): the halo exchange
         self._g_feat = None
         self._bwd_graphs: Dict = {}
         self._slot = 0
@@ -438,32 +652,62 @@ class ShardedScenePipeline:
         ``pose_clustered``: the ranks' blocks are pose clusters (``pose_order``) instead of index ranges;
         ``self.view_ids`` (also ``view_ids`` in ``forward``'s result) lists the views this rank owns, in the
         order of the rows ``backward`` takes and returns."""
-        hot, cfg, dev = self.hot, self.cfg, self.device
-        v_all = feature.shape[0]
+        order, begin, end = self._plan(feature.shape[0], img_meta, pose_clustered)
+        views = self.lg.views
+        self.feature = feature[[order[i] for i in views]].to(self.device, dtype=torch.float32).contiguous()
+        self._xchg = None
+        hf, wf = self.cfg.feat_hw
+        feat_cl = ops._empty_nhwc(len(views), self.c, hf, wf, self.hot.feature_dtype, self.device)
+        self._allocate(cost_out[order[begin:end]], [feat_cl, feat_cl])
+
+    def load_own(self, feature_own: torch.Tensor, cost_out_own: torch.Tensor, img_meta: dict,
+                 pose_clustered: bool = True) -> None:
+        """``load`` from the maps of this rank's OWN views: ``feature_own`` [Vb,C,Hf,Wf] fp32 and
+        ``cost_out_own`` [Vb,2,D,Hf,Wf] of the views ``owned_views(hot, img_meta, world, rank,
+        pose_clustered)`` names, in that order (host or device).  Only they are resident; every forward
+        gathers the halo views' packed maps from their owners (``HaloExchange``).  ``forward``,
+        ``forward_stream`` and ``backward`` then give the bits they give after ``load`` of the whole scene.
+        Collective: every rank of the group calls it."""
+        v_all = len(img_meta["lidar2img"]["extrinsic"])
+        begin, end = partition_views(v_all, self.world, self.rank)
+        for name, x in (("feature_own", feature_own), ("cost_out_own", cost_out_own)):
+            if x.shape[0] != end - begin:
+                raise ValueError(f"{name} must have one row per owned view ({end - begin}, view_ids), "
+                                 f"got {x.shape[0]}")
+        self._plan(v_all, img_meta, pose_clustered)
+        dev, hf, wf = self.device, *self.cfg.feat_hw
+        self.feature = feature_own.to(dev, dtype=torch.float32).contiguous()
+        self._xchg = None
+        self._xchg = HaloExchange(_max_local_views(self.nbr_full, self.world), (self.c, hf, wf),
+                                  self.hot.feature_dtype, dev, self.group, n_buffers=2)
+        self._gather_src = halo_gather_table(self.nbr_full, self.world, self.rank).to(dev)
+        vl = len(self.lg.views)
+        self._allocate(cost_out_own, [self._xchg.rows(vl, i) for i in range(2)])
+
+    def _plan(self, v_all: int, img_meta: dict, pose_clustered: bool) -> Tuple[List[int], int, int]:
+        """the views this rank owns (``owned_views``), its geometry and halo -> (order, begin, end)"""
         begin, end = partition_views(v_all, self.world, self.rank)
         if end <= begin:
             raise ValueError("more ranks than reference views")
-        geo_full = hot.geometry(img_meta, "cpu", prologue="host")           # ids of the whole scene
-        order = list(range(v_all))
-        if pose_clustered:
-            order = pose_order(img_meta["lidar2img"]["extrinsic"], geo_full.neighbor_ids_host, self.world)
-            if order != list(range(v_all)):
-                img_meta = permute_img_meta(img_meta, order)
-                geo_full = hot.geometry(img_meta, "cpu", prologue="host")   # ids in the permuted numbering
+        order, img_meta, self.nbr_full = _view_plan(self.hot, img_meta, self.world, pose_clustered)
         self.view_order = order
         self.view_ids = torch.tensor(order[begin:end], dtype=torch.int64)
-        self.nbr_full = geo_full.neighbor_ids_host
         self.halo_counts = halo_counts(self.nbr_full, self.world)
-        geo = hot.geometry(img_meta, dev, view_slice=slice(begin, end), prologue="host")
+        geo = self.hot.geometry(img_meta, self.device, view_slice=slice(begin, end), prologue="host")
         views, nbr_local = halo_views(geo.neighbor_ids_host, begin, end)
-        self.lg = LocalGeometry(geo, views, nbr_local.to(dev), begin, end)
-        vl, vb = len(views), end - begin
+        self.lg = LocalGeometry(geo, views, nbr_local.to(self.device), begin, end)
+        return order, begin, end
+
+    def _allocate(self, cost_out: torch.Tensor, feat_slots: List[torch.Tensor]) -> None:
+        """the resident cost volume, the packed feature buffer of each slot and the chain's outputs"""
+        hot, cfg, dev = self.hot, self.cfg, self.device
+        vl, vb = len(self.lg.views), self.lg.end - self.lg.begin
         d, t = cfg.num_depth, cfg.topk
         hf, wf = cfg.feat_hw
         f32 = dict(dtype=torch.float32, device=dev)
-        self.feature = feature[[order[i] for i in views]].to(dev, dtype=torch.float32).contiguous()
-        self.cost_out = cost_out[order[begin:end]].to(dev, dtype=torch.float32).contiguous()
-        self.feat_cl = ops._empty_nhwc(vl, self.c, hf, wf, hot.feature_dtype, dev)
+        self.cost_out = cost_out.to(dev, dtype=torch.float32).contiguous()
+        self._feat_slots = feat_slots
+        self.feat_cl = feat_slots[0]        # the packed buffer of the last forward (``backward`` reads it)
         self.variance = ops._empty_ndhwc(vb, self.c, d, hf, wf, hot.variance_dtype, dev)
         self.est_depth = torch.empty((vb, t, hf, wf), **f32)
         self.est_dens = torch.empty((vb, t, hf, wf), **f32)
@@ -475,18 +719,23 @@ class ShardedScenePipeline:
         torch.cuda.synchronize(dev)
 
     def _enqueue_compute(self, slot: int) -> None:
-        """pack -> sweep -> top-k -> back-projection(SUM) into the slot's partials; current stream; capturable."""
+        """pack (after ``load``) -> sweep -> top-k -> back-projection(SUM) into the slot's partials; current
+        stream; capturable."""
         cfg, lg, geo = self.cfg, self.lg, self.lg.geo
-        _lib.pack(self.feature, self.feat_cl)
-        _lib.plane_sweep_fwd(self.feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self.variance)
+        feat_cl = self._feat_slots[slot]
+        if self._xchg is None:
+            _lib.pack(self.feature, feat_cl)
+        _lib.plane_sweep_fwd(feat_cl, lg.neighbor_ids_local, geo.hom, geo.depth_values, self.variance)
         _lib.depth_topk_fwd(self.cost_out, None, None, self.est_depth, self.est_dens, self.est_idx, None,
                             near=cfg.near_far_range[0], interval=cfg.depth_interval)
         vol_sum, count = self._red[slot].partial_buffers()
-        _lib.backproject_fwd(self.feat_cl, geo.points, geo.projection, self.est_depth, self.est_dens, vol_sum,
+        _lib.backproject_fwd(feat_cl, geo.points, geo.projection, self.est_depth, self.est_dens, vol_sum,
                              vs_z=cfg.voxel_size[2], mode=BP_SUM, height=geo.height, width=geo.width,
                              channels_first=True, count=count)
 
     def _compute(self, slot: int, use_graph: bool = True) -> None:
+        if self._xchg is not None:          # own-view input: pack + barrier + gather, outside the graph
+            self._xchg(self.feature, self._gather_src, slot)
         if not use_graph:
             self._enqueue_compute(slot)
             return
@@ -532,7 +781,7 @@ class ShardedScenePipeline:
         self._slot ^= 1
         self._compute(slot, use_graph)
         res = self._combine(slot, mode)
-        self._last_slot = slot
+        self._last_slot, self.feat_cl = slot, self._feat_slots[slot]
         return res
 
     def forward_stream(self, mode: str = "p2p", n_scenes: int = 8, use_graph: bool = True):
@@ -554,7 +803,7 @@ class ShardedScenePipeline:
                 done = torch.cuda.Event()
                 done.record(self.s_comm)
             self._ev_free[slot] = done
-            self._last_slot = slot
+            self._last_slot, self.feat_cl = slot, self._feat_slots[slot]
         cur.wait_stream(self.s_comm)
         return res
 
